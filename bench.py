@@ -1,6 +1,6 @@
 """bench.py -- PointNet++ SSG semantic-segmentation forward, points/sec (BASELINE.json metric, config C2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--depth D]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--depth D] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -21,6 +21,10 @@ Our arm prints one JSON line with
                  CUDA hidden, in a child process; cpu_baseline_port = the C/OpenMP oracle port (oracle/)
   train, dp_check  config C5 (training iteration with the NCCL gradient all-reduce) and the data-parallel equivalence check
 `--impl reference` runs that unmodified reference as the reference arm (rank 0 only under torchrun), same metric and `config`.
+`--dump-outputs DIR` (our arm, c2) writes what the last step of each timed region returned to its caller, as float32 .npy files
+(rank 0's): log_probs [B, N, 19] (inputs in HBM), e2e_log_probs [B, N, 19] (pinned host) and e2e_labels [B, N] (argmax), 30 MB
+in all.  The inputs and the FPS start draws of the timed steps are seeded, so two runs with the same arguments, on two builds,
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -65,7 +69,22 @@ def parse():
                          "(tools/bench_train.py; same JSON contract); preprocess: raw scans -> network input (tools/bench_preprocess.py)")
     ap.add_argument("--mode", default="graph", choices=["graph", "eager"],
                     help="graph: one CUDA-graph replay per step (default); eager: ~40 launches per step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step of each region as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs covers the c2 workload of --impl ours")
+    return args
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: one float32 DIR/<name>.npy per array."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -436,9 +455,10 @@ def run_ours(args):
     seq_runner = GraphedSemSeg(net, depth=1) if args.mode == "graph" else None
 
     def region(batches, steps, to_host):
-        """K steps with `depth` batches in flight, timed as ONE region on the device; returns (ms, per-step completion times)."""
+        """K steps with `depth` batches in flight, timed as ONE region on the device; returns (ms, per-step completion times,
+        the output of the last step: a static buffer, valid until the next step)."""
         start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        dones, pending = [], []
+        dones, pending, out = [], [], None
         start.record()
         for i in range(steps):
             if runner is None:
@@ -446,8 +466,9 @@ def run_ours(args):
                     x = batches[i % NB_INPUTS]
                     if to_host:
                         net(x.to(dev, non_blocking=True), host_out=eager_host_out)
+                        out = eager_host_out
                     else:
-                        net(x)
+                        out = net(x)
                 ev = torch.cuda.Event(enable_timing=True)
                 ev.record()
                 dones.append(ev)
@@ -455,15 +476,22 @@ def run_ours(args):
             pending.append(runner.submit(batches[i % NB_INPUTS], to_host=to_host))
             if len(pending) >= depth:
                 t = pending.pop(0)
-                runner.result(t)              # device output: orders this stream after batch k; host output: waits for it
+                out = runner.result(t)        # device output: orders this stream after batch k; host output: waits for it
                 dones.append(t.done)
         for t in pending:
-            runner.result(t)
+            out = runner.result(t)
             dones.append(t.done)
         end.record()
         torch.cuda.synchronize()
         marks = sorted(start.elapsed_time(d) for d in dones)     # (batches run on their own streams and may finish out of order)
-        return start.elapsed_time(end), [b - a for a, b in zip([0.0] + marks[:-1], marks)]
+        return start.elapsed_time(end), [b - a for a, b in zip([0.0] + marks[:-1], marks)], out
+
+    outputs = {}
+
+    def keep(name, out):
+        """--dump-outputs: a float32 host copy of a region's last output, taken before the next region reuses the buffer."""
+        if args.dump_outputs and rank == 0:
+            outputs[name] = out.to("cpu", torch.float32, copy=True).numpy()
 
     eager_host_out = torch.empty((BATCH, NPOINTS, CLASSES), dtype=torch.float32).pin_memory() if runner is None else None
     if runner is not None:
@@ -478,20 +506,27 @@ def run_ours(args):
     if runner is not None:
         region(host_batches, Wp, "labels")
     barrier()
+    # the FPS start draws of the timed steps then depend on the seed and --steps only, not on how many draws the warm-up made
+    torch.manual_seed(1234 + rank)
 
     # ---- timed regions (the clock sampler spans all of them: one region is only ~10 ms long)
     with ClockSampler(local) as clocks:
         # 1: inputs resident in HBM, `depth` batches in flight
-        ms, per_step = region(dev_batches, args.steps, False)
+        ms, per_step, out = region(dev_batches, args.steps, False)
+        keep("log_probs", out)
         barrier()
         # 2: end to end from pinned host memory and back (full log-probabilities)
-        ms_e2e, _ = region(host_batches, args.steps, True)
+        ms_e2e, _, out = region(host_batches, args.steps, True)
+        keep("e2e_log_probs", out)
         barrier()
         # 3: the same with what the reference's evaluation loop keeps of the output: pred.argmax(-1) (pcdseg.py:75) as uint8
         ms_lab = 0.0
         if runner is not None:
-            ms_lab, _ = region(host_batches, args.steps, "labels")
+            ms_lab, _, out = region(host_batches, args.steps, "labels")
+            keep("e2e_labels", out)
             barrier()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- one batch at a time (round-1 protocol: per-step CUDA events, 512 MiB written between steps) for comparison
     seq = None
@@ -648,7 +683,8 @@ def main():
         if args.workload == "preprocess":
             import bench_preprocess
 
-            bench_preprocess.main([], cpu_baseline=None if args.no_cpu_baseline else cpu_preprocess_oracle)
+            bench_preprocess.main(["--steps", str(args.steps), "--warmup", str(args.warmup)],
+                                  cpu_baseline=None if args.no_cpu_baseline else cpu_preprocess_oracle)
             return
         import bench_train
 
@@ -666,12 +702,12 @@ def main():
         sys.path.insert(0, os.path.join(ROOT, "tools"))
         import bench_train
 
-        train = bench_train.main(["--steps", str(max(10, args.steps)), "--warmup", str(max(3, args.warmup)), "--no-cpu-baseline"],
+        train = bench_train.main(["--steps", str(args.steps), "--warmup", str(max(3, args.warmup)), "--no-cpu-baseline"],
                                  init_pg=False, emit=False)
         check = bench_train.dp_check(world, rank, dev)
         if line is not None:
             line["train"] = None if train is None else {
-                k: train[k] for k in ("metric", "value", "unit", "ms_per_step", "step_ms", "e2e", "allreduce_us", "allreduce_bytes",
+                k: train[k] for k in ("metric", "value", "unit", "steps", "ms_per_step", "step_ms", "e2e", "allreduce_us", "allreduce_bytes",
                                       "gpu_launches", "final_loss")}
             if train is not None:
                 line["train"]["config"] = train["config"]

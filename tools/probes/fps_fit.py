@@ -1,7 +1,8 @@
-import sys, json, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, json, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, ROOT)
 from pointnet12_b200 import ops, synthetic as syn
-sys.path.insert(0, '/root/repo/tools')
+sys.path.insert(0, os.path.join(ROOT, 'tools'))
 from microbench import time_ms
 dev = torch.device('cuda', 0)
 B, npoint = 8, 1024

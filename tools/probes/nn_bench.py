@@ -1,5 +1,6 @@
-import sys, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0, '/root/repo/tools')
+import os, sys, torch
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tools'))
 from pointnet12_b200 import ops, synthetic as syn
 from microbench import time_ms
 dev = torch.device('cuda', 0)
