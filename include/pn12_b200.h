@@ -408,8 +408,10 @@ int pn_three_interpolate_bwd_f32(const float* dx, int64_t ldx, int D1, int D2, c
 int pn_dropout_f32(const float* x, int64_t ldx, int64_t rows, int C, float p, const uint64_t* seed_offset,
                    const uint8_t* mask_in, uint8_t* mask_out, float* y, int64_t ldy, pn_stream_t stream);
 /* nn.CrossEntropyLoss()(x^T, target) as pcdseg.py:177-178 applies it to the network's log-probabilities:
- * loss = mean_r (logsumexp(x_r) - x_r[target_r]); dx (may be NULL) = (softmax(x_r) - onehot) * grad_scale / rows.
- * loss_sum: one fp64 scratch word, loss: one fp32 word (both device). */
+ * loss = mean_r (logsumexp(x_r) - x_r[target_r]); dx (may be NULL) = (softmax(x_r) - onehot) * grad_scale / n.
+ * Rows with target -100 (ignore_index) are left out of the mean and get dx = 0; n counts the other rows (all rows
+ * ignored: loss = NaN, like torch).  Any other target outside [0, C) makes the loss and that row of dx NaN.
+ * loss_sum: two fp64 scratch words (sum, n), loss: one fp32 word (both device). */
 int pn_cross_entropy_f32(const float* x, int64_t ldx, const int64_t* target, int64_t rows, int C, double* loss_sum,
                          float* loss, float* dx, int64_t lddx, float grad_scale, pn_stream_t stream);
 /* Backward of F.log_softmax (pointnet2.py:174): dx = dy - exp(y)*sum_c dy, y = the log-probabilities. */

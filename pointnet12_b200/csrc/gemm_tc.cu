@@ -203,7 +203,7 @@ train_gemm_kernel(const Args a) {
     float* tf = reinterpret_cast<float*>(bars + 32);                                           // [2][k_pad]: in_scale | in_shift (16-byte aligned)
     double* cta_sum = reinterpret_cast<double*>(tf + 2 * a.k_pad);                             // [2][n_pad]: this CTA's column sums over all its tiles
     float* bias_s = reinterpret_cast<float*>(cta_sum + 2 * a.n_pad);                           // [n_pad], zero beyond cout
-    float* pc = bias_s + a.n_pad;                                                               // [4][n_pad]: scale, shift, mean, invstd of the layer below
+    float* pc = bias_s + a.n_pad;                                                               // [4][n_pad]: scale, shift, mean, invstd of the layer below (forward: [0] = statistics pivots)
     float* stg_all = pc + 4 * a.n_pad;                                                          // [4 epilogue warps][32 rows][20]: output staging
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const unsigned bar_full = smem_u32(bars), bar_empty = smem_u32(bars + NS_MAX), bar_accf = smem_u32(bars + 2 * NS_MAX),
@@ -267,8 +267,11 @@ train_gemm_kernel(const Args a) {
             if (row2 < a.rows && c2 * KC < a.cin) asm volatile("prefetch.global.L2 [%0];" ::"l"(a.x + row2 * a.ldx + c2 * KC));
         }
     }
-    if (a.col_sum)
+    if (a.col_sum) {
         for (int n = tid; n < 2 * a.n_pad; n += THREADS) cta_sum[n] = 0.0;
+        if (!a.py)
+            for (int n = tid; n < a.n_pad; n += THREADS) pc[n] = 0.0f;     // the pivots, set by the first tile's epilogue
+    }
     for (int n = tid; n < a.n_pad; n += THREADS) bias_s[n] = (a.bias && n < a.cout) ? __ldg(a.bias + n) : 0.0f;
     if (a.py)
         for (int n = tid; n < a.n_pad; n += THREADS) {
@@ -471,11 +474,27 @@ train_gemm_kernel(const Args a) {
                             }
                         }
                     } else {
+                        // FORWARD statistics, shifted by a per-column pivot p (the CTA's first row): sum (y-p), sum (y-p)^2.
+                        // Unshifted, the fp32 square would carry a rounding of |mean|^2 * 2^-24 that does not average out
+                        // (a constant channel at 27.1 gets var = 7.5e-5 instead of 0), and var = E[y^2] - mean^2 keeps it.
+                        float* piv = pc;                         // (pc holds the layer below's constants in the backward only)
+                        if (it == 0) {
+                            if (q == 0 && lane == 0)
 #pragma unroll
-                        for (int j = 0; j < 32; ++j) {
-                            const float d = row_ok ? v[j] : 0.0f;
-                            f1[j] = d;
-                            f2[j] = d * d;
+                                for (int j = 0; j < 32; ++j) piv[col0 + j] = v[j];
+                            asm volatile("bar.sync 1, 128;" ::: "memory");       // the four epilogue warps
+                        }
+                        const float4* p4 = reinterpret_cast<const float4*>(piv + col0);
+#pragma unroll
+                        for (int j = 0; j < 32; j += 4) {
+                            const float4 pp = p4[j >> 2];
+                            const float pv[4] = {pp.x, pp.y, pp.z, pp.w};
+#pragma unroll
+                            for (int i = 0; i < 4; ++i) {
+                                const float d = row_ok ? v[j + i] - pv[i] : 0.0f;
+                                f1[j + i] = d;
+                                f2[j + i] = d * d;
+                            }
                         }
                     }
                     colsum_step_f<16>(f1, lane);
@@ -495,10 +514,20 @@ train_gemm_kernel(const Args a) {
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (a.col_sum) {
+    if (a.col_sum && my_tiles > 0) {
+        // forward: the shifted sums of the CTA's rows back to plain sums, in fp64 (s2 + 2 p s1 + n p^2 loses nothing
+        // that matters: var = E[y^2] - mean^2 in fp64 keeps a relative error of (mean/std)^2 * 2^-53)
+        const int64_t short_rows = (blockIdx.x == (tiles - 1) % gridDim.x) ? tiles * TM - a.rows : 0;
+        const double nc = (double)(my_tiles * TM - short_rows);
         for (int n = tid; n < a.cout; n += THREADS) {
-            atomicAdd(a.col_sum + n, cta_sum[n]);
-            atomicAdd(a.col_sumsq + n, cta_sum[a.n_pad + n]);
+            double s1 = cta_sum[n], s2 = cta_sum[a.n_pad + n];
+            if (!a.py) {
+                const double p = (double)pc[n];
+                s2 += p * (2.0 * s1 + nc * p);
+                s1 += nc * p;
+            }
+            atomicAdd(a.col_sum + n, s1);
+            atomicAdd(a.col_sumsq + n, s2);
         }
     }
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(tmem_cols));

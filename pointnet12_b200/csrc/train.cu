@@ -453,32 +453,55 @@ __global__ void dropout_kernel(const float* __restrict__ x, int64_t ldx, int64_t
 // ------------------------------------------------------------------------------------------------
 // nn.CrossEntropyLoss()(x.transpose(2,1), target) of pcdseg.py:177-178 on rows x [rows, C] (the reference feeds the
 // network's log-probabilities, so CrossEntropyLoss normalises them once more): loss = mean_i (lse(x_i) - x_i[t_i]);
-// dx[i,c] = (softmax(x_i)[c] - [c == t_i]) * grad_scale / rows.  One row per thread; loss summed in fp64.
+// dx[i,c] = (softmax(x_i)[c] - [c == t_i]) * grad_scale / n.  Rows labelled IGNORE_INDEX (CrossEntropyLoss's default
+// ignore_index) add nothing to the loss, get a zero gradient and are not counted in n, the number of the other rows;
+// n is counted on the device by label_count_kernel first (so the call needs no host synchronisation), and with every
+// row ignored the loss is 0/0 = NaN, as in torch.  One row per thread; loss summed in fp64.
+constexpr int64_t IGNORE_INDEX = -100;
+
+__global__ void __launch_bounds__(256)
+label_count_kernel(const int64_t* __restrict__ target, int64_t rows, double* __restrict__ count) {
+    int local = 0;
+    for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < rows; r += (int64_t)gridDim.x * blockDim.x)
+        local += target[r] != IGNORE_INDEX;
+    local = __reduce_add_sync(0xffffffffu, local);
+    if ((threadIdx.x & 31) == 0 && local) atomicAdd(count, (double)local);
+}
+
 __global__ void __launch_bounds__(256)
 cross_entropy_kernel(const float* __restrict__ x, int64_t ldx, const int64_t* __restrict__ target, int64_t rows, int C,
-                     double* __restrict__ loss_sum, float* __restrict__ dx, int64_t lddx, float grad_scale) {
+                     double* __restrict__ loss_sum, const double* __restrict__ count, float* __restrict__ dx, int64_t lddx,
+                     float grad_scale) {
     __shared__ double red[8];
     double local = 0.0;
+    const float k = grad_scale / (float)*count;
     for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < rows; r += (int64_t)gridDim.x * blockDim.x) {
+        if (target[r] == IGNORE_INDEX) {
+            if (dx)
+                for (int c = 0; c < C; ++c) dx[r * lddx + c] = 0.0f;
+            continue;
+        }
         const float* __restrict__ xr = x + r * ldx;
         float m = -CUDART_INF_F;
         for (int c = 0; c < C; ++c) m = fmaxf(m, xr[c]);
         float s = 0.0f;
         for (int c = 0; c < C; ++c) s += expf(xr[c] - m);
-        const float lse = m + logf(s);
+        const float ls = logf(s);
         const int64_t t = target[r];
         if (t < 0 || t >= C) {
-            // nn.CrossEntropyLoss raises on a label outside [0, C); an asynchronous kernel cannot, so the loss and this
+            // nn.CrossEntropyLoss raises on any other label outside [0, C); an asynchronous kernel cannot, so the loss and this
             // row's gradient are poisoned with NaN instead of being computed against a clamped label
             local += (double)CUDART_NAN_F;
             if (dx)
                 for (int c = 0; c < C; ++c) dx[r * lddx + c] = CUDART_NAN_F;
             continue;
         }
-        local += (double)(lse - xr[t]);
+        // lse(x) = m + log(s) is not formed: at |m| ~ 1e4 its float32 rounding (1e-3) would be the error of every softmax
+        // entry.  The loss is (m - x[t]) + log(s), the softmax exp(x - m) / s.
+        local += (double)((m - xr[t]) + ls);
         if (dx) {
-            const float k = grad_scale / (float)rows;
-            for (int c = 0; c < C; ++c) dx[r * lddx + c] = (expf(xr[c] - lse) - (c == (int)t ? 1.0f : 0.0f)) * k;
+            const float inv_s = 1.0f / s;
+            for (int c = 0; c < C; ++c) dx[r * lddx + c] = (expf(xr[c] - m) * inv_s - (c == (int)t ? 1.0f : 0.0f)) * k;
         }
     }
 #pragma unroll
@@ -492,8 +515,9 @@ cross_entropy_kernel(const float* __restrict__ x, int64_t ldx, const int64_t* __
     }
 }
 
-__global__ void loss_finalize_kernel(const double* __restrict__ loss_sum, int64_t rows, float* __restrict__ loss) {
-    *loss = (float)(*loss_sum / (double)rows);
+__global__ void loss_finalize_kernel(const double* __restrict__ loss_sum, const double* __restrict__ count,
+                                     float* __restrict__ loss) {
+    *loss = (float)(*loss_sum / *count);
 }
 
 // log_softmax backward: dx = dy - exp(y) * sum_c dy   (y = the log-probabilities)
@@ -767,13 +791,14 @@ PN_EXPORT int pn_cross_entropy_f32(const float* x, int64_t ldx, const int64_t* t
     PN_REQUIRE(x && target && loss_sum && loss, PN_ERR_BAD_ARG, "pn_cross_entropy_f32: null pointer");
     PN_REQUIRE(rows > 0 && C > 0 && ldx >= C && (!dx || lddx >= C), PN_ERR_BAD_ARG, "pn_cross_entropy_f32: bad shape");
     cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = cudaMemsetAsync(loss_sum, 0, sizeof(double), st);
+    cudaError_t e = cudaMemsetAsync(loss_sum, 0, 2 * sizeof(double), st);
     if (e != cudaSuccess) {
         set_error("pn_cross_entropy_f32: %s", cudaGetErrorString(e));
         return (int)e;
     }
-    cross_entropy_kernel<<<ew_blocks(rows, 256), 256, 0, st>>>(x, ldx, target, rows, C, loss_sum, dx, lddx, grad_scale);
-    loss_finalize_kernel<<<1, 1, 0, st>>>(loss_sum, rows, loss);
+    label_count_kernel<<<ew_blocks(rows, 256), 256, 0, st>>>(target, rows, loss_sum + 1);
+    cross_entropy_kernel<<<ew_blocks(rows, 256), 256, 0, st>>>(x, ldx, target, rows, C, loss_sum, loss_sum + 1, dx, lddx, grad_scale);
+    loss_finalize_kernel<<<1, 1, 0, st>>>(loss_sum, loss_sum + 1, loss);
     return finish_launch("pn_cross_entropy_f32");
 }
 

@@ -1047,13 +1047,14 @@ def dropout(x: torch.Tensor, p: float, seed_offset: Optional[torch.Tensor] = Non
 
 
 def cross_entropy(x: torch.Tensor, target: torch.Tensor, want_grad: bool = True, grad_scale: float = 1.0):
-    """nn.CrossEntropyLoss() over rows x [rows, C], target [rows] -> (loss 0-d tensor, dx or None)."""
+    """nn.CrossEntropyLoss() over rows x [rows, C], target [rows] -> (loss 0-d tensor, dx or None).  Label -100 is
+    ignored (its default ignore_index): left out of the mean, zero gradient."""
     x = _rowmat(x, "x")
     target = _i64(target.reshape(-1), "target")
     rows, Cc = x.shape
     if target.numel() != rows:
         raise ValueError("target must hold one label per row")
-    scratch = torch.empty((1,), dtype=torch.float64, device=x.device)
+    scratch = torch.empty((2,), dtype=torch.float64, device=x.device)
     loss = torch.empty((), dtype=torch.float32, device=x.device)
     dx = torch.empty((rows, Cc), dtype=torch.float32, device=x.device) if want_grad else None
     with _on_device(x):

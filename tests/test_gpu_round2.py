@@ -302,8 +302,9 @@ def test_two_threads_two_precisions(dev, ckpt_path):
 
 
 def test_cross_entropy_poisons_out_of_range_labels(dev):
-    """nn.CrossEntropyLoss raises on a label outside [0, C); the asynchronous kernel returns NaN instead of silently
-    training on a clamped label (round-1 advisor finding)."""
+    """nn.CrossEntropyLoss raises on a label outside [0, C) other than its ignore_index -100; the asynchronous kernel
+    returns NaN instead of silently training on a clamped label (round-1 advisor finding): labels C (19 here) and -1.
+    Label -100 is ignored, as torch does (tests/test_gpu_train_edges.py compares that case with torch)."""
     from pointnet12_b200 import ops
 
     x = torch.randn(64, 19, device=dev)
@@ -314,6 +315,12 @@ def test_cross_entropy_poisons_out_of_range_labels(dev):
     t[7] = 19
     loss, dx = ops.cross_entropy(x, t)
     assert bool(torch.isnan(loss)) and bool(torch.isnan(dx[7]).all()) and bool(torch.isfinite(dx[8]).all())
+    t[7] = -1
+    loss, dx = ops.cross_entropy(x, t)
+    assert bool(torch.isnan(loss)) and bool(torch.isnan(dx[7]).all()) and bool(torch.isfinite(dx[8]).all())
+    t[7] = -100
+    loss, dx = ops.cross_entropy(x, t)
+    assert bool(torch.isfinite(loss)) and not bool(dx[7].any()) and bool(torch.isfinite(dx).all())
 
 
 def test_labels_output_mode(dev, ckpt_path):
