@@ -70,4 +70,47 @@ __device__ __forceinline__ float sqdist_diff(float px, float py, float pz, float
     return __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
 }
 
+// Packed fp32 pairs: add / mul / fma .rn.f32x2 (FADD2 / FMUL2 / FFMA2) round each half exactly like the scalar .rn form,
+// two operations per instruction.  ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 (it does not for the scalar
+// .rn forms), which changes the rounding: a product that feeds a sum must be unpacked and summed with the scalar _rn
+// intrinsics, unless the rounding wanted is that of the fma (as in sqdist_expand).
+__device__ __forceinline__ unsigned long long pack2(float lo, float hi) {
+    unsigned long long r;
+    asm("mov.b64 %0, {%1,%2};" : "=l"(r) : "f"(lo), "f"(hi));
+    return r;
+}
+__device__ __forceinline__ void unpack2(unsigned long long v, float& lo, float& hi) {
+    asm("mov.b64 {%0,%1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
+}
+__device__ __forceinline__ unsigned long long add2(unsigned long long a, unsigned long long b) {
+    unsigned long long r;
+    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+    return r;
+}
+__device__ __forceinline__ unsigned long long mul2(unsigned long long a, unsigned long long b) {
+    unsigned long long r;
+    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
+    return r;
+}
+__device__ __forceinline__ unsigned long long fma2(unsigned long long a, unsigned long long b, unsigned long long c) {
+    unsigned long long r;
+    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
+    return r;
+}
+
+// sqdist_diff for two points at once (8 arithmetic instructions instead of 16); n* = the negated centroid broadcast to
+// both halves (p + (-c) == p - c)
+__device__ __forceinline__ void sqdist_diff2(unsigned long long px, unsigned long long py, unsigned long long pz,
+                                             unsigned long long ncx, unsigned long long ncy, unsigned long long ncz, float& d0,
+                                             float& d1) {
+    const unsigned long long dx = add2(px, ncx), dy = add2(py, ncy), dz = add2(pz, ncz);
+    const unsigned long long xx = mul2(dx, dx), yy = mul2(dy, dy), zz = mul2(dz, dz);
+    float x0, x1, y0, y1, z0, z1;      // the sums on the unpacked halves: packed, they would contract into FFMA2
+    unpack2(xx, x0, x1);
+    unpack2(yy, y0, y1);
+    unpack2(zz, z0, z1);
+    d0 = __fadd_rn(__fadd_rn(x0, y0), z0);
+    d1 = __fadd_rn(__fadd_rn(x1, y1), z1);
+}
+
 }  // namespace pn

@@ -25,6 +25,7 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -41,7 +42,8 @@ struct __align__(32) FpsMsg {
 
 constexpr int kFpsSmemHeader = 2 * kMaxCluster * (int)sizeof(FpsMsg) + 2 * 32 * (int)sizeof(uint2) + 64;   // + two mbarriers (async exchange)
 
-__device__ __forceinline__ unsigned map_to_cta_u32(unsigned addr, unsigned rank) {
+// the address of the same shared-memory location in CTA `rank` of the cluster
+__device__ __forceinline__ unsigned map_to_cta(unsigned addr, unsigned rank) {
     unsigned r;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
     return r;
@@ -91,9 +93,9 @@ fps_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t sC, in
     float cx = p[(int64_t)far * sN], cy = p[(int64_t)far * sN + sC], cz = p[(int64_t)far * sN + 2 * sC];
     if constexpr (CLUSTER) {
         if (async_x && tid == 0) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(&xbar[0])), "r"(1));
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(&xbar[1])), "r"(1));
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+            tc::mbar_init(tc::smem_u32(&xbar[0]), 1);
+            tc::mbar_init(tc::smem_u32(&xbar[1]), 1);
+            tc::mbar_init_fence();
         }
         __syncthreads();
         cg::this_cluster().sync();  // peers must be resident (and their barriers initialised) before DSMEM stores
@@ -146,14 +148,13 @@ fps_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t sC, in
             if (async_x) {
                 // CTA winner -> every CTA of the cluster with st.async, completion counted in bytes on the RECEIVER's mbarrier:
                 // a one-way DSMEM store instead of store + barrier.cluster round trip (1.76 -> ~0.8 us per iteration at 16 CTAs)
-                const unsigned l_bar = (unsigned)__cvta_generic_to_shared(&xbar[par]);
-                if (tid == 0)
-                    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(l_bar), "r"((unsigned)(CL * 20u)) : "memory");
+                const unsigned l_bar = tc::smem_u32(&xbar[par]);
+                if (tid == 0) tc::mbar_arrive_expect_tx(l_bar, CL * 20u);
                 if (warp == 0 && lane < (int)CL) {
                     const unsigned long long key = ((unsigned long long)bm << 32) | (unsigned long long)(~bi);
                     const int li = bi == kNoIndex ? 0 : (int)bi - base;
-                    const unsigned r_slot = map_to_cta_u32((unsigned)__cvta_generic_to_shared(&cl_slots[par * kMaxCluster + rank]), lane);
-                    const unsigned r_bar = map_to_cta_u32(l_bar, lane);
+                    const unsigned r_slot = map_to_cta(tc::smem_u32(&cl_slots[par * kMaxCluster + rank]), lane);
+                    const unsigned r_bar = map_to_cta(l_bar, lane);
                     asm volatile(
                         "st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(r_slot),
                         "r"((unsigned)(key & 0xFFFFFFFFull)), "r"((unsigned)(key >> 32)), "r"(__float_as_uint(sx[li])),
@@ -163,12 +164,7 @@ fps_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t sC, in
                                  "r"(__float_as_uint(sz[li])), "r"(r_bar)
                                  : "memory");
                 }
-                unsigned done = 0;
-                const unsigned parity = (unsigned)((i >> 1) & 1);
-                while (!done) {
-                    asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                                 : "=r"(done) : "r"(l_bar), "r"(parity) : "memory");
-                }
+                tc::mbar_wait(l_bar, (unsigned)((i >> 1) & 1));
             } else {
             if (warp == 0 && lane < (int)CL) {
                 FpsMsg m;
@@ -214,54 +210,6 @@ struct __align__(32) FpsSlot {
 constexpr int kMaxSlots = 64;
 constexpr int kSlotBytes = 20;  // bytes actually transmitted per slot (v4.b32 + b32)
 constexpr int kAsyncSmemHeader = 64 + 2 * kMaxSlots * (int)sizeof(FpsSlot);
-
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ unsigned map_to_cta(unsigned addr, unsigned rank) {
-    unsigned r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
-    unsigned done = 0;
-    while (!done) {
-        asm volatile(
-            "{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-            : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    }
-}
-
-// Packed fp32 pairs (FADD2 / FMUL2: two IEEE-rounded fp32 operations per instruction, bit-identical to the scalar
-// sequence): the distance update of two points costs 8 arithmetic instructions instead of 16.
-__device__ __forceinline__ unsigned long long pack2(float lo, float hi) {
-    unsigned long long r;
-    asm("mov.b64 %0, {%1,%2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-__device__ __forceinline__ unsigned long long add2(unsigned long long a, unsigned long long b) {
-    unsigned long long r;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-__device__ __forceinline__ unsigned long long mul2(unsigned long long a, unsigned long long b) {
-    unsigned long long r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-// ((dx*dx + dy*dy) + dz*dz) for two points at once; n* = the negated centroid broadcast to both halves (p + (-c) == p - c)
-__device__ __forceinline__ void sqdist_diff2(unsigned long long px, unsigned long long py, unsigned long long pz,
-                                             unsigned long long ncx, unsigned long long ncy, unsigned long long ncz, float& d0,
-                                             float& d1) {
-    const unsigned long long dx = add2(px, ncx), dy = add2(py, ncy), dz = add2(pz, ncz);
-    // ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 (it does not for the scalar .rn forms), which would
-    // change the rounding; the sums are therefore taken on the unpacked halves with the scalar _rn intrinsics.
-    const unsigned long long xx = mul2(dx, dx), yy = mul2(dy, dy), zz = mul2(dz, dz);
-    float x0, x1, y0, y1, z0, z1;
-    asm("mov.b64 {%0,%1}, %2;" : "=f"(x0), "=f"(x1) : "l"(xx));
-    asm("mov.b64 {%0,%1}, %2;" : "=f"(y0), "=f"(y1) : "l"(yy));
-    asm("mov.b64 {%0,%1}, %2;" : "=f"(z0), "=f"(z1) : "l"(zz));
-    d0 = __fadd_rn(__fadd_rn(x0, y0), z0);
-    d1 = __fadd_rn(__fadd_rn(x1, y1), z1);
-}
 
 // ZT: every CTA also keeps the z coordinate of the WHOLE cloud in shared memory (4 N bytes), so a winner travels as
 // one 16-byte st.async (distance, index, x, y) instead of two (z is looked up locally by index): half the remote
@@ -317,9 +265,9 @@ fps_async_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t 
         for (int i = tid; i < N; i += THREADS) zt[i] = p[(int64_t)i * sN + 2 * sC];
     }
     if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(&mbar[0])), "r"(1));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(&mbar[1])), "r"(1));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tc::mbar_init(tc::smem_u32(&mbar[0]), 1);
+        tc::mbar_init(tc::smem_u32(&mbar[1]), 1);
+        tc::mbar_init_fence();
     }
     int far = (int)start[b];
     far = min(max(far, 0), N - 1);
@@ -330,9 +278,9 @@ fps_async_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t 
     // remote addresses this lane sends to (lane < CL: CTA `lane`); parity 1 lives at a fixed offset
     const unsigned my_slot = rank * NW + warp;
     const unsigned dst_cta = lane < (int)CL ? lane : 0;
-    const unsigned r_slot0 = map_to_cta(smem_u32(&slots[my_slot]), dst_cta);
-    const unsigned r_bar0 = map_to_cta(smem_u32(&mbar[0]), dst_cta);
-    const unsigned l_bar0 = smem_u32(&mbar[0]);
+    const unsigned r_slot0 = map_to_cta(tc::smem_u32(&slots[my_slot]), dst_cta);
+    const unsigned r_bar0 = map_to_cta(tc::smem_u32(&mbar[0]), dst_cta);
+    const unsigned l_bar0 = tc::smem_u32(&mbar[0]);
     constexpr unsigned kParSlotOff = kMaxSlots * sizeof(FpsSlot), kParBarOff = sizeof(unsigned long long);
 
     int64_t* __restrict__ o = out + (int64_t)b * npoint;
@@ -346,9 +294,7 @@ fps_async_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t 
         }
         if (i == npoint - 1) break;  // the last arg-max would never be used
         if (tid == 0)
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(l_bar0 + par * kParBarOff),
-                         "r"((unsigned)(nslot * (ZT ? 16 : kSlotBytes)))
-                         : "memory");
+            tc::mbar_arrive_expect_tx(l_bar0 + par * kParBarOff, (unsigned)(nslot * (ZT ? 16 : kSlotBytes)));
         float bv = -1.0f;
         int bk = 0;
         const unsigned long long ncx = pack2(-cx, -cx), ncy = pack2(-cy, -cy), ncz = pack2(-cz, -cz);
@@ -388,7 +334,7 @@ fps_async_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t 
                              : "memory");
             }
         }
-        mbar_wait(l_bar0 + par * kParBarOff, (unsigned)((i >> 1) & 1));
+        tc::mbar_wait(l_bar0 + par * kParBarOff, (unsigned)((i >> 1) & 1));
         // reduce the CL*NW slots: one or two per lane
         unsigned sv = 0u, si = kNoIndex;
         float px = 0.f, py = 0.f, pz = 0.f;
@@ -488,9 +434,9 @@ fps_pruned_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t
         }
     const bool warp_empty = g0 >= N;
     if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(&mbar[0])), "r"(1));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(&mbar[1])), "r"(1));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tc::mbar_init(tc::smem_u32(&mbar[0]), 1);
+        tc::mbar_init(tc::smem_u32(&mbar[1]), 1);
+        tc::mbar_init_fence();
     }
     int far = (int)start[b];
     far = min(max(far, 0), N - 1);
@@ -500,9 +446,9 @@ fps_pruned_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t
 
     const unsigned my_slot = rank * NW + warp;
     const unsigned dst_cta = lane < (int)CL ? lane : 0;
-    const unsigned r_slot0 = map_to_cta(smem_u32(&slots[my_slot]), dst_cta);
-    const unsigned r_bar0 = map_to_cta(smem_u32(&mbar[0]), dst_cta);
-    const unsigned l_bar0 = smem_u32(&mbar[0]);
+    const unsigned r_slot0 = map_to_cta(tc::smem_u32(&slots[my_slot]), dst_cta);
+    const unsigned r_bar0 = map_to_cta(tc::smem_u32(&mbar[0]), dst_cta);
+    const unsigned l_bar0 = tc::smem_u32(&mbar[0]);
     constexpr unsigned kParSlotOff = kMaxSlots * sizeof(FpsSlot), kParBarOff = sizeof(unsigned long long);
 
     // the warp's cached winner: (distance bits, original index, coordinates); valid while no distance of the warp changes
@@ -519,9 +465,7 @@ fps_pruned_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t
         }
         if (i == npoint - 1) break;  // the last arg-max would never be used
         if (tid == 0)
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(l_bar0 + par * kParBarOff),
-                         "r"((unsigned)(nslot * kSlotBytes))
-                         : "memory");
+            tc::mbar_arrive_expect_tx(l_bar0 + par * kParBarOff, (unsigned)(nslot * kSlotBytes));
         // lower bound of the distance from the new centroid to any point of the warp's box, in the distance's own rounding
         const float ddx = fmaxf(fmaxf(__fsub_rn(lo[0], cx), __fsub_rn(cx, hi[0])), 0.0f);
         const float ddy = fmaxf(fmaxf(__fsub_rn(lo[1], cy), __fsub_rn(cy, hi[1])), 0.0f);
@@ -580,7 +524,7 @@ fps_pruned_kernel(const float* __restrict__ xyz, int64_t sB, int64_t sN, int64_t
                          "r"(__float_as_uint(wz)), "r"(r_bar)
                          : "memory");
         }
-        mbar_wait(l_bar0 + par * kParBarOff, (unsigned)((i >> 1) & 1));
+        tc::mbar_wait(l_bar0 + par * kParBarOff, (unsigned)((i >> 1) & 1));
         // reduce the CL*NW slots: one or two per lane
         unsigned sv = 0u, si = kNoIndex;
         float px = 0.f, py = 0.f, pz = 0.f;

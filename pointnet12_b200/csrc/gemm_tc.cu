@@ -21,10 +21,10 @@
 // 128 x cout in TMEM; the four EPILOGUE warps read a finished accumulator back (thread = row), add the bias, store y and
 // reduce the column sums with a shuffle butterfly in fp64 -- while the producers and the tensor core work on the next tile.
 // W can be given transposed (w[k, n]): the input-gradient GEMM dx = dy W of the backward pass reads W that way.
-#include <cuda_bf16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace pn {
 namespace gemm {
@@ -35,96 +35,6 @@ constexpr int A_IMG = TM * KC * 2;            // one bf16 image of a 128 x 32 ch
 constexpr int A_STAGE = 2 * A_IMG;            // hi + lo
 constexpr int W_MAX_BYTES = 128 * 1024;       // resident weights (hi + lo)
 constexpr int PF = 6;                         // L2 prefetch distance of the operand stream, in 32-column chunks
-
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(unsigned bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// PN12_GEMM_SPIN (compile-time experiment): busy-poll with test_wait instead of the potentially suspending try_wait.
-// Measured on B200: no difference (33.2 vs 33.0 us per 128 x 128 layer), so the suspending wait stays.
-#ifndef PN12_GEMM_SPIN
-#define PN12_GEMM_SPIN 0
-#endif
-__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
-    unsigned done = 0;
-    while (!done) {
-#if PN12_GEMM_SPIN
-        asm volatile("{ .reg .pred p; mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-#else
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-#endif
-    }
-}
-__device__ __forceinline__ bool elect() {
-    unsigned p;
-    asm volatile("{ .reg .pred q; elect.sync _|q, 0xffffffff; selp.u32 %0, 1, 0, q; }" : "=r"(p));
-    return p != 0;
-}
-__device__ __forceinline__ void commit(unsigned bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void ld32(unsigned taddr, unsigned (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// 8 consecutive k of one row -> 8 bf16 hi + 8 bf16 lo, one 16-byte store each (a core-matrix row)
-__device__ __forceinline__ void store_split8(unsigned char* hi_img, unsigned char* lo_img, unsigned off, const float (&v)[8]) {
-    unsigned h[4], l[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const __nv_bfloat162 hb2 = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);       // .x (low half) = even k
-        const unsigned hb = *reinterpret_cast<const unsigned*>(&hb2);
-        const float r0 = v[2 * j] - __uint_as_float(hb << 16);
-        const float r1 = v[2 * j + 1] - __uint_as_float(hb & 0xFFFF0000u);
-        const __nv_bfloat162 lb2 = __floats2bfloat162_rn(r0, r1);
-        h[j] = hb;
-        l[j] = *reinterpret_cast<const unsigned*>(&lb2);
-    }
-    *reinterpret_cast<uint4*>(hi_img + off) = make_uint4(h[0], h[1], h[2], h[3]);
-    *reinterpret_cast<uint4*>(lo_img + off) = make_uint4(l[0], l[1], l[2], l[3]);
-}
-
-// Sum over the 32 lanes of a warp for 32 columns held one row per lane: a butterfly in which every step halves the
-// columns a lane is responsible for (31 shuffles).  Afterwards lane j holds the sum of column j.
-template <int W>
-__device__ __forceinline__ void colsum_step_f(float (&v)[32], int lane) {
-    if constexpr (W >= 4) {
-        const bool up = (lane & W) != 0;
-#pragma unroll
-        for (int i = 0; i < W; ++i) {
-            const float send = up ? v[i] : v[i + W];
-            const float keep = up ? v[i + W] : v[i];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, W);
-        }
-        colsum_step_f<W / 2>(v, lane);
-    }
-}
-template <int W>
-__device__ __forceinline__ void colsum_step(double (&v)[32], int lane) {
-    if constexpr (W >= 1) {
-        const bool up = (lane & W) != 0;
-#pragma unroll
-        for (int i = 0; i < W; ++i) {
-            const double send = up ? v[i] : v[i + W];
-            const double keep = up ? v[i + W] : v[i];
-            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, W);
-        }
-        colsum_step<W / 2>(v, lane);
-    }
-}
 
 struct Args {
     const float* x; int64_t ldx; int64_t rows; int cin;
@@ -142,8 +52,8 @@ struct Args {
 // [n_pad x 32] then the lo image, K-major core matrices.  Done ONCE per GEMM into a scratch buffer; every CTA of the GEMM
 // then fetches the image with bulk copies.  (Converting inside the GEMM cost ~18 us per CTA for a 128 x 128 layer: 296 CTAs
 // gathering the same 64 KB with scattered 4-byte loads.)
-__global__ void train_pack_kernel(const float* __restrict__ w, int w_transposed, int cin, int cout, int k_pad, int n_pad,
-                                  unsigned char* __restrict__ out) {
+__device__ __forceinline__ void pack_weights(const float* __restrict__ w, int w_transposed, int cin, int cout, int k_pad, int n_pad,
+                                             unsigned char* __restrict__ out) {
     const int kblocks = k_pad / 8;
     const unsigned w_chunk_bytes = (unsigned)n_pad * KC * 4;
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n_pad * kblocks; e += gridDim.x * blockDim.x) {
@@ -160,33 +70,21 @@ __global__ void train_pack_kernel(const float* __restrict__ w, int w_transposed,
         const int c = kb / (KC / 8), kbi = kb % (KC / 8);
         unsigned char* img = out + (size_t)c * w_chunk_bytes;
         const unsigned off = (unsigned)(n >> 3) * (KC / 8) * 128u + (unsigned)kbi * 128u + (unsigned)(n & 7) * 16u;
-        store_split8(img, img + (size_t)n_pad * KC * 2, off, v);
+        tc::store_split8(img, img + (size_t)n_pad * KC * 2, off, v);
     }
+}
+
+__global__ void train_pack_kernel(const float* __restrict__ w, int w_transposed, int cin, int cout, int k_pad, int n_pad,
+                                  unsigned char* __restrict__ out) {
+    pack_weights(w, w_transposed, cin, cout, k_pad, n_pad, out);
 }
 
 // The same for MANY layers in one launch (blockIdx.y = item): all weights of a network, both orientations, packed once per
 // training iteration instead of once per GEMM call.
 __global__ void train_pack_many_kernel(const pn_train_pack_item* __restrict__ items) {
     const pn_train_pack_item it = items[blockIdx.y];
-    const int k_pad = (it.cin + KC - 1) / KC * KC, n_pad = (it.cout + 31) / 32 * 32;
-    const int kblocks = k_pad / 8;
-    const unsigned w_chunk_bytes = (unsigned)n_pad * KC * 4;
-    unsigned char* out = static_cast<unsigned char*>(it.out);
-    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n_pad * kblocks; e += gridDim.x * blockDim.x) {
-        const int n = it.transposed ? e % n_pad : e / kblocks, kb = it.transposed ? e / n_pad : e % kblocks;
-        float v[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            const int k = kb * 8 + j;
-            float t = 0.0f;
-            if (n < it.cout && k < it.cin) t = it.transposed ? __ldg(it.w + (int64_t)k * it.cout + n) : __ldg(it.w + (int64_t)n * it.cin + k);
-            v[j] = t;
-        }
-        const int c = kb / (KC / 8), kbi = kb % (KC / 8);
-        unsigned char* img = out + (size_t)c * w_chunk_bytes;
-        const unsigned off = (unsigned)(n >> 3) * (KC / 8) * 128u + (unsigned)kbi * 128u + (unsigned)(n & 7) * 16u;
-        store_split8(img, img + (size_t)n_pad * KC * 2, off, v);
-    }
+    pack_weights(it.w, it.transposed, it.cin, it.cout, (it.cin + KC - 1) / KC * KC, (it.cout + 31) / 32 * 32,
+                 static_cast<unsigned char*>(it.out));
 }
 
 __global__ void __launch_bounds__(THREADS, 2)
@@ -206,37 +104,26 @@ train_gemm_kernel(const Args a) {
     float* pc = bias_s + a.n_pad;                                                               // [4][n_pad]: scale, shift, mean, invstd of the layer below (forward: [0] = statistics pivots)
     float* stg_all = pc + 4 * a.n_pad;                                                          // [4 epilogue warps][32 rows][20]: output staging
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const unsigned bar_full = smem_u32(bars), bar_empty = smem_u32(bars + NS_MAX), bar_accf = smem_u32(bars + 2 * NS_MAX),
-                   bar_acce = smem_u32(bars + 3 * NS_MAX), bar_w = smem_u32(bars + 4 * NS_MAX);
+    const unsigned bar_full = tc::smem_u32(bars), bar_empty = tc::smem_u32(bars + NS_MAX), bar_accf = tc::smem_u32(bars + 2 * NS_MAX),
+                   bar_acce = tc::smem_u32(bars + 3 * NS_MAX), bar_w = tc::smem_u32(bars + 4 * NS_MAX);
 
     unsigned tmem_cols = 32;
     while ((int)tmem_cols < NA * a.n_pad) tmem_cols <<= 1;      // NA accumulators: the MMAs of the next tiles overlap the epilogue of tile i
     if (tid == 0) {
         for (int s = 0; s < NS; ++s) {
-            mbar_init(bar_full + 8 * s, THREADS / 2);
-            mbar_init(bar_empty + 8 * s, 1);
+            tc::mbar_init(bar_full + 8 * s, THREADS / 2);
+            tc::mbar_init(bar_empty + 8 * s, 1);
         }
         for (int b = 0; b < NA; ++b) {
-            mbar_init(bar_accf + 8 * b, 1);
-            mbar_init(bar_acce + 8 * b, THREADS / 2);
+            tc::mbar_init(bar_accf + 8 * b, 1);
+            tc::mbar_init(bar_acce + 8 * b, THREADS / 2);
         }
-        mbar_init(bar_w, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tc::mbar_init(bar_w, 1);
+        tc::mbar_init_fence();
         // the packed weights: bulk copies straight into their resident place, completion counted in bytes on bar_w
-        const unsigned wbytes = (unsigned)kch * w_chunk_bytes;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_w), "r"(wbytes) : "memory");
-        for (unsigned off = 0; off < wbytes; off += 32768u) {
-            const unsigned n = wbytes - off < 32768u ? wbytes - off : 32768u;
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             smem_u32(w_smem) + off),
-                         "l"(a.w_packed + off), "r"(n), "r"(bar_w)
-                         : "memory");
-        }
+        tc::bulk_load_pieces(tc::smem_u32(w_smem), a.w_packed, (unsigned)kch * w_chunk_bytes, bar_w);
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(tmem_cols));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    if (warp == 0) tc::tmem_alloc(tmem_slot, tmem_cols);
     const int64_t tiles = (a.rows + TM - 1) / TM;
     const int64_t my_tiles = blockIdx.x < tiles ? (tiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
     // the producers' first chunk is requested BEFORE the weight conversion, which then hides its latency
@@ -288,10 +175,10 @@ train_gemm_kernel(const Args a) {
             tf[a.k_pad + k] = k < a.cin ? __ldg(a.in_shift + k) : 0.0f;
         }
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc::fence_proxy_async();
+    tc::fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc::fence_after();
     const unsigned tbase = *tmem_slot;
 
     if (warp < 4) {
@@ -299,9 +186,8 @@ train_gemm_kernel(const Args a) {
         const int64_t total_chunks = my_tiles * kch;
         const int m = tid;
         const unsigned row_off = (unsigned)(m >> 3) * (KC / 8) * 128u + (unsigned)(m & 7) * 16u;
-        const unsigned idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(a.n_pad >> 3) << 17) | ((unsigned)(TM >> 4) << 24);
-        const unsigned long long dbase = ((unsigned long long)((128u >> 4) & 0x3FFF) << 16) |
-                                         ((unsigned long long)((((unsigned)KC / 8) * 128u >> 4) & 0x3FFF) << 32) | (1ull << 46);
+        const unsigned idesc = tc::idesc_bf16_f32(TM, a.n_pad);
+        const unsigned long long dbase = tc::sdesc_base((KC / 8) * 128u);
         for (int64_t gc = 0; gc < total_chunks; ++gc) {
             const int64_t it = gc / kch;
             const int c = (int)(gc - it * kch);
@@ -336,43 +222,33 @@ train_gemm_kernel(const Args a) {
                     cur[4 * i + 2] = row_ok ? t2 : 0.0f; cur[4 * i + 3] = row_ok ? t3 : 0.0f;
                 }
             }
-            if (gc >= NS) mbar_wait(bar_empty + 8 * s, (use - 1) & 1);
+            if (gc >= NS) tc::mbar_wait(bar_empty + 8 * s, (use - 1) & 1);
             unsigned char* st = a_smem + s * A_STAGE;
 #pragma unroll
             for (int kb = 0; kb < ((a.debug & 4) ? 0 : KC / 8); ++kb) {
                 float v8[8];
 #pragma unroll
                 for (int j = 0; j < 8; ++j) v8[j] = cur[kb * 8 + j];
-                store_split8(st, st + A_IMG, row_off + (unsigned)kb * 128u, v8);
+                tc::store_split8(st, st + A_IMG, row_off + (unsigned)kb * 128u, v8);
             }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            mbar_arrive(bar_full + 8 * s);
+            tc::fence_proxy_async();
+            tc::mbar_arrive(bar_full + 8 * s);
             if (warp == 0) {
                 const int b = (int)(it % NA);
-                mbar_wait(bar_full + 8 * s, use & 1);
-                if (gc == 0) mbar_wait(bar_w, 0);                      // the weight image has landed
-                if (c == 0 && it >= NA) mbar_wait(bar_acce + 8 * b, (unsigned)(it / NA - 1) & 1);   // epilogue of tile it-NA has read it
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                if (elect()) {
+                tc::mbar_wait(bar_full + 8 * s, use & 1);
+                if (gc == 0) tc::mbar_wait(bar_w, 0);                      // the weight image has landed
+                if (c == 0 && it >= NA) tc::mbar_wait(bar_acce + 8 * b, (unsigned)(it / NA - 1) & 1);   // epilogue of tile it-NA has read it
+                tc::fence_after();
+                if (tc::elect()) {
                     const unsigned acc = tbase + (unsigned)(b * a.n_pad);
-                    const unsigned a_hi = smem_u32(st), a_lo = a_hi + A_IMG;
-                    const unsigned b_hi = smem_u32(w_smem) + (unsigned)c * w_chunk_bytes, b_lo = b_hi + (unsigned)a.n_pad * KC * 2;
+                    const unsigned a_hi = tc::smem_u32(st), a_lo = a_hi + A_IMG;
+                    const unsigned b_hi = tc::smem_u32(w_smem) + (unsigned)c * w_chunk_bytes, b_lo = b_hi + (unsigned)a.n_pad * KC * 2;
 #pragma unroll
-                    for (int t = 0; t < ((a.debug & 1) ? 0 : KC / 16); ++t) {
-                        const unsigned long long dah = dbase | (unsigned long long)(((a_hi + t * 256) >> 4) & 0x3FFF);
-                        const unsigned long long dal = dbase | (unsigned long long)(((a_lo + t * 256) >> 4) & 0x3FFF);
-                        const unsigned long long dbh = dbase | (unsigned long long)(((b_hi + t * 256) >> 4) & 0x3FFF);
-                        const unsigned long long dbl = dbase | (unsigned long long)(((b_lo + t * 256) >> 4) & 0x3FFF);
-                        const unsigned acc0 = (c > 0 || t > 0) ? 1u : 0u;
-                        asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, q; }" ::"r"(acc),
-                                     "l"(dah), "l"(dbh), "r"(idesc), "r"(acc0) : "memory");
-                        asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, q; }" ::"r"(acc),
-                                     "l"(dah), "l"(dbl), "r"(idesc), "r"(1u) : "memory");
-                        asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, q; }" ::"r"(acc),
-                                     "l"(dal), "l"(dbh), "r"(idesc), "r"(1u) : "memory");
-                    }
-                    commit(bar_empty + 8 * s);
-                    if (c + 1 == kch) commit(bar_accf + 8 * b);
+                    for (int t = 0; t < ((a.debug & 1) ? 0 : KC / 16); ++t)
+                        tc::mma_bf16x3(acc, tc::sdesc(dbase, a_hi + t * 256), tc::sdesc(dbase, a_lo + t * 256),
+                                       tc::sdesc(dbase, b_hi + t * 256), tc::sdesc(dbase, b_lo + t * 256), idesc, (c > 0 || t > 0) ? 1u : 0u);
+                    tc::commit(bar_empty + 8 * s);
+                    if (c + 1 == kch) tc::commit(bar_accf + 8 * b);
                 }
                 __syncwarp();
             }
@@ -383,17 +259,17 @@ train_gemm_kernel(const Args a) {
         const int nch = a.n_pad / 32;
         for (int64_t it = 0; it < my_tiles; ++it) {
             const int b = (int)(it % NA);
-            mbar_wait(bar_accf + 8 * b, (unsigned)(it / NA) & 1);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tc::mbar_wait(bar_accf + 8 * b, (unsigned)(it / NA) & 1);
+            tc::fence_after();
             const int64_t row = (blockIdx.x + it * gridDim.x) * TM + q * 32 + lane;
             const bool row_ok = row < a.rows;
             for (int ch = 0; ch < nch; ++ch) {
                 const int col0 = ch * 32;
                 unsigned r[32];
-                if (!(a.debug & 16)) ld32(tbase + ((unsigned)(q * 32) << 16) + (unsigned)(b * a.n_pad + col0), r);
+                if (!(a.debug & 16)) tc::ld32(tbase + ((unsigned)(q * 32) << 16) + (unsigned)(b * a.n_pad + col0), r);
                 if (ch + 1 == nch) {                             // the accumulator has been read: the MMAs of tile it+2 may overwrite it
-                    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-                    mbar_arrive(bar_acce + 8 * b);
+                    tc::fence_before();
+                    tc::mbar_arrive(bar_acce + 8 * b);
                 }
                 float v[32];
                 const float4* b4 = reinterpret_cast<const float4*>(bias_s + col0);       // (a warp's lanes all want the same n)
@@ -497,13 +373,14 @@ train_gemm_kernel(const Args a) {
                             }
                         }
                     }
-                    colsum_step_f<16>(f1, lane);
-                    colsum_step_f<16>(f2, lane);
+                    const auto add = [](auto x, auto y) { return x + y; };
+                    tc::col_butterfly<16, 4>(f1, lane, add);
+                    tc::col_butterfly<16, 4>(f2, lane, add);
                     double d1[32], d2[32];
 #pragma unroll
                     for (int j = 0; j < 4; ++j) { d1[j] = (double)f1[j]; d2[j] = (double)f2[j]; }
-                    colsum_step<2>(d1, lane);
-                    colsum_step<2>(d2, lane);
+                    tc::col_butterfly<2, 1>(d1, lane, add);
+                    tc::col_butterfly<2, 1>(d2, lane, add);
                     // per-CTA accumulation in shared memory (four warps meet per column); one global atomic per column
                     // and CTA at the very end instead of one per tile
                     atomicAdd(&cta_sum[col0 + lane], d1[0]);
@@ -512,7 +389,7 @@ train_gemm_kernel(const Args a) {
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc::fence_before();
     __syncthreads();
     if (a.col_sum && my_tiles > 0) {
         // forward: the shifted sums of the CTA's rows back to plain sums, in fp64 (s2 + 2 p s1 + n p^2 loses nothing
@@ -530,7 +407,7 @@ train_gemm_kernel(const Args a) {
             atomicAdd(a.col_sumsq + n, s2);
         }
     }
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(tmem_cols));
+    if (warp == 0) tc::tmem_dealloc(tbase, tmem_cols);
 }
 
 static inline int round_up(int v, int m) { return (v + m - 1) / m * m; }

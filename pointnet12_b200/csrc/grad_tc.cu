@@ -16,9 +16,8 @@
 //     producers can refill it (3-stage ring);
 //   * at the end the accumulator is read back with tcgen05.ld and added to dW with fp32 atomics (the row slabs of one
 //     tile meet there); the producers of the first ci tile also carry the column sums of dy for db.
-#include <cuda_bf16.h>
-
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace pn {
 namespace gtc {
@@ -27,57 +26,6 @@ constexpr int TM = 128, TN = 128, KC = 32, NS = 3, THREADS = 256;
 constexpr int IMG = TM * KC * 2;              // one bf16 image of a 128 x 32 operand tile: 8 KB
 constexpr int STAGE = 4 * IMG;                // A hi, A lo, B hi, B lo
 constexpr int SMEM = NS * STAGE + 1024;
-
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(unsigned bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
-    unsigned done = 0;
-    while (!done) {
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    }
-}
-__device__ __forceinline__ bool elect() {
-    unsigned p;
-    asm volatile("{ .reg .pred q; elect.sync _|q, 0xffffffff; selp.u32 %0, 1, 0, q; }" : "=r"(p));
-    return p != 0;
-}
-__device__ __forceinline__ void commit(unsigned bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void ld32(unsigned taddr, unsigned (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// 8 consecutive rows (k) of one channel -> 8 bf16 hi + 8 bf16 lo, one 16-byte store each (a core-matrix row)
-__device__ __forceinline__ void store_split8(unsigned char* hi_img, unsigned char* lo_img, unsigned off, const float (&v)[8]) {
-    unsigned h[4], l[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const __nv_bfloat162 hb2 = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);       // .x (low half) = even k
-        const unsigned hb = *reinterpret_cast<const unsigned*>(&hb2);
-        const float r0 = v[2 * j] - __uint_as_float(hb << 16);
-        const float r1 = v[2 * j + 1] - __uint_as_float(hb & 0xFFFF0000u);
-        const __nv_bfloat162 lb2 = __floats2bfloat162_rn(r0, r1);
-        h[j] = hb;
-        l[j] = *reinterpret_cast<const unsigned*>(&lb2);
-    }
-    *reinterpret_cast<uint4*>(hi_img + off) = make_uint4(h[0], h[1], h[2], h[3]);
-    *reinterpret_cast<uint4*>(lo_img + off) = make_uint4(l[0], l[1], l[2], l[3]);
-}
 
 __global__ void __launch_bounds__(THREADS)
 grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ x, int64_t ldx, int64_t rows,
@@ -92,23 +40,20 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
     const int64_t r0 = (int64_t)blockIdx.z * rows_per_split;
     const int64_t r1 = min(rows, r0 + rows_per_split);
     const int chunks = (int)((r1 - r0 + KC - 1) / KC);
-    const unsigned bar_full = smem_u32(bars), bar_empty = smem_u32(bars + NS), bar_done = smem_u32(bars + 2 * NS);
+    const unsigned bar_full = tc::smem_u32(bars), bar_empty = tc::smem_u32(bars + NS), bar_done = tc::smem_u32(bars + 2 * NS);
 
     if (tid == 0) {
         for (int s = 0; s < NS; ++s) {
-            mbar_init(bar_full + 8 * s, THREADS);
-            mbar_init(bar_empty + 8 * s, 1);
+            tc::mbar_init(bar_full + 8 * s, THREADS);
+            tc::mbar_init(bar_empty + 8 * s, 1);
         }
-        mbar_init(bar_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tc::mbar_init(bar_done, 1);
+        tc::mbar_init_fence();
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(128));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (warp == 0) tc::tmem_alloc(tmem_slot, 128);
+    tc::fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc::fence_after();
     const unsigned tbase = *tmem_slot;
 
     // producer role of this thread: channel m of both operand tiles, k-blocks {half, half + 2} of every 32-row chunk
@@ -123,11 +68,8 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
     const bool x_tf = x_scale != nullptr;
     const float xs = (x_tf && b_ok) ? x_scale[ci0 + m] : 1.0f, xh = (x_tf && b_ok) ? x_shift[ci0 + m] : 0.0f;
     float bsum = 0.0f;
-    // instruction descriptor: D fp32, A / B bf16, both K-major, N = 128, M = 128
-    const unsigned idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(TN >> 3) << 17) | ((unsigned)(TM >> 4) << 24);
-    // shared-memory descriptor: K-direction core-matrix stride 128 B, 8-row group stride (KC/8)*128 B, version bit 46
-    const unsigned long long dbase = ((unsigned long long)((128u >> 4) & 0x3FFF) << 16) |
-                                     ((unsigned long long)((((unsigned)KC / 8) * 128u >> 4) & 0x3FFF) << 32) | (1ull << 46);
+    const unsigned idesc = tc::idesc_bf16_f32(TM, TN);
+    const unsigned long long dbase = tc::sdesc_base((KC / 8) * 128u);      // 8-row groups (KC / 8) * 128 B apart
 
     // register double buffer: the loads of chunk c+1 are in flight while chunk c is converted, stored and multiplied
     float va[2][8], vb[2][8];
@@ -166,7 +108,7 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
                     cb[q][j] = (b_ok && k0 + (half + 2 * q) * 8 + j < r1) ? t : 0.0f;
                 }
         }
-        if (c >= NS) mbar_wait(bar_empty + 8 * s, (use - 1) & 1);      // the MMAs that read this stage have completed
+        if (c >= NS) tc::mbar_wait(bar_empty + 8 * s, (use - 1) & 1);      // the MMAs that read this stage have completed
         unsigned char* st = smem + s * STAGE;
 #pragma unroll
         for (int q = 0; q < 2; ++q) {
@@ -175,47 +117,37 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
 #pragma unroll
                 for (int j = 0; j < 8; ++j) bsum += ca[q][j];
             }
-            store_split8(st, st + IMG, row_off + (unsigned)kb * 128u, ca[q]);
-            store_split8(st + 2 * IMG, st + 3 * IMG, row_off + (unsigned)kb * 128u, cb[q]);
+            tc::store_split8(st, st + IMG, row_off + (unsigned)kb * 128u, ca[q]);
+            tc::store_split8(st + 2 * IMG, st + 3 * IMG, row_off + (unsigned)kb * 128u, cb[q]);
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy stores -> visible to the MMA
-        mbar_arrive(bar_full + 8 * s);
+        tc::fence_proxy_async();
+        tc::mbar_arrive(bar_full + 8 * s);
         if (warp == 0) {
-            mbar_wait(bar_full + 8 * s, use & 1);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            if (elect()) {
-                const unsigned a_hi = smem_u32(st), a_lo = a_hi + IMG, b_hi = a_hi + 2 * IMG, b_lo = a_hi + 3 * IMG;
+            tc::mbar_wait(bar_full + 8 * s, use & 1);
+            tc::fence_after();
+            if (tc::elect()) {
+                const unsigned a_hi = tc::smem_u32(st), a_lo = a_hi + IMG, b_hi = a_hi + 2 * IMG, b_lo = a_hi + 3 * IMG;
 #pragma unroll
-                for (int t = 0; t < KC / 16; ++t) {
-                    const unsigned long long dah = dbase | (unsigned long long)(((a_hi + t * 256) >> 4) & 0x3FFF);
-                    const unsigned long long dal = dbase | (unsigned long long)(((a_lo + t * 256) >> 4) & 0x3FFF);
-                    const unsigned long long dbh = dbase | (unsigned long long)(((b_hi + t * 256) >> 4) & 0x3FFF);
-                    const unsigned long long dbl = dbase | (unsigned long long)(((b_lo + t * 256) >> 4) & 0x3FFF);
-                    const unsigned acc0 = (c > 0 || t > 0) ? 1u : 0u;
-                    asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, q; }" ::"r"(tbase),
-                                 "l"(dah), "l"(dbh), "r"(idesc), "r"(acc0) : "memory");
-                    asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, q; }" ::"r"(tbase),
-                                 "l"(dah), "l"(dbl), "r"(idesc), "r"(1u) : "memory");
-                    asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, q; }" ::"r"(tbase),
-                                 "l"(dal), "l"(dbh), "r"(idesc), "r"(1u) : "memory");
-                }
-                commit(bar_empty + 8 * s);
-                if (c + 1 == chunks) commit(bar_done);
+                for (int t = 0; t < KC / 16; ++t)
+                    tc::mma_bf16x3(tbase, tc::sdesc(dbase, a_hi + t * 256), tc::sdesc(dbase, a_lo + t * 256),
+                                   tc::sdesc(dbase, b_hi + t * 256), tc::sdesc(dbase, b_lo + t * 256), idesc, (c > 0 || t > 0) ? 1u : 0u);
+                tc::commit(bar_empty + 8 * s);
+                if (c + 1 == chunks) tc::commit(bar_done);
             }
             __syncwarp();
         }
     }
     // ---- epilogue: accumulator (lane = co row, column = ci) -> atomics into dW
     if (chunks > 0) {
-        mbar_wait(bar_done, 0);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc::mbar_wait(bar_done, 0);
+        tc::fence_after();
         const int row = (warp & 3) * 32 + lane;                       // a warp reads the TMEM lanes of its quarter
         const int co = co0 + row;
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
             const int col0 = (warp >> 2) * 64 + h * 32;
             unsigned r[32];
-            ld32(tbase + ((unsigned)((warp & 3) * 32) << 16) + (unsigned)col0, r);
+            tc::ld32(tbase + ((unsigned)((warp & 3) * 32) << 16) + (unsigned)col0, r);
             if (co < cout) {
                 float* dst = dw + (int64_t)co * lddw + ci0 + col0;
                 if (vec_red && ci0 + col0 + 32 <= cin) {
@@ -234,9 +166,9 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
         }
         if (do_bias) atomicAdd(&db[co0 + m], bsum);
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc::fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(128));
+    if (warp == 0) tc::tmem_dealloc(tbase, 128);
 }
 
 }  // namespace gtc

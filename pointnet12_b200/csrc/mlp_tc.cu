@@ -18,12 +18,12 @@
 // from (tcgen05.mma with A in TMEM).  Shared memory only holds weight tiles: pre-packed on the device into the
 // exact UMMA K-major core-matrix image (8 rows x 16 bytes, no swizzle), streamed per 64-wide K slice with one
 // cp.async.bulk (TMA engine) each into a 2-stage ring, completion on mbarriers (complete_tx), stage release by
-// tcgen05.commit.  Conventions (descriptor fields, A packing, TMEM addressing) were pinned on hardware with
-// tools/probes/tc_probe.cu.
+// tcgen05.commit.  The PTX and its conventions (descriptor fields, A packing, TMEM addressing) come from tcgen05.cuh.
 #include <cuda_bf16.h>
 #include <math_constants.h>
 
 #include "common.cuh"
+#include "tcgen05.cuh"
 
 namespace pn {
 
@@ -124,64 +124,6 @@ __global__ void tc_pack_layer_kernel(const float* __restrict__ w, const float* _
 }
 
 // ------------------------------------------------------------------------------------------------ device helpers
-__device__ __forceinline__ unsigned tc_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void tc_mbar_init(unsigned bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void tc_mbar_wait(unsigned bar, unsigned parity) {
-    unsigned done = 0;
-    while (!done) {
-        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    }
-}
-// one lane of a converged warp (the instruction sequence around it stays warp-uniform, so descriptors and barrier
-// addresses are computed in uniform registers instead of being moved there lane by lane)
-__device__ __forceinline__ bool tc_elect() {
-    unsigned p;
-    asm volatile("{ .reg .pred q; elect.sync _|q, 0xffffffff; selp.u32 %0, 1, 0, q; }" : "=r"(p));
-    return p != 0;
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(unsigned bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_ld32(unsigned taddr, unsigned (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tc_st16(unsigned taddr, const unsigned (&r)[16]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
-                 "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]),
-                 "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-                 : "memory");
-}
-// 32 fp32 values -> 16 packed bf16x2 "hi" words + 16 "lo" words (even k in the low half), stored at column c of both regions
-__device__ __forceinline__ void tc_store_split32(unsigned t_hi, unsigned t_lo, const float (&v)[32]) {
-    unsigned hi[16], lo[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) {
-        // cvt.rn.bf16x2.f32: two conversions per instruction; .x (low half) = even k
-        const __nv_bfloat162 h = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
-        const unsigned hb = *reinterpret_cast<const unsigned*>(&h);
-        const float r0 = v[2 * j] - __uint_as_float(hb << 16);
-        const float r1 = v[2 * j + 1] - __uint_as_float(hb & 0xFFFF0000u);
-        const __nv_bfloat162 l = __floats2bfloat162_rn(r0, r1);
-        hi[j] = hb;
-        lo[j] = *reinterpret_cast<const unsigned*>(&l);
-    }
-    tc_st16(t_hi, hi);
-    tc_st16(t_lo, lo);
-}
 // order-preserving float <-> uint key (for REDUX max over possibly negative values)
 __device__ __forceinline__ unsigned tc_key(float f) {
     const unsigned b = __float_as_uint(f);
@@ -191,29 +133,15 @@ __device__ __forceinline__ float tc_unkey(unsigned k) {
     return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
 }
 
-// Column-wise max over the 32 rows (= lanes) of a warp for 32 columns held one row per lane: a butterfly in which
-// every step halves the columns a lane is responsible for (16 + 8 + 4 + 2 + 1 = 31 shuffles and max per lane instead
-// of 32 REDUX instructions, which the hardware serialises).  Afterwards lane j holds the max of column j.
-template <int W>
-__device__ __forceinline__ void tc_colmax_step(float (&v)[32], int lane) {
-    if constexpr (W >= 1) {
-        const bool up = (lane & W) != 0;
-#pragma unroll
-        for (int i = 0; i < W; ++i) {
-            const float send = up ? v[i] : v[i + W];
-            const float keep = up ? v[i + W] : v[i];
-            v[i] = fmaxf(keep, __shfl_xor_sync(0xffffffffu, send, W));
-        }
-        tc_colmax_step<W / 2>(v, lane);
-    }
-}
+// Column-wise max over the 32 rows (= lanes) of a warp for 32 columns held one row per lane (a butterfly: 31 shuffles and
+// max per lane instead of 32 REDUX instructions, which the hardware serialises).  Afterwards lane j holds the max of column j.
 __device__ __forceinline__ float tc_colmax32(float (&v)[32], int lane) {
-    tc_colmax_step<16>(v, lane);
+    tc::col_butterfly<16, 1>(v, lane, [](float x, float y) { return fmaxf(x, y); });
     return v[0];
 }
 // The same over the 16 rows of each half-warp for the 16 columns in v[0..15]: lane j holds column j % 16 of its half.
 __device__ __forceinline__ float tc_colmax16(float (&v)[32], int lane) {
-    tc_colmax_step<8>(v, lane);
+    tc::col_butterfly<8, 1>(v, lane, [](float x, float y) { return fmaxf(x, y); });
     return v[0];
 }
 // Max-pool epilogue for groups of 16 rows (two groups per warp): 32 accumulator columns in r -> y[group, c0 .. c0+31]
@@ -443,27 +371,9 @@ __device__ __forceinline__ void sa_small_row(const TcIo& io, bool valid, int64_t
 // bf16 pairs two columns are four consecutive channels = one float4, so the four threads of a quad read 64
 // CONTIGUOUS bytes of a source row and a warp-wide load touches 8 rows instead of 32: the row-per-thread producer
 // is bound by L1 tag lookups (32 distinct lines per load instruction), this one needs a quarter of them.
-__device__ __forceinline__ void tc_st_16x256(unsigned taddr, unsigned a0, unsigned a1, unsigned b0, unsigned b1) {
-    asm volatile("tcgen05.st.sync.aligned.16x256b.x1.b32 [%0], {%1,%2,%3,%4};" ::"r"(taddr), "r"(a0), "r"(a1), "r"(b0), "r"(b1) : "memory");
-}
 __device__ __forceinline__ void tc_split4(const float4 v, unsigned& h0, unsigned& h1, unsigned& l0, unsigned& l1) {
-    const __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
-    h0 = *reinterpret_cast<const unsigned*>(&a);
-    h1 = *reinterpret_cast<const unsigned*>(&b);
-    const __nv_bfloat162 c = __floats2bfloat162_rn(v.x - __uint_as_float(h0 << 16), v.y - __uint_as_float(h0 & 0xFFFF0000u));
-    const __nv_bfloat162 d = __floats2bfloat162_rn(v.z - __uint_as_float(h1 << 16), v.w - __uint_as_float(h1 & 0xFFFF0000u));
-    l0 = *reinterpret_cast<const unsigned*>(&c);
-    l1 = *reinterpret_cast<const unsigned*>(&d);
-}
-
-// tcgen05.ld.16x256b.x4: 16 lanes x 32 columns; r[4m + 2rb + c] = row t/4 + 8rb, column 8m + 2(t%4) + c.
-__device__ __forceinline__ void tc_ld_16x256_x4(unsigned taddr, unsigned (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.16x256b.x4.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+    tc::split_bf16x2(v.x, v.y, h0, l0);
+    tc::split_bf16x2(v.z, v.w, h1, l1);
 }
 
 // log_softmax over the first n_real (<= 32) accumulator columns of the 16 TMEM lanes at `taddr`, quad layout: the four
@@ -473,7 +383,7 @@ __device__ __forceinline__ void tc_ld_16x256_x4(unsigned taddr, unsigned (&r)[16
 __device__ __forceinline__ void tc_logsoftmax_quad(unsigned taddr, const float* bias, int n_real, int lane, int64_t rowA,
                                                    int64_t rowB, float* y, int64_t ldy) {
     unsigned r[16];
-    tc_ld_16x256_x4(taddr, r);
+    tc::ld_16x256_x4(taddr, r);
     const int qd = lane & 3;
     float v[2][8];
     float mx[2] = {-CUDART_INF_F, -CUDART_INF_F};
@@ -590,8 +500,8 @@ __device__ __forceinline__ void fp_quad_producer(const TcIo& io, int64_t seg, in
             tc_split4(v[2 * blk], ha0, ha1, la0, la1);
             tc_split4(v[2 * blk + 1], hb0, hb1, lb0, lb1);
             const unsigned off = ((unsigned)(blk * 16) << 16) + (unsigned)cg * 8;
-            tc_st_16x256(t_ahi + off, ha0, ha1, hb0, hb1);
-            tc_st_16x256(t_alo + off, la0, la1, lb0, lb1);
+            tc::st_16x256(t_ahi + off, ha0, ha1, hb0, hb1);
+            tc::st_16x256(t_alo + off, la0, la1, lb0, lb1);
         }
     }
 }
@@ -647,8 +557,8 @@ __device__ __forceinline__ void fp_quad_producer_fast(const TcIo& io, int64_t se
             tc_split4(v[2 * blk], ha0, ha1, la0, la1);
             tc_split4(v[2 * blk + 1], hb0, hb1, lb0, lb1);
             const unsigned off = ((unsigned)(blk * 16) << 16) + (unsigned)cg * 8;
-            tc_st_16x256(t_ahi + off, ha0, ha1, hb0, hb1);
-            tc_st_16x256(t_alo + off, la0, la1, lb0, lb1);
+            tc::st_16x256(t_ahi + off, ha0, ha1, hb0, hb1);
+            tc::st_16x256(t_alo + off, la0, la1, lb0, lb1);
         }
         if (stamps) *stamps++ = clock64();
     }
@@ -666,31 +576,28 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
     float* sbias = reinterpret_cast<float*>(smem + NS * ch.stage_bytes);
     unsigned long long* bars = reinterpret_cast<unsigned long long*>(smem + NS * ch.stage_bytes + ((ch.bias_floats * 4 + 15) & ~15));
     unsigned* tmem_slot = reinterpret_cast<unsigned*>(bars + 2 * kTcMaxStages + 1);
-    const unsigned bar_full0 = tc_smem_u32(&bars[0]), bar_empty0 = tc_smem_u32(&bars[kTcMaxStages]);   // stage st: + 8 st bytes
-    const unsigned bar_done = tc_smem_u32(&bars[2 * kTcMaxStages]);
-    const unsigned stage0 = tc_smem_u32(smem);
+    const unsigned bar_full0 = tc::smem_u32(&bars[0]), bar_empty0 = tc::smem_u32(&bars[kTcMaxStages]);   // stage st: + 8 st bytes
+    const unsigned bar_done = tc::smem_u32(&bars[2 * kTcMaxStages]);
+    const unsigned stage0 = tc::smem_u32(smem);
 
     const int tid = threadIdx.x, lane = tid & 31;
     const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);   // warp-uniform for the compiler: MMA operands stay in uniform registers
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc_smem_u32(tmem_slot)), "r"(ch.tmem_cols));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    if (warp == 0) tc::tmem_alloc(tmem_slot, ch.tmem_cols);
     if (tid == 0) {
         for (int st = 0; st < NS; ++st) {
-            tc_mbar_init(bar_full0 + 8 * st, 1);
-            tc_mbar_init(bar_empty0 + 8 * st, 1);
+            tc::mbar_init(bar_full0 + 8 * st, 1);
+            tc::mbar_init(bar_empty0 + 8 * st, 1);
         }
-        tc_mbar_init(bar_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tc::mbar_init(bar_done, 1);
+        tc::mbar_init_fence();
     }
     {
         const float* gb = reinterpret_cast<const float*>(blob + ch.bias_off);
         for (int i = tid; i < ch.bias_floats; i += THREADS) sbias[i] = gb[i];
     }
-    tc_fence_before();
+    tc::fence_before();
     __syncthreads();
-    tc_fence_after();
+    tc::fence_after();
     const unsigned tbase = __shfl_sync(0xffffffffu, *tmem_slot, 0);
     constexpr int HALVES = THREADS / 128, CSTEP = 32 * HALVES;
     const int wl = warp & 3, half = warp >> 2;                      // lane quarter / column slice (of HALVES) of this warp
@@ -747,11 +654,11 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                             for (int k0 = half * 32; k0 < kchunk; k0 += CSTEP) {   // this thread's row
                                 float v[32];
                                 row_load32<IN>(io, rc, kbase + k0, L.k_real, v);
-                                tc_store_split32(t_ahi + k0 / 2, t_alo + k0 / 2, v);
+                                tc::store_split32(t_ahi + k0 / 2, t_alo + k0 / 2, v);
                             }
                         }
-                        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-                        tc_fence_before();
+                        tc::wait_st();
+                        tc::fence_before();
                         __syncthreads();
                         stamp(2);
                     }
@@ -771,24 +678,14 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                             const unsigned char* src = wpass + (size_t)rows_P * ((s0 + s) * kTcKSub) * 4 + (size_t)r0 * kw * 2;
                             const unsigned dst = stage0 + fill_st * (unsigned)ch.stage_bytes;
                             const unsigned full = bar_full0 + 8 * fill_st;
-                            tc_mbar_wait(bar_empty0 + 8 * fill_st, ((fill / NS) & 1) ^ 1);
-                            if (tc_elect()) {
-                                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "r"(bytes) : "memory");
+                            tc::mbar_wait(bar_empty0 + 8 * fill_st, ((fill / NS) & 1) ^ 1);
+                            if (tc::elect()) {
+                                tc::mbar_arrive_expect_tx(full, bytes);
                                 if (rows_p == rows_P) {   // hi and lo images are adjacent: one copy
-                                    asm volatile(
-                                        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                                        "l"(src), "r"(bytes), "r"(full)
-                                        : "memory");
+                                    tc::bulk_load(dst, src, bytes, full);
                                 } else {
-                                    asm volatile(
-                                        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                                        "l"(src), "r"(bytes / 2), "r"(full)
-                                        : "memory");
-                                    asm volatile(
-                                        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                                            dst + bytes / 2),
-                                        "l"(src + (size_t)rows_P * kw * 2), "r"(bytes / 2), "r"(full)
-                                        : "memory");
+                                    tc::bulk_load(dst, src, bytes / 2, full);
+                                    tc::bulk_load(dst + bytes / 2, src + (size_t)rows_P * kw * 2, bytes / 2, full);
                                 }
                             }
                             __syncwarp();
@@ -798,40 +695,24 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                     }
                     if (warp == 0) {
                         // ---- MMA warp (same scheme): the MMAs of a slice are issued as soon as it has landed
-                        tc_fence_after();
-                        const unsigned idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(rows_p >> 3) << 17) | (8u << 24);
+                        tc::fence_after();
+                        const unsigned idesc = tc::idesc_bf16_f32(128, rows_p);
                         for (int s = 0; s < ns; ++s) {
                             const int kw = min(kTcKSub, L.k_pad - (s0 + s) * kTcKSub);
-                            tc_mbar_wait(bar_full0 + 8 * use_st, (use / NS) & 1);
-                            tc_fence_after();
+                            tc::mbar_wait(bar_full0 + 8 * use_st, (use / NS) & 1);
+                            tc::fence_after();
                             stamp(6);
                             const unsigned b_hi = stage0 + use_st * (unsigned)ch.stage_bytes, b_lo = b_hi + (unsigned)rows_p * kw * 2;
-                            const unsigned long long dbase = ((unsigned long long)((128u >> 4) & 0x3FFF) << 16) |
-                                                             ((unsigned long long)((((unsigned)kw / 8) * 128u >> 4) & 0x3FFF) << 32) |
-                                                             (1ull << 46);
-                            if (tc_elect()) {
+                            const unsigned long long dbase = tc::sdesc_base(((unsigned)kw / 8) * 128u);
+                            if (tc::elect()) {
                                 for (int t = 0; t < kw / 16; ++t) {
                                     const unsigned kcol = (unsigned)(s * kTcKSub + t * 16) / 2;   // A columns of this K step
-                                    const unsigned long long dh = dbase | (unsigned long long)(((b_hi + t * 256) >> 4) & 0x3FFF);
-                                    const unsigned long long dl = dbase | (unsigned long long)(((b_lo + t * 256) >> 4) & 0x3FFF);
+                                    const unsigned long long dh = tc::sdesc(dbase, b_hi + t * 256), dl = tc::sdesc(dbase, b_lo + t * 256);
                                     const unsigned acc0 = (a > 0 || s > 0 || t > 0) ? 1u : 0u;
-                                    asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, q; }" ::"r"(
-                                                     tbase),
-                                                 "r"(a_hi_col + kcol), "l"(dh), "r"(idesc), "r"(acc0)
-                                                 : "memory");
-                                    if (ch.split) {
-                                        asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, q; }" ::"r"(
-                                                         tbase),
-                                                     "r"(a_hi_col + kcol), "l"(dl), "r"(idesc), "r"(1u)
-                                                     : "memory");
-                                        asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, q; }" ::"r"(
-                                                         tbase),
-                                                     "r"(a_lo_col + kcol), "l"(dh), "r"(idesc), "r"(1u)
-                                                     : "memory");
-                                    }
+                                    tc::mma_bf16x3(tbase, a_hi_col + kcol, a_lo_col + kcol, dh, dl, idesc, acc0, ch.split);
                                 }
-                                tc_commit(bar_empty0 + 8 * use_st);
-                                if (s + 1 == ns) tc_commit(bar_done);
+                                tc::commit(bar_empty0 + 8 * use_st);
+                                if (s + 1 == ns) tc::commit(bar_done);
                             }
                             __syncwarp();
                             stamp(7);
@@ -841,9 +722,9 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                         stamp(3);
                     }
                     // ---- everyone waits for this chunk's MMAs (the A region / accumulator are then free to touch)
-                    tc_mbar_wait(bar_done, done_phase);
+                    tc::mbar_wait(bar_done, done_phase);
                     done_phase ^= 1;
-                    tc_fence_after();
+                    tc::fence_after();
                     stamp(4);
                 }
                 // ---- epilogue of pass p: accumulator columns [0, rows_p)
@@ -851,7 +732,7 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                 if (!last) {
                     for (int c0 = half * 32; c0 < rows_p; c0 += CSTEP) {
                         unsigned r[32];
-                        tc_ld32(t_x + c0, r);
+                        tc::ld32(t_x + c0, r);
                         float v[32];
                         if (l == 0 && io.res != nullptr) {   // the skip half of the layer, computed beforehand per row
                             const float4* rr = reinterpret_cast<const float4*>(io.res + (rc.valid ? rc.row : 0) * io.ldr + n0 + c0);
@@ -869,15 +750,15 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                             const float f = __uint_as_float(r[j]) + bias[c0 + j];
                             v[j] = L.relu ? fmaxf(f, 0.0f) : f;
                         }
-                        tc_store_split32(t_ahi + c0 / 2, t_alo + c0 / 2, v);
+                        tc::store_split32(t_ahi + c0 / 2, t_alo + c0 / 2, v);
                     }
-                    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-                    tc_fence_before();
+                    tc::wait_st();
+                    tc::fence_before();
                     __syncthreads();
                 } else if (io.out_mode == TC_OUT_ROWS) {
                     for (int c0 = half * 32; c0 < rows_p; c0 += CSTEP) {
                         unsigned r[32];
-                        tc_ld32(t_x + c0, r);
+                        tc::ld32(t_x + c0, r);
                         if (rc.valid) {
                             float* dst = io.y + rc.row * io.ldy + n0 + c0;
                             const int nleft = L.n_real - (n0 + c0);
@@ -901,7 +782,7 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                             }
                         }
                     }
-                    tc_fence_before();
+                    tc::fence_before();
                     __syncthreads();
                 } else if (io.out_mode == TC_OUT_MAX) {
                     // group = 32 consecutive rows = this warp: REDUX max per channel, lane j keeps channel c0 + j
@@ -910,7 +791,7 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                     const int64_t g = __shfl_sync(0xffffffffu, grp, 0);
                     for (int c0 = half * 32; c0 < rows_p; c0 += CSTEP) {
                         unsigned r[32];
-                        tc_ld32(t_x + c0, r);
+                        tc::ld32(t_x + c0, r);
                         if (io.group == 16) {
                             tc_store_max16(r, bias, L.relu, rc.valid, rc.row, lane, c0, L.n_real - n0, io.y + n0, io.ldy);
                             continue;
@@ -924,21 +805,21 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                         const int n = n0 + c0 + lane;
                         if (any_valid && n < L.n_real) io.y[g * io.ldy + n] = mine;
                     }
-                    tc_fence_before();
+                    tc::fence_before();
                     __syncthreads();
                 } else {   // TC_OUT_LOGSOFTMAX over the n_real (<= 64) classes of the row: column-half 0 warps only
                     if (half == 0) {
                         float m = -CUDART_INF_F, ssum = 0.0f;
                         for (int c0 = 0; c0 < rows_p; c0 += 32) {
                             unsigned r[32];
-                            tc_ld32(t_x + c0, r);
+                            tc::ld32(t_x + c0, r);
 #pragma unroll
                             for (int j = 0; j < 32; ++j)
                                 if (c0 + j < L.n_real) m = fmaxf(m, __uint_as_float(r[j]) + bias[c0 + j]);
                         }
                         for (int c0 = 0; c0 < rows_p; c0 += 32) {
                             unsigned r[32];
-                            tc_ld32(t_x + c0, r);
+                            tc::ld32(t_x + c0, r);
 #pragma unroll
                             for (int j = 0; j < 32; ++j)
                                 if (c0 + j < L.n_real) ssum += __expf((__uint_as_float(r[j]) + bias[c0 + j]) - m);
@@ -946,7 +827,7 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                         const float ls = __logf(ssum);
                         for (int c0 = 0; c0 < rows_p; c0 += 32) {
                             unsigned r[32];
-                            tc_ld32(t_x + c0, r);
+                            tc::ld32(t_x + c0, r);
                             if (rc.valid) {
                                 float* dst = io.y + rc.row * io.ldy + c0;
 #pragma unroll
@@ -955,16 +836,16 @@ mlp_tc_kernel(const __grid_constant__ TcChain ch, const unsigned char* __restric
                             }
                         }
                     }
-                    tc_fence_before();
+                    tc::fence_before();
                     __syncthreads();
                 }
                 stamp(5);
             }
         }
     }
-    tc_fence_before();
+    tc::fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tbase), "r"(ch.tmem_cols));
+    if (warp == 0) tc::tmem_dealloc(tbase, ch.tmem_cols);
 }
 
 // ------------------------------------------------------------------------------------------------ resident kernel
@@ -993,13 +874,13 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
     unsigned* tmem_slot = reinterpret_cast<unsigned*>(bars + 1 + GROUPS);
     volatile unsigned* tile_slot = reinterpret_cast<volatile unsigned*>(bars + 6);   // [GROUPS <= 4]
     unsigned* mma_lock = reinterpret_cast<unsigned*>(bars + 8);
-    const unsigned bar_w = tc_smem_u32(&bars[0]);
-    const unsigned smem_w = tc_smem_u32(smem);
+    const unsigned bar_w = tc::smem_u32(&bars[0]);
+    const unsigned smem_w = tc::smem_u32(smem);
 
     const int tid = threadIdx.x, lane = tid & 31;
     const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);   // warp-uniform for the compiler: MMA operands stay in uniform registers
     const int g = warp / WPG, gw = warp % WPG;
-    const unsigned bar_done = tc_smem_u32(&bars[1 + g]);
+    const unsigned bar_done = tc::smem_u32(&bars[1 + g]);
     const int64_t tiles_per_seg = (io.seg_rows + 127) / 128;
     const int64_t ntiles = io.nseg * tiles_per_seg;
     // Dynamic tile scheduling (io.tile_ctr): every group draws its tiles from one global counter, so a CTA whose SM was
@@ -1008,15 +889,12 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
     // last ticket resets the counter for the next launch that is handed the same word.
     const bool dyn = io.tile_ctr != nullptr;
     const unsigned last_ticket = (unsigned)ntiles + gridDim.x * GROUPS - 1u;
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc_smem_u32(tmem_slot)), "r"(512));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    if (warp == 0) tc::tmem_alloc(tmem_slot, 512);
     if (tid == 0) {
         *mma_lock = 0u;
-        tc_mbar_init(bar_w, 1);
-        for (int i = 0; i < GROUPS; ++i) tc_mbar_init(tc_smem_u32(&bars[1 + i]), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tc::mbar_init(bar_w, 1);
+        for (int i = 0; i < GROUPS; ++i) tc::mbar_init(tc::smem_u32(&bars[1 + i]), 1);
+        tc::mbar_init_fence();
         bool any = true;
         if (dyn) {
             any = false;
@@ -1028,19 +906,12 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
             }
         }
         if (any) {   // (a CTA that arrives after the last tile was taken must not leave with a copy in flight)
-            // the whole blob, in pieces of at most 32 KB, all completing on one barrier
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_w), "r"(ch.blob_bytes) : "memory");
-            for (unsigned off = 0; off < ch.blob_bytes; off += 32768u) {
-                const unsigned n = ch.blob_bytes - off < 32768u ? ch.blob_bytes - off : 32768u;
-                asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_w + off),
-                             "l"(blob + off), "r"(n), "r"(bar_w)
-                             : "memory");
-            }
+            tc::bulk_load_pieces(smem_w, blob, ch.blob_bytes, bar_w);     // the whole blob
         }
     }
-    tc_fence_before();
+    tc::fence_before();
     __syncthreads();
-    tc_fence_after();
+    tc::fence_after();
     const unsigned tbase = __shfl_sync(0xffffffffu, *tmem_slot, 0) + (unsigned)(g * GCOLS);
     const int wl = gw & 3, half = gw >> 2;                           // lane quarter (== warp % 4) / column half
     const unsigned tlane = tbase + ((unsigned)(wl * 32) << 16);      // this warp's 32 TMEM lanes
@@ -1087,18 +958,18 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                     if (half == 0) {
                         float v[32];
                         sa_small_row(io, rc.valid, rc.row, v);
-                        tc_store_split32(t_ahi, t_alo, v);
+                        tc::store_split32(t_ahi, t_alo, v);
                     }
                 } else {
                     for (int k0 = half * 32; k0 < L.k_pad; k0 += CSTEP) {   // this thread's row
                         float v[32];
                         row_load32<IN>(io, rc, k0, L.k_real, v);
-                        tc_store_split32(t_ahi + k0 / 2, t_alo + k0 / 2, v);
+                        tc::store_split32(t_ahi + k0 / 2, t_alo + k0 / 2, v);
                     }
                 }
-                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+                tc::wait_st();
                 if (rec) drow[dcol++] = clock64();
-                tc_fence_before();
+                tc::fence_before();
                 tc_group_bar(1 + g, GTHREADS);
             }
             if (ch.probe & 1) break;
@@ -1107,7 +978,7 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                 // ---- MMA issue.  The whole warp walks the (warp-uniform) loop and one elected lane issues: every operand of
                 // tcgen05.mma then lives in a uniform register.  (Issued from inside an `if (lane == 0)` branch the same loop
                 // costs an ELECT + 3 x R2UR.BROADCAST waterfall per MMA, ~90 cycles against the 64 the tensor pipe needs.)
-                if (!w_ready) tc_mbar_wait(bar_w, 0);
+                if (!w_ready) tc::mbar_wait(bar_w, 0);
                 // One group issues a whole layer at a time.  Without the lock the groups interleave their MMAs in the tensor
                 // queue, both layers complete together and the groups stay in lock-step: MMA phases with idle CUDA cores, then
                 // epilogue phases with an idle tensor pipe.  With it the first group's accumulator is ready after one layer's
@@ -1119,62 +990,49 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                     if (lane == 0) while (atomicCAS(mma_lock, 0u, 1u) != 0u) {}
                     __syncwarp();
                 }
-                tc_fence_after();
+                tc::fence_after();
                 const unsigned wl_base = smem_w + L.w_off;
-                const unsigned idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(L.n_pad >> 3) << 17) | (8u << 24);
+                const unsigned idesc = tc::idesc_bf16_f32(128, L.n_pad);
                 const int ns = L.k_pad / kTcKSub;                    // k_pad is a multiple of 32: every slice is 32 wide
                 // shared-memory descriptor: LBO = 128 B (next 8 K values), SBO = 512 B (next 8 rows), version bit 46; the
                 // start-address field (bits 0-13, 16-byte units) advances by 16 per 16-wide K step, n_pad * 8 per slice,
                 // and the lo image of a slice sits n_pad * 4 units after its hi image
-                const unsigned d_hi32 = (unsigned)((((32u / 8) * 128u >> 4) & 0x3FFF) | (1u << 14));
-                unsigned d_lo32 = (((128u >> 4) & 0x3FFF) << 16) | ((wl_base >> 4) & 0x3FFF);
+                const unsigned d_hi32 = tc::sdesc_hi32((32u / 8) * 128u);
+                unsigned d_lo32 = tc::sdesc_lo32(wl_base);
                 const unsigned lo_img = (unsigned)L.n_pad * 4u, slice = (unsigned)L.n_pad * 8u;
-                const bool issuer = tc_elect();
+                const bool issuer = tc::elect();
                 unsigned kcol = 0;
                 for (int s = 0; s < ns; ++s) {
 #pragma unroll
                     for (int t = 0; t < 2; ++t) {
                         const unsigned long long dh = ((unsigned long long)d_hi32 << 32) | (unsigned long long)(d_lo32 + 16u * t);
                         const unsigned long long dl = dh + lo_img;
-                        const unsigned acc0 = (s > 0 || t > 0) ? 1u : 0u;
-                        if (issuer) {
-                            asm volatile("{ .reg .pred q; setp.ne.b32 q, %4, 0; tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, q; }" ::"r"(
-                                             tbase),
-                                         "r"(a_hi_col + kcol), "l"(dh), "r"(idesc), "r"(acc0)
-                                         : "memory");
-                            if (ch.split) {
-                                asm volatile("tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, 1;" ::"r"(tbase), "r"(a_hi_col + kcol),
-                                             "l"(dl), "r"(idesc)
-                                             : "memory");
-                                asm volatile("tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, 1;" ::"r"(tbase), "r"(a_lo_col + kcol),
-                                             "l"(dh), "r"(idesc)
-                                             : "memory");
-                            }
-                        }
+                        if (issuer)
+                            tc::mma_bf16x3(tbase, a_hi_col + kcol, a_lo_col + kcol, dh, dl, idesc, (s > 0 || t > 0) ? 1u : 0u, ch.split);
                         kcol += 8;
                     }
                     d_lo32 += slice;
                 }
-                if (issuer) tc_commit(bar_done);
+                if (issuer) tc::commit(bar_done);
                 __syncwarp();
                 if (use_lock && lane == 0) atomicExch(mma_lock, 0u);
                 if (rec) drow[dcol++] = clock64();
             }
-            tc_mbar_wait(bar_done, done_phase);
+            tc::mbar_wait(bar_done, done_phase);
             done_phase ^= 1;
             if (rec) drow[dcol++] = clock64();
             if (!w_ready) {     // the bias table arrived with the weights: every reader observes the barrier once
-                tc_mbar_wait(bar_w, 0);
+                tc::mbar_wait(bar_w, 0);
                 w_ready = true;
             }
-            tc_fence_after();
+            tc::fence_after();
 
             // ---- epilogue: accumulator columns [0, n_pad)
             const float* bias = sbias + L.b_off;
             if (!last) {
                 for (int c0 = half * 32; c0 < L.n_pad; c0 += CSTEP) {
                     unsigned r[32];
-                    tc_ld32(t_x + c0, r);
+                    tc::ld32(t_x + c0, r);
                     float v[32];
                     if (l == 0 && io.res != nullptr) {   // the skip half of the layer, computed beforehand per row
                         const float4* rr = reinterpret_cast<const float4*>(io.res + (rc.valid ? rc.row : 0) * io.ldr + c0);
@@ -1192,13 +1050,13 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                         const float f = __uint_as_float(r[j]) + bias[c0 + j];
                         v[j] = L.relu ? fmaxf(f, 0.0f) : f;
                     }
-                    tc_store_split32(t_ahi + c0 / 2, t_alo + c0 / 2, v);
+                    tc::store_split32(t_ahi + c0 / 2, t_alo + c0 / 2, v);
                 }
-                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+                tc::wait_st();
             } else if (io.out_mode == TC_OUT_ROWS) {
                 for (int c0 = half * 32; c0 < L.n_pad; c0 += CSTEP) {
                     unsigned r[32];
-                    tc_ld32(t_x + c0, r);
+                    tc::ld32(t_x + c0, r);
                     if (rc.valid) {
                         float* dst = io.y + rc.row * io.ldy + c0;
                         const int nleft = L.n_real - c0;
@@ -1229,7 +1087,7 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                 const int64_t gi = __shfl_sync(0xffffffffu, grp, 0);
                 for (int c0 = half * 32; c0 < L.n_pad; c0 += CSTEP) {
                     unsigned r[32];
-                    tc_ld32(t_x + c0, r);
+                    tc::ld32(t_x + c0, r);
                     if (io.group == 16) {
                         tc_store_max16(r, bias, L.relu, rc.valid, rc.row, lane, c0, L.n_real, io.y, io.ldy);
                         continue;
@@ -1258,14 +1116,14 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                     float m = -CUDART_INF_F, ssum = 0.0f;
                     for (int c0 = 0; c0 < L.n_pad; c0 += 32) {
                         unsigned r[32];
-                        tc_ld32(t_x + c0, r);
+                        tc::ld32(t_x + c0, r);
 #pragma unroll
                         for (int j = 0; j < 32; ++j)
                             if (c0 + j < L.n_real) m = fmaxf(m, __uint_as_float(r[j]) + bias[c0 + j]);
                     }
                     for (int c0 = 0; c0 < L.n_pad; c0 += 32) {
                         unsigned r[32];
-                        tc_ld32(t_x + c0, r);
+                        tc::ld32(t_x + c0, r);
 #pragma unroll
                         for (int j = 0; j < 32; ++j)
                             if (c0 + j < L.n_real) ssum += __expf((__uint_as_float(r[j]) + bias[c0 + j]) - m);
@@ -1273,7 +1131,7 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                     const float ls = __logf(ssum);
                     for (int c0 = 0; c0 < L.n_pad; c0 += 32) {
                         unsigned r[32];
-                        tc_ld32(t_x + c0, r);
+                        tc::ld32(t_x + c0, r);
                         if (rc.valid) {
                             float* dst = io.y + rc.row * io.ldy + c0;
 #pragma unroll
@@ -1288,16 +1146,16 @@ mlp_tc_res_kernel(const __grid_constant__ TcChain ch, const unsigned char* __res
                 if (next_ticket == last_ticket) atomicExch(io.tile_ctr, 0u);
                 tile_slot[g] = next_ticket;
             }
-            tc_fence_before();
+            tc::fence_before();
             tc_group_bar(1 + g, GTHREADS);
         }
         if (rec) drow[dcol++] = clock64();
         tile = dyn ? (int64_t)tile_slot[g] : tile + (int64_t)gridDim.x * GROUPS;
     }
-    if (ch.probe && tid == 0) tc_mbar_wait(bar_w, 0);   // (probe modes may skip every reader of the weights)
-    tc_fence_before();
+    if (ch.probe && tid == 0) tc::mbar_wait(bar_w, 0);   // (probe modes may skip every reader of the weights)
+    tc::fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*tmem_slot), "r"(512));
+    if (warp == 0) tc::tmem_dealloc(*tmem_slot, 512);
 }
 
 static size_t tc_res_smem_bytes(const TcChain& c) { return (size_t)((c.blob_bytes + 15u) & ~15u) + 9 * 8 + 16; }

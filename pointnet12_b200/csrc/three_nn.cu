@@ -185,26 +185,6 @@ constexpr int kNbWarps = 4;
 
 __device__ __forceinline__ bool nn_better(float d, int i, float dk, int ik) { return d < dk || (d == dk && i < ik); }
 
-__device__ __forceinline__ unsigned long long nn_pack2(float lo, float hi) {
-    unsigned long long r;
-    asm("mov.b64 %0, {%1,%2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-__device__ __forceinline__ unsigned long long nn_mul2(unsigned long long a, unsigned long long b) {
-    unsigned long long r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-__device__ __forceinline__ unsigned long long nn_fma2(unsigned long long a, unsigned long long b, unsigned long long c) {
-    unsigned long long r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
-__device__ __forceinline__ unsigned long long nn_add2(unsigned long long a, unsigned long long b) {
-    unsigned long long r;
-    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
 // monotone map float -> unsigned (for REDUX max over possibly negative distances) and back
 __device__ __forceinline__ unsigned nn_ordered(float f) {
     const unsigned u = __float_as_uint(f);
@@ -295,8 +275,8 @@ three_nn_blocks_kernel(const float* __restrict__ xyz1, int64_t aB, int64_t aN, i
         float d0 = CUDART_INF_F, d1 = CUDART_INF_F, d2 = CUDART_INF_F;
         int i0 = kNbPadIndex, i1 = kNbPadIndex, i2 = kNbPadIndex;
         const bool any_ok = __any_sync(0xffffffffu, ok);
-        const unsigned long long ax2 = nn_pack2(ax, ax), ay2 = nn_pack2(ay, ay), az2 = nn_pack2(az, az), sa2 = nn_pack2(sa, sa),
-                                 minus2 = nn_pack2(-2.0f, -2.0f);
+        const unsigned long long ax2 = pack2(ax, ax), ay2 = pack2(ay, ay), az2 = pack2(az, az), sa2 = pack2(sa, sa),
+                                 minus2 = pack2(-2.0f, -2.0f);
         for (int visited = 0; any_ok && visited < nblk; ++visited) {
             // nearest unvisited block of this lane, then of the warp
             float mine = lb[0];
@@ -325,12 +305,12 @@ three_nn_blocks_kernel(const float* __restrict__ xyz1, int64_t aB, int64_t aN, i
             for (int q = 0; q < BP / 2; ++q) {
                 const float4 A = pp[2 * q], Bv = pp[2 * q + 1];
                 // dot = fma(az,bz, fma(ay,by, ax*bx));  d = fma(-2, dot, |a|^2) + |b|^2   (sqdist_expand, two candidates at once)
-                unsigned long long t = nn_mul2(ax2, nn_pack2(A.x, A.y));
-                t = nn_fma2(ay2, nn_pack2(A.z, A.w), t);
-                t = nn_fma2(az2, nn_pack2(Bv.x, Bv.y), t);
-                t = nn_add2(nn_fma2(minus2, t, sa2), nn_pack2(Bv.z, Bv.w));
+                unsigned long long t = mul2(ax2, pack2(A.x, A.y));
+                t = fma2(ay2, pack2(A.z, A.w), t);
+                t = fma2(az2, pack2(Bv.x, Bv.y), t);
+                t = add2(fma2(minus2, t, sa2), pack2(Bv.z, Bv.w));
                 float e0, e1;
-                asm("mov.b64 {%0,%1}, %2;" : "=f"(e0), "=f"(e1) : "l"(t));
+                unpack2(t, e0, e1);
                 if (!__any_sync(0xffffffffu, !(e0 > d2) || !(e1 > d2))) continue;        // the common case, warp-uniform
                 if (__any_sync(0xffffffffu, !(e0 > d2))) nn_insert(e0, pi[2 * q], d0, d1, d2, i0, i1, i2);
                 if (__any_sync(0xffffffffu, !(e1 > d2))) nn_insert(e1, pi[2 * q + 1], d0, d1, d2, i0, i1, i2);
