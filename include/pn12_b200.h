@@ -401,6 +401,24 @@ int pn_group_bwd_f32(const float* dgrouped, int64_t ldg, int col0, int D, const 
  * dpoints2[b, idx[b,n,k], :] += weight[b,n,k] * dx[(b,n), D1:].  dpoints2 contiguous [B,S,D2], zeroed by the caller. */
 int pn_three_interpolate_bwd_f32(const float* dx, int64_t ldx, int D1, int D2, const int64_t* idx, const float* weight,
                                  int B, int N, int S, float* dpoints1, float* dpoints2, pn_stream_t stream);
+/* Coordinate gradient of the gather + recentre of sample_and_group (model/pointnet_util.py:127-131; MSG :243-247; group-all
+ * :151-156): dxyz[b, idx[b,s,k], :] += dgrouped[(b,s,k), col0 : col0+3] (the xyz_rel columns: col0 = 0 in sample_and_group
+ * order, D in MSG order) and, for the in-place recentring, dnew_xyz[b,s,:] = -sum_k dgrouped[(b,s,k), col0 : col0+3]
+ * (written; dnew_xyz = NULL for group-all, which is not recentred).  dxyz contiguous [B,N,3], zeroed by the caller;
+ * dnew_xyz contiguous [B,S,3]. */
+int pn_group_bwd_xyz_f32(const float* dgrouped, int64_t ldg, int col0, const int64_t* idx, int B, int N, int S, int K,
+                         float* dxyz, float* dnew_xyz, pn_stream_t stream);
+/* pn_three_interpolate_bwd_f32 plus the gradient w.r.t. the coordinates of both clouds, through the 3-NN weights of
+ * model/pointnet_util.py:295-300 (dists = square_distance(xyz1, xyz2); dists[dists < 1e-10] = 1e-10; weight = 1/dists,
+ * normalised).  points2 [B,S,D2] and xyz1 [B,N,3] / xyz2 [B,S,3] (element strides, like pn_three_nn_f32) are the forward's
+ * inputs; the distances are recomputed with the 3-NN kernels' rounding sequence, so the clamp decision and 1/d are the
+ * forward's.  A clamped distance passes no gradient.  dxyz1 [B,N,3] is written; dpoints2 [B,S,D2] and dxyz2 [B,S,3]
+ * (contiguous) are accumulated into buffers the caller zeroed.  Needs S >= 3 (S == 1 is a broadcast without coordinate
+ * gradient; S == 2 has no 3-NN forward). */
+int pn_three_interpolate_bwd_xyz_f32(const float* dx, int64_t ldx, int D1, int D2, const int64_t* idx, const float* weight,
+                                     const float* points2, int64_t p2B, int64_t p2S, int64_t p2C, const float* xyz1, int64_t aB,
+                                     int64_t aN, int64_t aC, const float* xyz2, int64_t bB, int64_t bS, int64_t bC, int B, int N,
+                                     int S, float* dpoints1, float* dpoints2, float* dxyz1, float* dxyz2, pn_stream_t stream);
 /* nn.Dropout(p) in training mode (pointnet2.py:172): y = x*keep/(1-p).  mask_in (bytes, dense [rows*C]) != NULL:
  * keep = mask_in -- also the backward pass.  Otherwise keep ~ Bernoulli(1-p) from a Philox4x32-10 stream keyed by
  * seed_offset[0] with counter offset seed_offset[1] (DEVICE memory, so a replayed CUDA graph sees fresh values) and

@@ -91,6 +91,9 @@ _SIGNATURES = {
     "pn_transpose_f32": [vp, i32, i32, vp, vp],
     "pn_group_bwd_f32": [vp, i64, i32, i32, vp, i32, i32, i32, i32, vp, vp],
     "pn_three_interpolate_bwd_f32": [vp, i64, i32, i32, vp, vp, i32, i32, i32, vp, vp, vp],
+    "pn_group_bwd_xyz_f32": [vp, i64, i32, vp, i32, i32, i32, i32, vp, vp, vp],
+    "pn_three_interpolate_bwd_xyz_f32": [vp, i64, i32, i32, vp, vp, vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64,
+                                         i32, i32, i32, vp, vp, vp, vp, vp],
     "pn_dropout_f32": [vp, i64, i64, i32, f32, vp, vp, vp, vp, i64, vp],
     "pn_cross_entropy_f32": [vp, i64, vp, i64, i32, vp, vp, vp, i64, f32, vp],
     "pn_log_softmax_bwd_f32": [vp, i64, vp, i64, i64, i32, vp, i64, vp],

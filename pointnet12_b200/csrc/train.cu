@@ -394,6 +394,146 @@ __global__ void three_interpolate_bwd_kernel(const float* __restrict__ dx, int64
     }
 }
 
+// Coordinate gradient of the grouping (pointnet_util.py:127-131, :243-247; group-all :151-156).  The three xyz_rel
+// columns at col0 of row (b,s,k) go to dxyz[b, idx[b,s,k]] (a padded ball repeats its first hit: each repeat adds its own
+// share); the recentring subtracted new_xyz[b,s] from every row of the group, so dnew[b,s] = -sum_k (dnew = NULL: group-all,
+// not recentred).  One warp per group, lanes over k.
+__global__ void __launch_bounds__(256)
+group_bwd_xyz_kernel(const float* __restrict__ dg, int64_t ldg, int col0, const int64_t* __restrict__ idx, int N, int S,
+                     int K, int64_t groups, float* __restrict__ dxyz, float* __restrict__ dnew) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t grp = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); grp < groups; grp += warps) {
+        const int64_t b = grp / S;
+        float sx = 0.0f, sy = 0.0f, sz = 0.0f;
+        for (int k = lane; k < K; k += 32) {
+            const int64_t row = grp * K + k;
+            const float* r = dg + row * ldg + col0;
+            const float x = r[0], y = r[1], z = r[2];
+            int64_t j = idx[row];
+            j = j < 0 ? 0 : (j >= N ? N - 1 : j);
+            float* o = dxyz + (b * N + j) * 3;
+            atomicAdd(o, x);
+            atomicAdd(o + 1, y);
+            atomicAdd(o + 2, z);
+            sx += x;
+            sy += y;
+            sz += z;
+        }
+        if (dnew) {
+#pragma unroll
+            for (int o = 16; o; o >>= 1) {
+                sx += __shfl_xor_sync(0xffffffffu, sx, o);
+                sy += __shfl_xor_sync(0xffffffffu, sy, o);
+                sz += __shfl_xor_sync(0xffffffffu, sz, o);
+            }
+            if (lane == 0) {
+                dnew[grp * 3] = -sx;
+                dnew[grp * 3 + 1] = -sy;
+                dnew[grp * 3 + 2] = -sz;
+            }
+        }
+    }
+}
+
+// three_interpolate_bwd_kernel plus the gradient of the 3-NN weights w.r.t. both clouds (pointnet_util.py:295-307).  One
+// warp per fine row n of cloud b, lanes over the channels; the row of dx is read once.  With a = xyz1[n], b_k = xyz2[idx_k]:
+//   d_k = the forward's fp32 expansion-formula distance (sqdist_expand: same clamp decision, same 1/d as the 3-NN kernels)
+//   r_k = 1/max(d_k, 1e-10), R = sum r, w_k = r_k/R (the forward's weights), g_k = <dinterp, p2[idx_k]>
+//   dL/dd_j = -(g_j - sum_k w_k g_k) / R * r_j^2, or 0 where d_j was clamped (the masked assignment stops the gradient)
+//   dxyz1[n] = sum_j dL/dd_j * 2(a - b_j),   dxyz2[idx_j] += -dL/dd_j * 2(a - b_j)
+// VEC: the dx row (from D1), the p2 rows and the dp2 rows are read / added as float4.
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+three_interpolate_bwd_xyz_kernel(const float* __restrict__ dx, int64_t ldx, int D1, int D2, const int64_t* __restrict__ idx,
+                                 const float* __restrict__ weight, const float* __restrict__ p2, int64_t p2B, int64_t p2S,
+                                 int64_t p2C, const float* __restrict__ xyz1, int64_t aB, int64_t aN, int64_t aC,
+                                 const float* __restrict__ xyz2, int64_t bB, int64_t bS, int64_t bC, int N, int S, int64_t rows,
+                                 float* __restrict__ dp1, float* __restrict__ dp2, float* __restrict__ dxyz1,
+                                 float* __restrict__ dxyz2) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t row = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5); row < rows; row += warps) {
+        const int64_t b = row / N, n = row - b * N;
+        const float* g = dx + row * ldx;
+        int64_t j[3];
+        float w[3], dot[3] = {0.0f, 0.0f, 0.0f};
+        const float* q[3];
+        float* o[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            int64_t jj = idx[row * 3 + k];
+            j[k] = jj < 0 ? 0 : (jj >= S ? S - 1 : jj);
+            w[k] = weight[row * 3 + k];
+            q[k] = p2 + b * p2B + j[k] * p2S;
+            o[k] = dp2 + (b * S + j[k]) * D2;
+        }
+        if (VEC) {
+            for (int c = lane * 4; c < D1; c += 128)
+                *reinterpret_cast<float4*>(dp1 + row * D1 + c) = *reinterpret_cast<const float4*>(g + c);
+            for (int c = lane * 4; c < D2; c += 128) {
+                const float4 gv = *reinterpret_cast<const float4*>(g + D1 + c);
+#pragma unroll
+                for (int k = 0; k < 3; ++k) {
+                    const float4 pv = *reinterpret_cast<const float4*>(q[k] + c);
+                    dot[k] = fmaf(gv.x, pv.x, fmaf(gv.y, pv.y, fmaf(gv.z, pv.z, fmaf(gv.w, pv.w, dot[k]))));
+                    atomicAdd(reinterpret_cast<float4*>(o[k] + c), make_float4(gv.x * w[k], gv.y * w[k], gv.z * w[k], gv.w * w[k]));
+                }
+            }
+        } else {
+            for (int c = lane; c < D1; c += 32) dp1[row * D1 + c] = g[c];
+            for (int c = lane; c < D2; c += 32) {
+                const float gv = g[D1 + c];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) {
+                    dot[k] = fmaf(gv, q[k][c * p2C], dot[k]);
+                    atomicAdd(o[k] + c, gv * w[k]);
+                }
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 3; ++k)
+#pragma unroll
+            for (int s = 16; s; s >>= 1) dot[k] += __shfl_xor_sync(0xffffffffu, dot[k], s);
+        if (lane != 0) continue;
+        const float* pa = xyz1 + b * aB + n * aN;
+        const float ax = pa[0], ay = pa[aC], az = pa[2 * aC];
+        const float sa = sqnorm3(ax, ay, az);
+        float r[3], ex[3], ey[3], ez[3];
+        bool live[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const float* pb = xyz2 + b * bB + j[k] * bS;
+            const float bx = pb[0], by = pb[bC], bz = pb[2 * bC];
+            const float d = sqdist_expand(ax, ay, az, sa, bx, by, bz, sqnorm3(bx, by, bz));
+            live[k] = !(d < 1e-10f);
+            r[k] = __fdiv_rn(1.0f, live[k] ? d : 1e-10f);
+            ex[k] = ax - bx;
+            ey[k] = ay - by;
+            ez[k] = az - bz;
+        }
+        const float R = r[0] + r[1] + r[2];
+        const float mean = w[0] * dot[0] + w[1] * dot[1] + w[2] * dot[2];
+        float gx = 0.0f, gy = 0.0f, gz = 0.0f;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            // 2 dL/dd_k; the product is grouped so that r^2 (up to 1e20) never stands alone
+            const float t = live[k] ? -2.0f * ((dot[k] - mean) / R * r[k]) * r[k] : 0.0f;
+            const float tx = t * ex[k], ty = t * ey[k], tz = t * ez[k];
+            gx += tx;
+            gy += ty;
+            gz += tz;
+            float* o2 = dxyz2 + (b * S + j[k]) * 3;
+            atomicAdd(o2, -tx);
+            atomicAdd(o2 + 1, -ty);
+            atomicAdd(o2 + 2, -tz);
+        }
+        dxyz1[row * 3] = gx;
+        dxyz1[row * 3 + 1] = gy;
+        dxyz1[row * 3 + 2] = gz;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // Dropout.  Philox4x32-10 keyed by (seed), counter = (element / 4, offset): four uniform words per call.
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
@@ -774,6 +914,43 @@ PN_EXPORT int pn_three_interpolate_bwd_f32(const float* dx, int64_t ldx, int D1,
     three_interpolate_bwd_kernel<<<ew_blocks(total, 256), 256, 0, (cudaStream_t)stream>>>(dx, ldx, D1, D2, idx, weight, N, S, total,
                                                                                          dpoints1, dpoints2);
     return finish_launch("pn_three_interpolate_bwd_f32");
+}
+
+PN_EXPORT int pn_group_bwd_xyz_f32(const float* dgrouped, int64_t ldg, int col0, const int64_t* idx, int B, int N, int S, int K,
+                                   float* dxyz, float* dnew_xyz, pn_stream_t stream) {
+    PN_REQUIRE(dgrouped && idx && dxyz, PN_ERR_BAD_ARG, "pn_group_bwd_xyz_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && S > 0 && K > 0 && col0 >= 0 && ldg >= col0 + 3, PN_ERR_BAD_ARG, "pn_group_bwd_xyz_f32: bad shape");
+    const int64_t groups = (int64_t)B * S;
+    group_bwd_xyz_kernel<<<ew_blocks(groups * 32, 256), 256, 0, (cudaStream_t)stream>>>(dgrouped, ldg, col0, idx, N, S, K, groups,
+                                                                                       dxyz, dnew_xyz);
+    return finish_launch("pn_group_bwd_xyz_f32");
+}
+
+PN_EXPORT int pn_three_interpolate_bwd_xyz_f32(const float* dx, int64_t ldx, int D1, int D2, const int64_t* idx,
+                                               const float* weight, const float* points2, int64_t p2B, int64_t p2S, int64_t p2C,
+                                               const float* xyz1, int64_t aB, int64_t aN, int64_t aC, const float* xyz2,
+                                               int64_t bB, int64_t bS, int64_t bC, int B, int N, int S, float* dpoints1,
+                                               float* dpoints2, float* dxyz1, float* dxyz2, pn_stream_t stream) {
+    PN_REQUIRE(dx && idx && weight && points2 && xyz1 && xyz2 && dpoints2 && dxyz1 && dxyz2 && (D1 == 0 || dpoints1),
+               PN_ERR_BAD_ARG, "pn_three_interpolate_bwd_xyz_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && D1 >= 0 && D2 > 0 && ldx >= D1 + D2, PN_ERR_BAD_ARG, "pn_three_interpolate_bwd_xyz_f32: bad shape");
+    // S == 1 is the broadcast of pointnet_util.py:292-293, whose weights (1, 0, 0) do not come from distances; S == 2 has no
+    // 3-NN forward (pn_three_nn_f32 needs S >= 3)
+    PN_REQUIRE(S >= 3, PN_ERR_BAD_ARG, "pn_three_interpolate_bwd_xyz_f32: need S >= 3 (got %d)", S);
+    const int64_t rows = (int64_t)B * N;
+    const bool vec = D1 % 4 == 0 && D2 % 4 == 0 && ldx % 4 == 0 && p2C == 1 && p2S % 4 == 0 && p2B % 4 == 0 &&
+                     ((uintptr_t)dx & 15) == 0 && ((uintptr_t)points2 & 15) == 0 && ((uintptr_t)dpoints2 & 15) == 0 &&
+                     ((uintptr_t)dpoints1 & 15) == 0;
+    const unsigned grid = (unsigned)ew_blocks(rows * 32, 256);
+    if (vec)
+        three_interpolate_bwd_xyz_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(
+            dx, ldx, D1, D2, idx, weight, points2, p2B, p2S, p2C, xyz1, aB, aN, aC, xyz2, bB, bS, bC, N, S, rows, dpoints1, dpoints2,
+            dxyz1, dxyz2);
+    else
+        three_interpolate_bwd_xyz_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(
+            dx, ldx, D1, D2, idx, weight, points2, p2B, p2S, p2C, xyz1, aB, aN, aC, xyz2, bB, bS, bC, N, S, rows, dpoints1, dpoints2,
+            dxyz1, dxyz2);
+    return finish_launch("pn_three_interpolate_bwd_xyz_f32");
 }
 
 PN_EXPORT int pn_dropout_f32(const float* x, int64_t ldx, int64_t rows, int C, float p, const uint64_t* seed_offset,

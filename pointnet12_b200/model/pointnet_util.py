@@ -281,10 +281,13 @@ class PointNetSetAbstraction(nn.Module):
 
     # The level splits into a geometry half (depends on xyz only: FPS + ball query) and a feature half
     # (grouping + MLP + max).  The networks run the geometry of all levels on side streams.
-    def geometry(self, xyz_pm: torch.Tensor, start_idx: Optional[torch.Tensor] = None):
-        """xyz_pm [B,N,3] -> (new_xyz [B,S,3], group_idx [B,S,K])."""
-        new_xyz = ops.index_points(xyz_pm, farthest_point_sample(xyz_pm, self.npoint, start_idx))
-        return new_xyz, ops.ball_query(self.radius, self.nsample, xyz_pm, new_xyz)
+    def geometry(self, xyz_pm: torch.Tensor, start_idx: Optional[torch.Tensor] = None, with_fps: bool = False):
+        """xyz_pm [B,N,3] -> (new_xyz [B,S,3], group_idx [B,S,K]), and fps_idx [B,S] as a third element when `with_fps`
+        (the training path differentiates new_xyz = xyz[fps_idx] when the coordinates require a gradient)."""
+        fps_idx = farthest_point_sample(xyz_pm, self.npoint, start_idx)
+        new_xyz = ops.index_points(xyz_pm, fps_idx)
+        idx = ops.ball_query(self.radius, self.nsample, xyz_pm, new_xyz)
+        return (new_xyz, idx, fps_idx) if with_fps else (new_xyz, idx)
 
     def features(self, xyz_pm, pts_pm, new_xyz, idx) -> torch.Tensor:
         """-> pooled [B,S,C'] point-major."""

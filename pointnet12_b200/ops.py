@@ -1026,6 +1026,43 @@ def three_interpolate_backward(dx: torch.Tensor, D1: int, D2: int, idx: torch.Te
     return dp1, dp2
 
 
+def group_backward_xyz(dgrouped: torch.Tensor, col0: int, idx: torch.Tensor, N: int, recentred: bool = True):
+    """Coordinate gradient of the grouping: dgrouped [B*S*K, >= col0+3] with the xyz_rel columns at col0 -> (dxyz [B,N,3],
+    dnew_xyz [B,S,3] = -sum over each group, or None when the group was not recentred (group-all))."""
+    dgrouped = _rowmat(dgrouped, "dgrouped")
+    idx = _i64(idx, "idx")
+    B, S, K = idx.shape
+    dxyz = torch.zeros((B, N, 3), dtype=torch.float32, device=dgrouped.device)
+    dnew = torch.empty((B, S, 3), dtype=torch.float32, device=dgrouped.device) if recentred else None
+    with _on_device(dgrouped):
+        nv.call("pn_group_bwd_xyz_f32", dgrouped.data_ptr(), _ld(dgrouped), int(col0), idx.data_ptr(), B, int(N), S, K,
+                dxyz.data_ptr(), _p(dnew), _stream())
+    return dxyz, dnew
+
+
+def three_interpolate_backward_xyz(dx: torch.Tensor, D1: int, D2: int, idx: torch.Tensor, weight: torch.Tensor,
+                                   points2: torch.Tensor, xyz1: torch.Tensor, xyz2: torch.Tensor):
+    """three_interpolate_backward plus the gradient through the 3-NN weights: points2 [B,S,D2], xyz1 [B,N,3], xyz2 [B,S,3]
+    (the forward's inputs, any strides) -> (dpoints1 [B,N,D1] or None, dpoints2 [B,S,D2], dxyz1 [B,N,3], dxyz2 [B,S,3]).
+    Needs S >= 3."""
+    dx = _rowmat(dx, "dx")
+    idx = _i64(idx, "idx")
+    weight = _f32(weight, "weight").contiguous()
+    points2 = _cloud(points2, "points2")
+    xyz1, xyz2 = _cloud(xyz1, "xyz1", 3), _cloud(xyz2, "xyz2", 3)
+    B, N, _ = idx.shape
+    S = points2.shape[1]
+    dp1 = torch.empty((B, N, D1), dtype=torch.float32, device=dx.device) if D1 else None
+    dp2 = torch.zeros((B, S, D2), dtype=torch.float32, device=dx.device)
+    dxyz1 = torch.empty((B, N, 3), dtype=torch.float32, device=dx.device)
+    dxyz2 = torch.zeros((B, S, 3), dtype=torch.float32, device=dx.device)
+    with _on_device(dx):
+        nv.call("pn_three_interpolate_bwd_xyz_f32", dx.data_ptr(), _ld(dx), int(D1), int(D2), idx.data_ptr(), weight.data_ptr(),
+                points2.data_ptr(), *points2.stride(), xyz1.data_ptr(), *xyz1.stride(), xyz2.data_ptr(), *xyz2.stride(), B, N, S,
+                _p(dp1), dp2.data_ptr(), dxyz1.data_ptr(), dxyz2.data_ptr(), _stream())
+    return dp1, dp2, dxyz1, dxyz2
+
+
 def dropout(x: torch.Tensor, p: float, seed_offset: Optional[torch.Tensor] = None, mask: Optional[torch.Tensor] = None,
             want_mask: bool = True):
     """-> (y, mask uint8 [rows, C]).  mask given: applied as is (also the backward pass); else drawn from the Philox

@@ -246,7 +246,8 @@ def _rows_of(grad: torch.Tensor, C: int) -> torch.Tensor:
 class SetAbstractionFn(torch.autograd.Function):
     """Grouping + shared MLP (batch-stat BN) + max over nsample of PointNetSetAbstraction.forward
     (model/pointnet_util.py:187-199) or of one scale of PointNetSetAbstractionMsg.forward (:239-257; `branch` selects the
-    scale, channel order [features, xyz_rel]).  Sampling / ball query carry no gradient and are done by the caller."""
+    scale, channel order [features, xyz_rel]).  Sampling / ball query carry no gradient and are done by the caller; the
+    gather + recentring pass gradients to xyz_pm and new_xyz when they require one (pn_group_bwd_xyz_f32)."""
 
     @staticmethod
     def _layers(mod, branch):
@@ -271,20 +272,28 @@ class SetAbstractionFn(torch.autograd.Function):
     def backward(ctx, dpooled):
         B, N, S, K, D = ctx.geom
         layers = SetAbstractionFn._layers(ctx.mod, ctx.branch)
-        need_dx = D > 0 and ctx.needs_input_grad[3]
-        dx0, grads = mlp_backward(ctx.saved, layers, _rows_of(dpooled, dpooled.shape[-1]), K, need_dx, arena=ctx.arena)
+        need_dpts = D > 0 and ctx.needs_input_grad[3]
+        need_xyz = ctx.needs_input_grad[2] or ctx.needs_input_grad[4]
+        dx0, grads = mlp_backward(ctx.saved, layers, _rows_of(dpooled, dpooled.shape[-1]), K, need_dpts or need_xyz,
+                                  arena=ctx.arena)
         # the feature channels sit behind the three xyz columns (SSG order) or in front of them (MSG order)
-        dpts = ops.group_backward(dx0, 3 if ctx.branch is None else 0, D, ctx.idx, N) if need_dx else None
+        msg = ctx.branch is not None
+        dpts = ops.group_backward(dx0, 0 if msg else 3, D, ctx.idx, N) if need_dpts else None
+        dxyz = dnew = None
+        if need_xyz:
+            dxyz, dnew = ops.group_backward_xyz(dx0, D if msg else 0, ctx.idx, N, recentred=ctx.needs_input_grad[4])
         ctx.saved = None
-        return (None, None, None, dpts, None, None, *_layer_grads(layers, grads))
+        return (None, None, dxyz if ctx.needs_input_grad[2] else None, dpts, dnew, None, *_layer_grads(layers, grads))
 
 
 class FeaturePropagationFn(torch.autograd.Function):
     """Interpolation + skip concat + shared MLP (batch-stat BN) of PointNetFeaturePropagation.forward
-    (model/pointnet_util.py:301-312); the 3-NN search carries no gradient and is done by the caller."""
+    (model/pointnet_util.py:301-312); the 3-NN search (the choice of neighbours) carries no gradient and is done by the
+    caller.  xyz1 [B,N,3] / xyz2 [B,S,3] (point-major) receive the gradient through the interpolation weights when they
+    require one (pn_three_interpolate_bwd_xyz_f32)."""
 
     @staticmethod
-    def forward(ctx, mod, p1, p2, idx, w, *params):
+    def forward(ctx, mod, p1, p2, idx, w, xyz1, xyz2, *params):
         B, N, _ = idx.shape
         layers = [(c, b, True) for c, b in zip(mod.mlp_convs, mod.mlp_bns)]
         x0 = ops.three_interpolate(p1, p2, idx, w).view(B * N, -1)
@@ -292,6 +301,8 @@ class FeaturePropagationFn(torch.autograd.Function):
         out, saved = mlp_forward(x0, layers, arena=ctx.arena)
         ctx.mod, ctx.saved, ctx.nn = mod, saved, (idx, w)
         ctx.geom = (B, N, p2.shape[1], p1.shape[2] if p1 is not None else 0, p2.shape[2])
+        # the coordinate gradient goes through the 3-NN weights and needs the coarse features and both clouds
+        ctx.xyz = (p2, xyz1, xyz2) if ctx.needs_input_grad[5] or ctx.needs_input_grad[6] else None
         return out.view(B, N, -1)
 
     @staticmethod
@@ -300,9 +311,17 @@ class FeaturePropagationFn(torch.autograd.Function):
         B, N, S, D1, D2 = ctx.geom
         layers = [(c, b, True) for c, b in zip(mod.mlp_convs, mod.mlp_bns)]
         dx0, grads = mlp_backward(ctx.saved, layers, _rows_of(dout, dout.shape[-1]), None, True, arena=ctx.arena)
-        dp1, dp2 = ops.three_interpolate_backward(dx0, D1, D2, ctx.nn[0], ctx.nn[1], S)
-        ctx.saved = None
+        dxyz1 = dxyz2 = None
+        if ctx.xyz is not None and S > 1:
+            dp1, dp2, dxyz1, dxyz2 = ops.three_interpolate_backward_xyz(dx0, D1, D2, ctx.nn[0], ctx.nn[1], *ctx.xyz)
+        else:
+            dp1, dp2 = ops.three_interpolate_backward(dx0, D1, D2, ctx.nn[0], ctx.nn[1], S)
+            if ctx.xyz is not None:           # S == 1: the coarse point is broadcast (:292-293), no distance is involved
+                dxyz1 = torch.zeros((B, N, 3), dtype=torch.float32, device=dx0.device)
+                dxyz2 = torch.zeros((B, S, 3), dtype=torch.float32, device=dx0.device)
+        ctx.saved = ctx.xyz = None
         return (None, dp1 if ctx.needs_input_grad[1] else None, dp2 if ctx.needs_input_grad[2] else None, None, None,
+                dxyz1 if ctx.needs_input_grad[5] else None, dxyz2 if ctx.needs_input_grad[6] else None,
                 *_layer_grads(layers, grads))
 
 
@@ -573,9 +592,30 @@ def pointnet_seg_train(net, x: torch.Tensor):
 
 # ------------------------------------------------------------------------------------------------
 # train-mode forwards called by the modules (model/pointnet_util.py, model/pointnet2.py)
+class GatherPointsFn(torch.autograd.Function):
+    """new_xyz = index_points(xyz, fps_idx) of sample_and_group (pointnet_util.py:117) with its gradient w.r.t. xyz: the
+    scatter-add of pn_group_bwd_f32 through fps_idx seen as groups of one point."""
+
+    @staticmethod
+    def forward(ctx, xyz_pm, fps_idx):
+        ctx.fps_idx, ctx.N = fps_idx, xyz_pm.shape[1]
+        return ops.index_points(xyz_pm, fps_idx)
+
+    @staticmethod
+    def backward(ctx, dnew):
+        B, S = ctx.fps_idx.shape
+        return ops.group_backward(_rows_of(dnew, 3), 0, 3, ctx.fps_idx.view(B, S, 1), ctx.N), None
+
+
+def _wants_grad(t: Optional[torch.Tensor]) -> bool:
+    return t is not None and t.requires_grad and torch.is_grad_enabled()
+
+
 def set_abstraction_train(mod, xyz: torch.Tensor, points: Optional[torch.Tensor], start_idx=None, geometry=None):
-    """geometry: (new_xyz [B,S,3], group_idx [B,S,K]) when the caller has computed them already (side stream)."""
-    xyz_pm = xyz.detach().permute(0, 2, 1)
+    """geometry: (new_xyz [B,S,3], group_idx [B,S,K]) when the caller has computed them already (side stream), with
+    fps_idx [B,S] as a third element when xyz requires a gradient (new_xyz is then re-gathered differentiably)."""
+    grad_xyz = _wants_grad(xyz)
+    xyz_pm = (xyz if grad_xyz else xyz.detach()).permute(0, 2, 1)
     pts_pm = points.permute(0, 2, 1) if points is not None else None
     if mod.group_all:
         # sample_and_group_all (pointnet_util.py:140-157): one group holding every point, centroid = origin, no recentring
@@ -586,8 +626,12 @@ def set_abstraction_train(mod, xyz: torch.Tensor, points: Optional[torch.Tensor]
     else:
         if geometry is None:
             with torch.no_grad():
-                geometry = mod.geometry(xyz_pm, start_idx)
-        new_xyz, idx = geometry
+                geometry = mod.geometry(xyz_pm.detach(), start_idx, with_fps=grad_xyz)
+        new_xyz, idx = geometry[0], geometry[1]
+        if grad_xyz:
+            if len(geometry) < 3:
+                raise ValueError("set_abstraction_train: xyz requires a gradient, so the geometry must carry the FPS indices")
+            new_xyz = GatherPointsFn.apply(xyz_pm, geometry[2])
     layers = SetAbstractionFn._layers(mod, None)
     pooled = SetAbstractionFn.apply(mod, None, xyz_pm, pts_pm, new_xyz, idx, *_layer_params(layers))
     return new_xyz.permute(0, 2, 1), pooled.permute(0, 2, 1)
@@ -598,14 +642,16 @@ def set_abstraction_msg_train(mod, xyz: torch.Tensor, points: Optional[torch.Ten
     grouping ([features, xyz_rel]) -> shared MLP with batch statistics -> max; the scales are concatenated on the channels."""
     from .model.pointnet_util import farthest_point_sample
 
-    xyz_pm = xyz.detach().permute(0, 2, 1)
+    grad_xyz = _wants_grad(xyz)
+    xyz_pm = (xyz if grad_xyz else xyz.detach()).permute(0, 2, 1)
     pts_pm = points.permute(0, 2, 1) if points is not None else None
     with torch.no_grad():
-        new_xyz = ops.index_points(xyz_pm, farthest_point_sample(xyz_pm, mod.npoint, start_idx))
+        fps_idx = farthest_point_sample(xyz_pm.detach(), mod.npoint, start_idx)
+    new_xyz = GatherPointsFn.apply(xyz_pm, fps_idx) if grad_xyz else ops.index_points(xyz_pm, fps_idx)
     outs = []
     for i, radius in enumerate(mod.radius_list):
         with torch.no_grad():
-            idx = ops.ball_query(radius, mod.nsample_list[i], xyz_pm, new_xyz)
+            idx = ops.ball_query(radius, mod.nsample_list[i], xyz_pm.detach(), new_xyz.detach())
         layers = SetAbstractionFn._layers(mod, i)
         outs.append(SetAbstractionFn.apply(mod, i, xyz_pm, pts_pm, new_xyz, idx, *_layer_params(layers)))
     return new_xyz.permute(0, 2, 1), torch.cat(outs, dim=2).permute(0, 2, 1)
@@ -619,7 +665,8 @@ def feature_propagation_train(mod, xyz1, xyz2, points1, points2, geometry=None):
     idx, w = geometry
     p1 = points1.permute(0, 2, 1) if points1 is not None else None
     layers = [(c, b, True) for c, b in zip(mod.mlp_convs, mod.mlp_bns)]
-    out = FeaturePropagationFn.apply(mod, p1, points2.permute(0, 2, 1), idx, w, *_layer_params(layers))
+    out = FeaturePropagationFn.apply(mod, p1, points2.permute(0, 2, 1), idx, w, xyz1.permute(0, 2, 1), xyz2.permute(0, 2, 1),
+                                     *_layer_params(layers))
     return out.permute(0, 2, 1)
 
 
@@ -646,16 +693,18 @@ def dropout_seed(device) -> torch.Tensor:
 def semseg_geometry(net, points: torch.Tensor, fps_starts):
     """Everything of a PointNet2SemSeg forward that depends on the coordinates only (no gradient): sampling + ball query of
     the four set-abstraction levels and the four 3-NN searches, on the current stream.
-    -> ([(new_xyz [B,S,3], group_idx [B,S,K])] * 4, [(nn_idx [B,N,3], weight [B,N,3])] * 4 indexed like fp1..fp4)."""
+    -> ([(new_xyz [B,S,3], group_idx [B,S,K])] * 4, [(nn_idx [B,N,3], weight [B,N,3])] * 4 indexed like fp1..fp4); the
+    set-abstraction tuples also carry fps_idx [B,S] when `points` requires a gradient."""
     sa = [net.sa1, net.sa2, net.sa3, net.sa4]
     fp = [net.fp1, net.fp2, net.fp3, net.fp4]
+    with_fps = points.requires_grad
     with torch.no_grad():
         xs_pm = [points[:, :3, :].detach().permute(0, 2, 1)]
         sa_geo, fp_geo = [], [None] * 4
         for i, m in enumerate(sa):
-            new_xyz, idx = m.geometry(xs_pm[i], fps_starts[i])
-            xs_pm.append(new_xyz)
-            sa_geo.append((new_xyz, idx))
+            geo = m.geometry(xs_pm[i], fps_starts[i], with_fps=with_fps)
+            xs_pm.append(geo[0])
+            sa_geo.append(geo)
         for i in (3, 2, 1, 0):
             fp_geo[i] = fp[i].geometry(xs_pm[i], xs_pm[i + 1])
     return sa_geo, fp_geo
@@ -722,12 +771,13 @@ def _semseg_forward_train(net, points: torch.Tensor, fps_starts=None, dropout_ma
     capturing = torch.cuda.is_current_stream_capturing()
     sa_geo, fp_geo, sa_ready, fp_ready = [], [None] * 4, [], [None] * 4
     geo.wait_stream(user)
+    with_fps = _wants_grad(xyz)                                  # the coordinates' gradient needs the FPS indices
     with torch.no_grad(), torch.cuda.stream(geo):
         xs_pm = [xyz.detach().permute(0, 2, 1)]
         for i, m in enumerate(sa):
-            new_xyz, idx = m.geometry(xs_pm[i], fps_starts[i])
-            xs_pm.append(new_xyz)
-            sa_geo.append((new_xyz, idx))
+            level = m.geometry(xs_pm[i], fps_starts[i], with_fps=with_fps)
+            xs_pm.append(level[0])
+            sa_geo.append(level)
             ev = torch.cuda.Event()
             ev.record(geo)
             sa_ready.append(ev)
