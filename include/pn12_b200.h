@@ -346,6 +346,14 @@ int pn_bn_bwd_apply_f32(const float* y, int64_t ldy, int64_t rows, int C, const 
                         const int32_t* argmax, int K, const float* scale, const float* shift, const float* mean,
                         const float* invstd, int relu, const double* s1, const double* s2, float* dy, int64_t lddy,
                         float* dgamma, float* dbeta, pn_stream_t stream);
+/* Backward of act(bn(y)) when BatchNorm normalises with FIXED statistics (eval mode: scale, shift, mean, invstd from the
+ * running mean / variance), in one pass: g = dz * [y*scale+shift > 0] (relu; argmax != NULL: routed from the pooled
+ * gradient as in pn_bn_bwd_stats_f32), dy = scale*g, s1 += sum g, s2 += sum g*xhat with xhat = (y-mean)*invstd (fp64,
+ * zeroed by the caller), then dgamma += s2, dbeta += s1 (either may be NULL; accumulated like pn_bn_bwd_apply_f32). */
+int pn_bn_eval_bwd_f32(const float* y, int64_t ldy, int64_t rows, int C, const float* dz, int64_t lddz,
+                       const int32_t* argmax, int K, const float* scale, const float* shift, const float* mean,
+                       const float* invstd, int relu, double* s1, double* s2, float* dy, int64_t lddy, float* dgamma,
+                       float* dbeta, pn_stream_t stream);
 /* Weight gradient of a 1x1 conv: dw[co,ci] += sum_r dy[r,co]*x[r,ci], db[co] += sum_r dy[r,co] (db may be NULL).
  * Split over the rows, accumulated with fp32 atomics: dw / db must be zeroed (or hold a gradient to add to). */
 int pn_grad_weight_f32(const float* dy, int64_t lddy, const float* x, int64_t ldx, int64_t rows, int cout, int cin,
@@ -391,6 +399,15 @@ int pn_train_gemm_bnbwd_bf16x3(const float* dy, int64_t lddy, int64_t rows, int 
                                float* dz, int64_t lddz, const float* prev_y, int64_t ld_prev, const float* prev_scale,
                                const float* prev_shift, const float* prev_mean, const float* prev_invstd, double* s1, double* s2,
                                void* w_scratch, pn_stream_t stream);
+/* The same input-gradient GEMM when the layer below normalises with FIXED statistics (eval-mode BatchNorm: its scale, shift,
+ * mean, invstd from the running statistics): no batch coupling, so the epilogue stores that layer's dy_prev = scale*g
+ * (g = (dy W) * [prev_y*scale+shift > 0]) instead of dy W -- exactly what pn_bn_eval_bwd_f32 would write in a pass of its own
+ * -- adds sum g / sum g*xhat to s1 / s2 (fp64 [cout], zeroed by the caller), then dgamma += s2, dbeta += s1 (either may be
+ * NULL). */
+int pn_train_gemm_bneval_bf16x3(const float* dy, int64_t lddy, int64_t rows, int cin, const float* w, int w_transposed, int cout,
+                                float* dy_prev, int64_t ld_dy_prev, const float* prev_y, int64_t ld_prev, const float* prev_scale,
+                                const float* prev_shift, const float* prev_mean, const float* prev_invstd, double* s1, double* s2,
+                                float* dgamma, float* dbeta, void* w_scratch, pn_stream_t stream);
 /* out [cols, rows] = in [rows, cols]^T (the weight of the input-gradient GEMM dx = dy W = pn_linear_f32(dy, W^T)). */
 int pn_transpose_f32(const float* in, int rows, int cols, float* out, pn_stream_t stream);
 /* Backward of the gather of sample_and_group (model/pointnet_util.py:128-131): dfeat[b, idx[b,s,k], :] +=

@@ -81,6 +81,7 @@ _SIGNATURES = {
     "pn_bn_act_max_f32": [vp, i64, i64, i32, i32, vp, vp, i32, vp, i64, vp, vp],
     "pn_bn_bwd_stats_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp],
     "pn_bn_bwd_apply_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, vp, vp],
+    "pn_bn_eval_bwd_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, vp, vp],
     "pn_grad_weight_f32": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp],
     "pn_grad_weight_bf16x3": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp],
     "pn_grad_weight_bn_bf16x3": [vp, i64, vp, i64, vp, vp, i32, i64, i32, i32, vp, i64, vp, vp],
@@ -88,6 +89,7 @@ _SIGNATURES = {
     "pn_train_pack_many": [vp, i32, i32, i32, vp],
     "pn_train_gemm_bf16x3": [vp, i64, i64, i32, vp, vp, i32, vp, i32, vp, i32, vp, i64, vp, vp, vp, vp],
     "pn_train_gemm_bnbwd_bf16x3": [vp, i64, i64, i32, vp, i32, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp],
+    "pn_train_gemm_bneval_bf16x3": [vp, i64, i64, i32, vp, i32, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
     "pn_transpose_f32": [vp, i32, i32, vp, vp],
     "pn_group_bwd_f32": [vp, i64, i32, i32, vp, i32, i32, i32, i32, vp, vp],
     "pn_three_interpolate_bwd_f32": [vp, i64, i32, i32, vp, vp, i32, i32, i32, vp, vp, vp],

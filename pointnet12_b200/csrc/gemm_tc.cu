@@ -45,6 +45,7 @@ struct Args {
     int k_pad, n_pad, x_vec, debug, ns, na;
     // backward statistics in the epilogue (all NULL for the forward): the layer BELOW's pre-normalisation output and constants
     const float* py; int64_t ldpy; const float* p_scale; const float* p_shift; const float* p_mean; const float* p_invstd;
+    int p_eval;      // the layer below normalises with FIXED statistics: store its dy = scale*g instead of dz (pn_train_gemm_bneval_bf16x3)
     const unsigned char* w_packed;   // bf16 hi/lo image of the weights in the kernel's shared-memory layout (train_pack_kernel)
 };
 
@@ -87,6 +88,69 @@ __global__ void train_pack_many_kernel(const pn_train_pack_item* __restrict__ it
                  static_cast<unsigned char*>(it.out));
 }
 
+// The BatchNorm-backward terms of the layer BELOW for the 32 columns col0.. of one row: this GEMM's output v is dz of that
+// layer (gradient w.r.t. its activated output); with its pre-normalisation output yp: g = dz * [yp*scale+shift > 0],
+// xhat = (yp - mean) * invstd; f1 = g, f2 = g*xhat (the two sums its backward needs).  store_dy: v becomes scale*g.
+__device__ __forceinline__ void bwd_terms(const Args& a, const float* pc, int64_t row, bool row_ok, int col0, float (&v)[32],
+                                          float (&f1)[32], float (&f2)[32], bool store_dy) {
+    const float* __restrict__ ypr = a.py + row * a.ldpy + col0;
+    const bool vec = col0 + 32 <= a.cout && ((a.ldpy & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.py) & 15) == 0);
+#pragma unroll
+    for (int j = 0; j < 32; j += 4) {
+        float yp[4] = {0.f, 0.f, 0.f, 0.f};
+        if (row_ok) {
+            if (vec) {
+                const float4 t = __ldg(reinterpret_cast<const float4*>(ypr + j));
+                yp[0] = t.x; yp[1] = t.y; yp[2] = t.z; yp[3] = t.w;
+            } else {
+#pragma unroll
+                for (int i = 0; i < 4; ++i)
+                    if (col0 + j + i < a.cout) yp[i] = __ldg(ypr + j + i);
+            }
+        }
+        const float4 sc = *reinterpret_cast<const float4*>(pc + col0 + j);
+        const float4 sh = *reinterpret_cast<const float4*>(pc + a.n_pad + col0 + j);
+        const float4 mu = *reinterpret_cast<const float4*>(pc + 2 * a.n_pad + col0 + j);
+        const float4 is = *reinterpret_cast<const float4*>(pc + 3 * a.n_pad + col0 + j);
+        const float scv[4] = {sc.x, sc.y, sc.z, sc.w}, shv[4] = {sh.x, sh.y, sh.z, sh.w};
+        const float muv[4] = {mu.x, mu.y, mu.z, mu.w}, isv[4] = {is.x, is.y, is.z, is.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const float g = (row_ok && fmaf(yp[i], scv[i], shv[i]) > 0.0f) ? v[j + i] : 0.0f;
+            f1[j + i] = g;
+            f2[j + i] = g * ((yp[i] - muv[i]) * isv[i]);
+            if (store_dy) v[j + i] = scv[i] * g;
+        }
+    }
+}
+
+// Column sums of f1 / f2 over a warp's 32 rows added to the CTA's shared-memory sums s1 / s2 (32 columns each): the
+// butterfly's first three steps (16 + 8 + 4 columns exchanged: afterwards a lane holds 4 columns summed over 8 rows) in fp32,
+// the last two and everything beyond in fp64.  Four warps meet per column; one global atomic per column and CTA at the end.
+__device__ __forceinline__ void reduce_into(float (&f1)[32], float (&f2)[32], int lane, double* s1, double* s2) {
+    const auto add = [](auto x, auto y) { return x + y; };
+    tc::col_butterfly<16, 4>(f1, lane, add);
+    tc::col_butterfly<16, 4>(f2, lane, add);
+    double d1[32], d2[32];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) { d1[j] = (double)f1[j]; d2[j] = (double)f2[j]; }
+    tc::col_butterfly<2, 1>(d1, lane, add);
+    tc::col_butterfly<2, 1>(d2, lane, add);
+    atomicAdd(&s1[lane], d1[0]);
+    atomicAdd(&s2[lane], d2[0]);
+}
+
+// dgamma += s2, dbeta += s1 (either may be NULL) after pn_train_gemm_bneval_bf16x3.
+__global__ void bneval_finalize_kernel(const double* __restrict__ s1, const double* __restrict__ s2, int C, float* __restrict__ dgamma,
+                                       float* __restrict__ dbeta) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    if (dgamma) dgamma[c] += (float)s2[c];
+    if (dbeta) dbeta[c] += (float)s1[c];
+}
+
+// EVAL: the eval-mode epilogue (Args::p_eval), a separate instantiation so that the training GEMM's registers are not shared
+template <bool EVAL>
 __global__ void __launch_bounds__(THREADS, 2)
 train_gemm_kernel(const Args a) {
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -282,6 +346,13 @@ train_gemm_kernel(const Args a) {
                     v[j + 3] = __uint_as_float(r[j + 3]) + bb.w;
                 }
                 if ((a.debug & 2) && v[0] != 12345.678f) continue;
+                if (EVAL) {
+                    // fixed statistics below: g and g*xhat as in the branch further down, their sums first, then the stored
+                    // value is the layer below's dy = scale*g (no BatchNorm pass of its own)
+                    float f1[32], f2[32];
+                    bwd_terms(a, pc, row, row_ok, col0, v, f1, f2, true);
+                    reduce_into(f1, f2, lane, cta_sum + col0, cta_sum + a.n_pad + col0);
+                }
                 if (!(a.debug & 64)) {
                     if (col0 + 32 <= a.cout && ((a.ldy & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.y) & 15) == 0)) {
                         // A thread owns a ROW of the accumulator, so storing straight from registers makes every store
@@ -313,42 +384,12 @@ train_gemm_kernel(const Args a) {
                             if (col0 + j < a.cout) dst[j] = v[j];
                     }
                 }
-                if (a.col_sum && !(a.debug & 32)) {
+                if (!EVAL && a.col_sum && !(a.debug & 32)) {
                     // column sums over the warp's 32 rows: the butterfly's first three steps (16 + 8 + 4 columns exchanged:
                     // afterwards a lane holds 4 columns summed over 8 rows) in fp32, the last two and everything beyond in fp64
                     float f1[32], f2[32];
                     if (a.py) {
-                        // BACKWARD statistics: this GEMM's output is dz of the layer below (gradient w.r.t. its activated
-                        // output); with that layer's pre-normalisation output yp: g = dz * [yp*scale+shift > 0],
-                        // xhat = (yp - mean) * invstd, and the two sums its BatchNorm backward needs are sum g, sum g*xhat
-                        const float* __restrict__ ypr = a.py + row * a.ldpy + col0;
-                        const bool vec = col0 + 32 <= a.cout && ((a.ldpy & 3) == 0) && ((reinterpret_cast<uintptr_t>(a.py) & 15) == 0);
-#pragma unroll
-                        for (int j = 0; j < 32; j += 4) {
-                            float yp[4] = {0.f, 0.f, 0.f, 0.f};
-                            if (row_ok) {
-                                if (vec) {
-                                    const float4 t = __ldg(reinterpret_cast<const float4*>(ypr + j));
-                                    yp[0] = t.x; yp[1] = t.y; yp[2] = t.z; yp[3] = t.w;
-                                } else {
-#pragma unroll
-                                    for (int i = 0; i < 4; ++i)
-                                        if (col0 + j + i < a.cout) yp[i] = __ldg(ypr + j + i);
-                                }
-                            }
-                            const float4 sc = *reinterpret_cast<const float4*>(pc + col0 + j);
-                            const float4 sh = *reinterpret_cast<const float4*>(pc + a.n_pad + col0 + j);
-                            const float4 mu = *reinterpret_cast<const float4*>(pc + 2 * a.n_pad + col0 + j);
-                            const float4 is = *reinterpret_cast<const float4*>(pc + 3 * a.n_pad + col0 + j);
-                            const float scv[4] = {sc.x, sc.y, sc.z, sc.w}, shv[4] = {sh.x, sh.y, sh.z, sh.w};
-                            const float muv[4] = {mu.x, mu.y, mu.z, mu.w}, isv[4] = {is.x, is.y, is.z, is.w};
-#pragma unroll
-                            for (int i = 0; i < 4; ++i) {
-                                const float g = (row_ok && fmaf(yp[i], scv[i], shv[i]) > 0.0f) ? v[j + i] : 0.0f;
-                                f1[j + i] = g;
-                                f2[j + i] = g * ((yp[i] - muv[i]) * isv[i]);
-                            }
-                        }
+                        bwd_terms(a, pc, row, row_ok, col0, v, f1, f2, false);
                     } else {
                         // FORWARD statistics, shifted by a per-column pivot p (the CTA's first row): sum (y-p), sum (y-p)^2.
                         // Unshifted, the fp32 square would carry a rounding of |mean|^2 * 2^-24 that does not average out
@@ -373,18 +414,7 @@ train_gemm_kernel(const Args a) {
                             }
                         }
                     }
-                    const auto add = [](auto x, auto y) { return x + y; };
-                    tc::col_butterfly<16, 4>(f1, lane, add);
-                    tc::col_butterfly<16, 4>(f2, lane, add);
-                    double d1[32], d2[32];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) { d1[j] = (double)f1[j]; d2[j] = (double)f2[j]; }
-                    tc::col_butterfly<2, 1>(d1, lane, add);
-                    tc::col_butterfly<2, 1>(d2, lane, add);
-                    // per-CTA accumulation in shared memory (four warps meet per column); one global atomic per column
-                    // and CTA at the very end instead of one per tile
-                    atomicAdd(&cta_sum[col0 + lane], d1[0]);
-                    atomicAdd(&cta_sum[a.n_pad + col0 + lane], d2[0]);
+                    reduce_into(f1, f2, lane, cta_sum + col0, cta_sum + a.n_pad + col0);
                 }
             }
         }
@@ -442,7 +472,8 @@ PN_EXPORT size_t pn_train_gemm_scratch_bytes(int cin, int cout) {
 static int train_gemm_launch(const float* x, int64_t ldx, int64_t rows, int cin, const float* in_scale, const float* in_shift,
                              int in_relu, const float* w, int w_transposed, const float* bias, int cout, float* y, int64_t ldy,
                              double* col_sum, double* col_sumsq, const float* py, int64_t ldpy, const float* p_scale,
-                             const float* p_shift, const float* p_mean, const float* p_invstd, void* w_scratch, pn_stream_t stream);
+                             const float* p_shift, const float* p_mean, const float* p_invstd, void* w_scratch, pn_stream_t stream,
+                             int p_eval = 0);
 
 PN_EXPORT int pn_train_gemm_bf16x3(const float* x, int64_t ldx, int64_t rows, int cin, const float* in_scale,
                                    const float* in_shift, int in_relu, const float* w, int w_transposed, const float* bias,
@@ -463,10 +494,26 @@ PN_EXPORT int pn_train_gemm_bnbwd_bf16x3(const float* dy, int64_t lddy, int64_t 
                              prev_scale, prev_shift, prev_mean, prev_invstd, w_scratch, stream);
 }
 
+PN_EXPORT int pn_train_gemm_bneval_bf16x3(const float* dy, int64_t lddy, int64_t rows, int cin, const float* w, int w_transposed,
+                                          int cout, float* dy_prev, int64_t ld_dy_prev, const float* prev_y, int64_t ld_prev,
+                                          const float* prev_scale, const float* prev_shift, const float* prev_mean,
+                                          const float* prev_invstd, double* s1, double* s2, float* dgamma, float* dbeta,
+                                          void* w_scratch, pn_stream_t stream) {
+    PN_REQUIRE(dy_prev && prev_y && prev_scale && prev_shift && prev_mean && prev_invstd && s1 && s2, PN_ERR_BAD_ARG,
+               "pn_train_gemm_bneval_bf16x3: null pointer");
+    PN_REQUIRE(ld_prev >= cout, PN_ERR_BAD_ARG, "pn_train_gemm_bneval_bf16x3: ld_prev smaller than cout");
+    const int rc = train_gemm_launch(dy, lddy, rows, cin, nullptr, nullptr, 0, w, w_transposed, nullptr, cout, dy_prev, ld_dy_prev, s1, s2,
+                                     prev_y, ld_prev, prev_scale, prev_shift, prev_mean, prev_invstd, w_scratch, stream, 1);
+    if (rc != 0 || !(dgamma || dbeta)) return rc;
+    pn::gemm::bneval_finalize_kernel<<<(unsigned)pn::ceil_div(cout, 128), 128, 0, (cudaStream_t)stream>>>(s1, s2, cout, dgamma, dbeta);
+    return pn::finish_launch("pn_train_gemm_bneval_bf16x3");
+}
+
 static int train_gemm_launch(const float* x, int64_t ldx, int64_t rows, int cin, const float* in_scale, const float* in_shift,
                              int in_relu, const float* w, int w_transposed, const float* bias, int cout, float* y, int64_t ldy,
                              double* col_sum, double* col_sumsq, const float* py, int64_t ldpy, const float* p_scale,
-                             const float* p_shift, const float* p_mean, const float* p_invstd, void* w_scratch, pn_stream_t stream) {
+                             const float* p_shift, const float* p_mean, const float* p_invstd, void* w_scratch, pn_stream_t stream,
+                             int p_eval) {
     using namespace pn;
     using namespace pn::gemm;
     PN_REQUIRE(x && y && w_scratch, PN_ERR_BAD_ARG, "pn_train_gemm_bf16x3: null pointer");
@@ -481,6 +528,7 @@ static int train_gemm_launch(const float* x, int64_t ldx, int64_t rows, int cin,
     a.in_scale = in_scale; a.in_shift = in_shift; a.in_relu = in_relu;
     a.w = w; a.w_transposed = w_transposed; a.bias = bias; a.cout = cout;
     a.y = y; a.ldy = ldy; a.col_sum = col_sum; a.col_sumsq = col_sumsq;
+    a.p_eval = p_eval;
     a.py = py; a.ldpy = ldpy; a.p_scale = p_scale; a.p_shift = p_shift; a.p_mean = p_mean; a.p_invstd = p_invstd;
     a.k_pad = round_up(cin, KC);
     a.n_pad = round_up(cout, 32);
@@ -513,7 +561,8 @@ static int train_gemm_launch(const float* x, int64_t ldx, int64_t rows, int cin,
         if (sms <= 0) sms = 148;
     }
     if (smem > smem_set) {
-        cudaError_t e = cudaFuncSetAttribute(train_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(train_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(train_gemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) {
             cudaGetLastError();
             set_error("pn_train_gemm_bf16x3: cannot reserve %zu bytes of shared memory: %s", smem, cudaGetErrorString(e));
@@ -529,6 +578,9 @@ static int train_gemm_launch(const float* x, int64_t ldx, int64_t rows, int cin,
     }
     const int64_t tiles = ceil_div(rows, TM);
     const int64_t grid = tiles < (int64_t)sms * per_sm ? tiles : (int64_t)sms * per_sm;
-    train_gemm_kernel<<<(unsigned)grid, THREADS, smem, (cudaStream_t)stream>>>(a);
+    if (p_eval)
+        train_gemm_kernel<true><<<(unsigned)grid, THREADS, smem, (cudaStream_t)stream>>>(a);
+    else
+        train_gemm_kernel<false><<<(unsigned)grid, THREADS, smem, (cudaStream_t)stream>>>(a);
     return finish_launch("pn_train_gemm_bf16x3");
 }

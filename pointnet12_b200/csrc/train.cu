@@ -17,6 +17,8 @@
 //   backward  pn_log_softmax_bwd_f32, pn_dropout_f32 (mask reuse)
 //             pn_bn_bwd_stats_f32                 sum(g), sum(g*xhat) with g = dz * [z > 0] (pooled: routed by arg-max)
 //             pn_bn_bwd_apply_f32                 dy = gamma*invstd*(g - mean(g) - xhat*mean(g*xhat)); dgamma, dbeta
+//             pn_bn_eval_bwd_f32                  eval-mode BatchNorm (running statistics): dy = scale*g, dgamma, dbeta
+//                                                 in one pass (no batch coupling)
 //             pn_grad_weight_f32                  dW += dy^T x, db += sum(dy)     (split over the rows, fp32 atomics)
 //             pn_linear_f32 on W^T (pn_transpose_f32)   dx = dy W
 //             pn_group_bwd_f32, pn_three_interpolate_bwd_f32    scatter-add through the gathers
@@ -235,6 +237,60 @@ __global__ void bn_bwd_apply_kernel(const float* __restrict__ y, int64_t ldy, in
         const float m1 = (float)(s1[c] * inv_n), m2 = (float)(s2[c] * inv_n);
         dy[r * lddy + c] = sc * (g - m1 - xh * m2);      // scale = gamma * invstd
     }
+}
+
+// Backward of act(bn(y)) with FIXED statistics (eval-mode BatchNorm: running mean / variance), one pass: the statistics
+// do not depend on the batch, so dy = scale*g needs no column reduction first.  g = dz * [y*scale+shift > 0] (POOLED:
+// routed from dz[row/K] by the arg-max of bn_act_max, either layout); dy = scale*g; s1 += sum g, s2 += sum g*xhat with
+// xhat = (y-mean)*invstd (fp64 per block, one atomic per column per block).  Same block shape as col_stats_kernel.
+template <bool POOLED>
+__global__ void __launch_bounds__(32 * ST_LANES)
+bn_eval_bwd_kernel(const float* __restrict__ y, int64_t ldy, int64_t rows, int C, int64_t rows_per_block,
+                   const float* __restrict__ dz, int64_t lddz, const int32_t* __restrict__ argmax, int K,
+                   const float* __restrict__ scale, const float* __restrict__ shift, const float* __restrict__ mean,
+                   const float* __restrict__ invstd, int relu, double* __restrict__ s1, double* __restrict__ s2,
+                   float* __restrict__ dy, int64_t lddy) {
+    __shared__ double r1[ST_LANES][33], r2[ST_LANES][33];
+    const int lane = threadIdx.x & 31, ry = threadIdx.x >> 5;
+    const int c = blockIdx.y * 32 + lane;
+    const int64_t r0 = (int64_t)blockIdx.x * rows_per_block;
+    const int64_t r1e = min(rows, r0 + rows_per_block);
+    double a1 = 0.0, a2 = 0.0;
+    if (c < C) {
+        const float sc = scale[c], sh = shift[c], mu = mean[c], is = invstd[c];
+        for (int64_t r = r0 + ry; r < r1e; r += ST_LANES) {
+            const float v = y[r * ldy + c];
+            float g;
+            if (!POOLED) {
+                g = dz[r * lddz + c];
+            } else {
+                const int64_t grp = r / K;
+                g = (argmax[grp * C + c] == (int)(r - grp * K)) ? dz[grp * lddz + c] : 0.0f;
+            }
+            if (relu && !(fmaf(v, sc, sh) > 0.0f)) g = 0.0f;
+            dy[r * lddy + c] = sc * g;
+            a1 += (double)g;
+            a2 = fma((double)g, (double)((v - mu) * is), a2);
+        }
+    }
+    r1[ry][lane] = a1;
+    r2[ry][lane] = a2;
+    __syncthreads();
+    if (ry == 0 && c < C) {
+#pragma unroll
+        for (int i = 1; i < ST_LANES; ++i) { a1 += r1[i][lane]; a2 += r2[i][lane]; }
+        atomicAdd(&s1[c], a1);
+        atomicAdd(&s2[c], a2);
+    }
+}
+
+// dgamma += s2, dbeta += s1 (either may be NULL): the affine gradients of the fixed-statistics backward.
+__global__ void bn_eval_bwd_finalize_kernel(const double* __restrict__ s1, const double* __restrict__ s2, int C,
+                                            float* __restrict__ dgamma, float* __restrict__ dbeta) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    if (dgamma) dgamma[c] += (float)s2[c];
+    if (dbeta) dbeta[c] += (float)s1[c];
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -855,6 +911,27 @@ PN_EXPORT int pn_bn_bwd_apply_f32(const float* y, int64_t ldy, int64_t rows, int
         bn_bwd_apply_kernel<1><<<blocks, 256, 0, st>>>(y, ldy, rows, C, dz, lddz, nullptr, 1, scale, shift, mean, invstd, relu, s1,
                                                        s2, dy, lddy, dgamma, dbeta);
     return finish_launch("pn_bn_bwd_apply_f32");
+}
+
+PN_EXPORT int pn_bn_eval_bwd_f32(const float* y, int64_t ldy, int64_t rows, int C, const float* dz, int64_t lddz,
+                                 const int32_t* argmax, int K, const float* scale, const float* shift, const float* mean,
+                                 const float* invstd, int relu, double* s1, double* s2, float* dy, int64_t lddy,
+                                 float* dgamma, float* dbeta, pn_stream_t stream) {
+    PN_REQUIRE(y && dz && scale && shift && mean && invstd && s1 && s2 && dy, PN_ERR_BAD_ARG, "pn_bn_eval_bwd_f32: null pointer");
+    PN_REQUIRE(rows > 0 && C > 0 && ldy >= C && lddz >= C && lddy >= C, PN_ERR_BAD_ARG, "pn_bn_eval_bwd_f32: bad shape");
+    PN_REQUIRE(!argmax || (K > 0 && rows % K == 0), PN_ERR_BAD_ARG, "pn_bn_eval_bwd_f32: rows must be a multiple of K");
+    dim3 grid;
+    int64_t rpb;
+    stats_grid(rows, C, &grid, &rpb);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (argmax)
+        bn_eval_bwd_kernel<true><<<grid, 32 * ST_LANES, 0, st>>>(y, ldy, rows, C, rpb, dz, lddz, argmax, K, scale, shift, mean,
+                                                                invstd, relu, s1, s2, dy, lddy);
+    else
+        bn_eval_bwd_kernel<false><<<grid, 32 * ST_LANES, 0, st>>>(y, ldy, rows, C, rpb, dz, lddz, nullptr, 1, scale, shift, mean,
+                                                                 invstd, relu, s1, s2, dy, lddy);
+    if (dgamma || dbeta) bn_eval_bwd_finalize_kernel<<<(unsigned)ceil_div(C, 128), 128, 0, st>>>(s1, s2, C, dgamma, dbeta);
+    return finish_launch("pn_bn_eval_bwd_f32");
 }
 
 PN_EXPORT int pn_grad_weight_f32(const float* dy, int64_t lddy, const float* x, int64_t ldx, int64_t rows, int cout,

@@ -13,7 +13,8 @@ reference.  Everything is computed on point-major rows [B*N, C] by the C-ABI ker
     same for every point of a cloud, so that half of conv1 becomes a per-cloud bias
     (bias_bstride) and the per-point work drops from 1088 to 64 input channels.
 
-Inference only (train() mode raises); no CPU fallback.
+In train() mode, and in eval() mode on an input that requires a gradient, the nets and their spatial transformers /
+encoder run on the autograd blocks of pointnet12_b200/train.py instead; no CPU fallback.
 """
 from __future__ import annotations
 
@@ -23,7 +24,7 @@ import torch
 import torch.nn as nn
 
 from .. import ops
-from .pointnet_util import FoldedLayers, _eval_only
+from .pointnet_util import FoldedLayers, autograd_path
 
 
 def _chain_global_max(folded: FoldedLayers, convs, bns, relus, rows: torch.Tensor, B: int, N: int) -> Optional[torch.Tensor]:
@@ -126,7 +127,11 @@ class _STN(nn.Module):
         return out
 
     def forward(self, x):
-        _eval_only(self)
+        if autograd_path(self, x):        # autograd blocks (pointnet12_b200/train.py)
+            from ..train import stn_train
+
+            ops._need_cuda(x, "input")
+            return stn_train(self, x.permute(0, 2, 1))
         return self.transform_rows(_point_rows(x))
 
 
@@ -186,9 +191,14 @@ class PointNetEncoder(nn.Module):
         return g, pointfeat, trans, trans_feat
 
     def forward(self, x):
-        _eval_only(self)
         B, _, N = x.shape
-        g, pointfeat, trans, trans_feat = self.encode_rows(_point_rows(x))
+        if autograd_path(self, x):        # autograd blocks (pointnet12_b200/train.py)
+            from ..train import pointnet_encoder_train
+
+            ops._need_cuda(x, "input")
+            g, pointfeat, trans, trans_feat = pointnet_encoder_train(self, x.permute(0, 2, 1))
+        else:
+            g, pointfeat, trans, trans_feat = self.encode_rows(_point_rows(x))
         if self.global_feat:
             return g, trans, trans_feat
         cat = torch.cat([g.view(B, 1024, 1).expand(B, 1024, N), pointfeat.permute(0, 2, 1)], 1)   # API parity only
@@ -212,7 +222,7 @@ class PointNetCls(nn.Module):
         self._folded = FoldedLayers()
 
     def forward(self, x, dropout_mask=None):
-        if self.training:
+        if autograd_path(self, x):
             from ..train import pointnet_cls_train
 
             return pointnet_cls_train(self, x, dropout_mask)
@@ -242,7 +252,7 @@ class PointNetSeg(nn.Module):
         self._folded_tail = FoldedLayers()
 
     def forward(self, x):
-        if self.training:          # batch-statistics BatchNorm + autograd (pointnet12_b200/train.py), pcdseg.py:166-186
+        if autograd_path(self, x):          # autograd blocks (pointnet12_b200/train.py), pcdseg.py:166-186
             from ..train import pointnet_seg_train
 
             return pointnet_seg_train(self, x)
@@ -323,7 +333,7 @@ class PointNetDenseCls(nn.Module):
         self._folded = FoldedLayers()
 
     def forward(self, point_cloud, label, dropout_mask=None):
-        if self.training:
+        if autograd_path(self, point_cloud, label):
             from ..train import pointnet_densecls_train
 
             return pointnet_densecls_train(self, point_cloud, label, dropout_mask)

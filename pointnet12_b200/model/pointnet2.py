@@ -14,7 +14,7 @@ import torch.nn as nn
 
 from .. import ops
 from .pointnet_util import (FoldedLayers, PointNetFeaturePropagation, PointNetSetAbstraction,
-                            PointNetSetAbstractionMsg, _eval_only, draw_fps_starts, farthest_point_sample)
+                            PointNetSetAbstractionMsg, _eval_only, autograd_path, draw_fps_starts, farthest_point_sample)
 
 
 def _ssg(npoint, radius, nsample, in_channel, mlp):
@@ -125,7 +125,7 @@ class PointNet2ClsMsg(_Net):
 
     def forward(self, xyz, dropout_masks=None, fps_starts=None):
         _, fs = self._encode(("sa1", "sa2", "sa3"), xyz, None, fps_starts)
-        if self.training:          # batch-statistics BatchNorm, dropout, autograd (pointnet12_b200/train.py)
+        if autograd_path(self, xyz):          # autograd blocks (pointnet12_b200/train.py)
             from ..train import cls_head_train
 
             return cls_head_train(self, fs[3].reshape(xyz.shape[0], 1024), dropout_masks), fs[3]
@@ -144,7 +144,7 @@ class PointNet2ClsSsg(_Net):
 
     def forward(self, xyz, dropout_masks=None, fps_starts=None):
         _, fs = self._encode(("sa1", "sa2", "sa3"), xyz, None, fps_starts)
-        if self.training:
+        if autograd_path(self, xyz):
             from ..train import cls_head_train
 
             return cls_head_train(self, fs[3].reshape(xyz.shape[0], 1024), dropout_masks)
@@ -166,7 +166,7 @@ class PointNet2PartSegSsg(_Net):
         xs, fs = self._encode(("sa1", "sa2", "sa3"), xyz, None, fps_starts)
         f2 = self.fp3(xs[2], xs[3], fs[2], fs[3])
         f1 = self.fp2(xs[1], xs[2], fs[1], f2)
-        if self.training:
+        if autograd_path(self, xyz):
             from ..train import seg_head_train
 
             return seg_head_train(self, self.fp1(xyz, xs[1], None, f1), dropout_mask)
@@ -191,7 +191,7 @@ class PointNet2PartSegMsg_one_hot(_Net):
         f2 = self.fp3(xs[2], xs[3], fs[2], fs[3])
         f1 = self.fp2(xs[1], xs[2], fs[1], f2)
         skip = torch.cat([cls_label.view(B, 16, 1).expand(B, 16, N), xyz, norm_plt], 1)   # host-side glue [B,22,N]
-        if self.training:
+        if autograd_path(self, xyz, norm_plt, cls_label):
             from ..train import seg_head_train
 
             return seg_head_train(self, self.fp1(xyz, xs[1], skip, f1), dropout_mask)[0]
@@ -225,8 +225,10 @@ class PointNet2SemSeg(_Net):
         (answered on the idle SMs WHILE level-1 sampling runs), sampling / grouping of levels 2-4, the 3-NN searches --
         runs on internal side streams beside the critical path FPS1 -> sa1..sa4 -> fp4..fp1; fp1 and the
         segmentation head run as one tensor-core chain whose first layer is folded into fp2's chain."""
-        if self.training:
-            from ..train import semseg_forward_train        # SURVEY 8 f-1: batch-stat BN, dropout, autograd
+        if autograd_path(self, points):
+            from ..train import semseg_forward_train        # SURVEY 8 f-1: the autograd blocks
+            if host_out is not None and torch.is_grad_enabled() and points.requires_grad:
+                raise ValueError("PointNet2SemSeg: host_out cannot be combined with an input that requires a gradient")
             return semseg_forward_train(self, points, fps_starts)
         ops._need_cuda(points, "points")
         B, _, N = points.shape

@@ -256,6 +256,16 @@ def _eval_only(module: nn.Module) -> None:
             "(BatchNorm is folded from running statistics); call .eval() first")
 
 
+def autograd_path(module: nn.Module, *inputs) -> bool:
+    """Whether a module runs on the autograd blocks of pointnet12_b200/train.py: in training mode, and in eval mode when grad
+    mode is on and one of its floating-point inputs requires a gradient -- there BatchNorm normalises with its running
+    statistics and dropout is the identity, as in the torch modules.  Otherwise the fused eval forward runs (no grad_fn)."""
+    if module.training:
+        return True
+    return torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.is_floating_point() and t.requires_grad
+                                           for t in inputs)
+
+
 def _mlp_rows(rows: torch.Tensor, layers) -> torch.Tensor:
     for w, b in layers:
         rows = ops.linear(rows, w, b, relu=True)
@@ -313,8 +323,8 @@ class PointNetSetAbstraction(nn.Module):
     def forward(self, xyz: torch.Tensor, points: Optional[torch.Tensor], start_idx: Optional[torch.Tensor] = None):
         """xyz [B,3,N], points [B,D,N] or None -> new_xyz [B,3,S], new_points [B,C',S].
         `start_idx` (extension): the FPS start indices, when the caller has already drawn them."""
-        if self.training:
-            from ..train import set_abstraction_train      # batch-statistics BatchNorm + autograd (SURVEY 8 f-1)
+        if autograd_path(self, xyz, points):
+            from ..train import set_abstraction_train      # autograd blocks (SURVEY 8 f-1)
             return set_abstraction_train(self, xyz, points, start_idx)
         xyz_pm = xyz.permute(0, 2, 1)
         pts_pm = points.permute(0, 2, 1) if points is not None else None
@@ -358,7 +368,7 @@ class PointNetSetAbstractionMsg(nn.Module):
         self._folded = [FoldedLayers() for _ in mlp_list]
 
     def forward(self, xyz: torch.Tensor, points: Optional[torch.Tensor], start_idx: Optional[torch.Tensor] = None):
-        if self.training:
+        if autograd_path(self, xyz, points):
             from ..train import set_abstraction_msg_train
 
             return set_abstraction_msg_train(self, xyz, points, start_idx)
@@ -550,7 +560,7 @@ class PointNetFeaturePropagation(nn.Module):
 
     def forward(self, xyz1, xyz2, points1, points2):
         """xyz1 [B,3,N], xyz2 [B,3,S], points1 [B,D1,N] or None, points2 [B,D2,S] -> [B,D',N]."""
-        if self.training:
+        if autograd_path(self, xyz1, xyz2, points1, points2):
             from ..train import feature_propagation_train
             return feature_propagation_train(self, xyz1, xyz2, points1, points2)
         idx, w = self.geometry(xyz1.permute(0, 2, 1), xyz2.permute(0, 2, 1))

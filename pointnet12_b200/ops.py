@@ -817,9 +817,44 @@ def _rowmat(t: torch.Tensor, name: str) -> torch.Tensor:
 
 
 class BatchStats:
-    """Batch statistics of one BatchNorm layer in training mode: scale/shift for the forward, mean/invstd for the backward."""
+    """Statistics one BatchNorm layer normalises with: scale/shift for the forward, mean/invstd for the backward.
+    running=False: the batch's own (training mode); running=True: the module's running statistics (running_stats)."""
 
-    __slots__ = ("scale", "shift", "mean", "invstd", "rows")
+    __slots__ = ("scale", "shift", "mean", "invstd", "rows", "running")
+
+    def __init__(self):
+        self.running = False
+
+
+def uses_running_stats(bn) -> bool:
+    """nn.BatchNorm's rule: batch statistics in training mode or when the module keeps no running statistics."""
+    return not bn.training and bn.running_mean is not None and bn.running_var is not None
+
+
+def running_stats(bn) -> BatchStats:
+    """BatchStats from bn's running statistics, the expressions of fold_conv_bn: scale = gamma/sqrt(var+eps), shift =
+    beta - mean*scale, invstd = 1/sqrt(var+eps).  Nothing of bn is written.  Cached on the module until a parameter or buffer
+    changes (storage or version) -- a write that bypasses the version counter (through .data) is not seen, as with the folded
+    weights of the eval path; under CUDA-graph capture they are computed inside the graph instead, so that a replay
+    follows the parameters an optimizer has updated in place since."""
+    capturing = bn.running_mean.is_cuda and torch.cuda.is_current_stream_capturing()
+    tensors = (bn.weight, bn.bias, bn.running_mean, bn.running_var)
+    key = (float(bn.eps),) + tuple((t.data_ptr(), t._version) if t is not None else None for t in tensors)
+    cached = bn.__dict__.get("_pn_running_stats")
+    if cached is not None and cached[0] == key and not capturing:
+        return cached[1]
+    with torch.no_grad():
+        mean = bn.running_mean.detach().float()
+        root = torch.sqrt(bn.running_var.detach().float() + bn.eps)
+        invstd = 1.0 / root
+        scale = bn.weight.detach().float() / root if bn.weight is not None else invstd
+        shift = (bn.bias.detach().float() if bn.bias is not None else torch.zeros_like(mean)) - mean * scale
+        st = BatchStats()
+        st.scale, st.shift, st.mean, st.invstd = scale.contiguous(), shift.contiguous(), mean.contiguous(), invstd.contiguous()
+    st.rows, st.running = None, True
+    if not capturing:
+        bn.__dict__["_pn_running_stats"] = (key, st)
+    return st
 
 
 def bn_batch_stats(y: torch.Tensor, bn, momentum_update: bool = True) -> BatchStats:
@@ -917,6 +952,31 @@ def train_gemm_bnbwd(dy: torch.Tensor, w: torch.Tensor, prev_y: torch.Tensor, pr
     return dz
 
 
+def train_gemm_bneval(dy: torch.Tensor, w: torch.Tensor, prev_y: torch.Tensor, prev_st: BatchStats, acc: torch.Tensor,
+                      dgamma: Optional[torch.Tensor] = None, dbeta: Optional[torch.Tensor] = None, transposed: bool = True,
+                      packed: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """pn_train_gemm_bneval_bf16x3: the input-gradient GEMM dy @ W of a layer whose input came from a BatchNorm with FIXED
+    statistics prev_st (running_stats) applied to prev_y, with that BatchNorm's backward in the epilogue: returns the layer
+    below's dy = scale * g (what bn_eval_backward would return for dz = dy @ W), adds its affine gradients to dgamma / dbeta.
+    acc: float64 [2, C] scratch, ZEROED."""
+    dy = _rowmat(dy, "dy")
+    rows, cin = dy.shape
+    w = _f32(w, "w").contiguous()
+    cout = w.shape[1] if transposed else w.shape[0]
+    prev_y = _rowmat(prev_y, "prev_y")
+    if prev_y.shape != (rows, cout):
+        raise ValueError("prev_y must be [rows, cout]")
+    out = torch.empty((rows, cout), dtype=torch.float32, device=dy.device)
+    scratch = packed if packed is not None else torch.empty((int(nv.lib().pn_train_gemm_scratch_bytes(cin, cout)),),
+                                                            dtype=torch.uint8, device=dy.device)
+    with _on_device(dy):
+        nv.call("pn_train_gemm_bneval_bf16x3", dy.data_ptr(), _ld(dy), rows, cin, None if packed is not None else w.data_ptr(),
+                int(transposed), cout, out.data_ptr(), cout, prev_y.data_ptr(), _ld(prev_y), prev_st.scale.data_ptr(),
+                prev_st.shift.data_ptr(), prev_st.mean.data_ptr(), prev_st.invstd.data_ptr(), acc[0].data_ptr(), acc[1].data_ptr(),
+                _p(dgamma), _p(dbeta), scratch.data_ptr(), _stream())
+    return out
+
+
 def bn_act(y: torch.Tensor, st: BatchStats, relu: bool = True, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     y = _rowmat(y, "y")
     rows, Cc = y.shape
@@ -962,6 +1022,27 @@ def bn_act_backward(y: torch.Tensor, st: BatchStats, dz: torch.Tensor, relu: boo
         if not acc_ready:        # (acc_ready: the reductions were accumulated by the epilogue of train_gemm_bnbwd)
             nv.call("pn_bn_bwd_stats_f32", *common, _stream())
         nv.call("pn_bn_bwd_apply_f32", *common, dy.data_ptr(), Cc, dgamma.data_ptr(), dbeta.data_ptr(), _stream())
+    return (dy, dgamma, dbeta) if fresh else dy
+
+
+def bn_eval_backward(y: torch.Tensor, st: BatchStats, dz: torch.Tensor, relu: bool = True,
+                     argmax: Optional[torch.Tensor] = None, K: int = 1, dgamma: Optional[torch.Tensor] = None,
+                     dbeta: Optional[torch.Tensor] = None, acc: Optional[torch.Tensor] = None):
+    """pn_bn_eval_bwd_f32: backward of act(bn(y)) with fixed statistics (running_stats), one pass: dy = scale * g.
+    dgamma / dbeta and argmax / K as in bn_act_backward; acc: float64 [2, C] scratch, ZEROED."""
+    y, dz = _rowmat(y, "y"), _rowmat(dz, "dz")
+    rows, Cc = y.shape
+    if acc is None:
+        acc = torch.zeros((2, Cc), dtype=torch.float64, device=y.device)
+    dy = torch.empty((rows, Cc), dtype=torch.float32, device=y.device)
+    fresh = dgamma is None
+    if fresh:
+        dgb = torch.zeros((2, Cc), dtype=torch.float32, device=y.device)
+        dgamma, dbeta = dgb[0], dgb[1]
+    with _on_device(y):
+        nv.call("pn_bn_eval_bwd_f32", y.data_ptr(), _ld(y), rows, Cc, dz.data_ptr(), _ld(dz), _p(argmax), int(K),
+                st.scale.data_ptr(), st.shift.data_ptr(), st.mean.data_ptr(), st.invstd.data_ptr(), int(relu),
+                acc[0].data_ptr(), acc[1].data_ptr(), dy.data_ptr(), Cc, dgamma.data_ptr(), dbeta.data_ptr(), _stream())
     return (dy, dgamma, dbeta) if fresh else dy
 
 

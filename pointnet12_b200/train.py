@@ -8,7 +8,10 @@ The drop-in contract is the reference's own: in train() mode the modules of mode
 model/pointnet2.py and model/pointnet.py (both models pcdseg.py can train among them) return tensors that carry a grad_fn, so the reference's loop (torch loss, loss.backward(), any torch optimizer) runs
 unchanged; every kernel underneath -- forward with batch-statistics BatchNorm, dropout, and the whole backward -- is ours
 (csrc/train.cu + linear.cu + the sampling / grouping kernels of the inference path).  One torch.autograd.Function per
-block (set abstraction, feature propagation, segmentation head): autograd only connects them.
+block (set abstraction, feature propagation, segmentation head): autograd only connects them.  The same blocks serve eval()
+mode when an input requires a gradient (model/pointnet_util.autograd_path): every BatchNorm / Dropout module follows its own
+mode as in torch -- running statistics, left untouched, for a BatchNorm in .eval() (also frozen layers of a train() net), no
+dropout for a Dropout in .eval().
 
 On top of that, the pieces a B200-native training loop uses instead of the torch ones:
     cross_entropy(logp, target)    the reference's loss as one kernel (forward + gradient)
@@ -120,9 +123,22 @@ def _grad_sink(p: torch.Tensor, shape) -> Tuple[torch.Tensor, bool]:
     return torch.zeros(shape, dtype=torch.float32, device=p.device), False
 
 
+def _dropout_on(drop, mask: Optional[torch.Tensor] = None) -> bool:
+    """nn.Dropout's rule: applied in training mode only, when p > 0 or a keep-mask is given.  When it is not applied, no
+    dropout seed is drawn and a given mask is ignored."""
+    return drop.training and (float(drop.p) > 0.0 or mask is not None)
+
+
 FUSED_BN = os.environ.get("PN12_TRAIN_FUSED", "1") != "0"     # BatchNorm fused into the training GEMMs (pn_train_gemm_bf16x3)
 PACK_ONCE = os.environ.get("PN12_TRAIN_PACK_ONCE", "1") != "0"      # all weight images converted by one launch per iteration
 FUSED_BN_BWD = os.environ.get("PN12_TRAIN_FUSED_BWD", "0") != "0"   # BatchNorm-backward reductions in the input-gradient GEMM's epilogue
+
+
+# The eval-mode BatchNorm backward goes into the input-gradient GEMM's epilogue when the layer below has fewer channels than
+# this.  Measured on C2's layers (NVIDIA B200, profiles/r03_eval_grad_bench.json): the fused epilogue wins at 32 and 64
+# channels (sa1, sa2: 7-10 % per layer) and loses at 128 on the 192 000 rows of fp1 (188 vs 170 us: the epilogue, already
+# the GEMM's bottleneck at that width, then also reads the layer below's y), so 128-wide layers keep GEMM + one pass.
+BNEVAL_EPILOGUE_BELOW = 128
 
 
 def mlp_forward(x: torch.Tensor, layers: Sequence[Tuple], pool_K: Optional[int] = None, arena=None):
@@ -132,26 +148,36 @@ def mlp_forward(x: torch.Tensor, layers: Sequence[Tuple], pool_K: Optional[int] 
     Fused path (tensor-core mode, layers that fit pn_train_gemm_bf16x3): a layer is ONE kernel -- the GEMM applies the
     previous layer's normalise + ReLU while loading its operand and accumulates this layer's batch statistics in its
     epilogue -- plus the tiny finalize; only the pre-normalisation outputs y exist in memory.  `pending` is the BatchStats
-    still to be applied to the current x.  saved[l] = (x, pending-at-input, y, stats, relu, argmax)."""
+    still to be applied to the current x.  saved[l] = (x, pending-at-input, y, stats, relu, argmax).
+    A BatchNorm in eval mode (ops.uses_running_stats) normalises with its running statistics, which it leaves untouched:
+    the GEMM accumulates no column sums for it and nothing is finalized."""
     saved = []
     pending = None
     rows = x.shape[0]
     widest = max(c.weight.shape[0] for c, _, _ in layers)
-    accs = torch.zeros((len(layers), 2, widest), dtype=torch.float64, device=x.device)     # one fill for the block's statistics
+    accs = None
     for li, (conv, bn, relu) in enumerate(layers):
         w = _w2d(conv)
         bias = conv.bias.detach() if conv.bias is not None else None
         fused = (FUSED_BN and bn is not None and ops.mlp_mode() == "bf16x3"
                  and ops.train_gemm_supported(w.shape[1], w.shape[0]))
+        running = bn is not None and ops.uses_running_stats(bn)
         st, am = None, None
         if bn is not None and not relu and li != len(layers) - 1:
             # (a BatchNorm without ReLU is supported as the LAST layer of a chain only: PointNetEncoder's bn3 ahead of the max)
             raise NotImplementedError("training path: an inner BatchNorm layer must be followed by ReLU")
         if fused:
-            acc = accs[li, :, :w.shape[0]]
-            y = ops.train_gemm(x, w, bias, in_stats=pending, stats_acc=acc,
-                               packed=arena.lookup(conv.weight, False) if arena is not None else None)
-            st = ops.bn_finalize(acc, rows, bn)
+            if running:
+                y = ops.train_gemm(x, w, bias, in_stats=pending,
+                                   packed=arena.lookup(conv.weight, False) if arena is not None else None)
+                st = ops.running_stats(bn)
+            else:
+                if accs is None:          # one fill for the block's statistics
+                    accs = torch.zeros((len(layers), 2, widest), dtype=torch.float64, device=x.device)
+                acc = accs[li, :, :w.shape[0]]
+                y = ops.train_gemm(x, w, bias, in_stats=pending, stats_acc=acc,
+                                   packed=arena.lookup(conv.weight, False) if arena is not None else None)
+                st = ops.bn_finalize(acc, rows, bn)
             saved.append((x, pending, y, st, relu, None))
             x, pending = y, st
             continue
@@ -159,7 +185,7 @@ def mlp_forward(x: torch.Tensor, layers: Sequence[Tuple], pool_K: Optional[int] 
             x, pending = ops.bn_act(x, pending, True), None
         y = _gemm(x, w, bias, arena=arena)
         if bn is not None:
-            st = ops.bn_batch_stats(y, bn)
+            st = ops.running_stats(bn) if running else ops.bn_batch_stats(y, bn)
             saved.append((x, None, y, st, relu, None))
             x, pending = y, st
         else:
@@ -180,31 +206,52 @@ def mlp_forward(x: torch.Tensor, layers: Sequence[Tuple], pool_K: Optional[int] 
 
 
 def mlp_backward(saved, layers: Sequence[Tuple], dz: torch.Tensor, pool_K: Optional[int], need_dx: bool, arena=None):
-    """-> (dx or None, [per layer: (dW [Co,Ci], db, dgamma, dbeta)]; None where the gradient went straight into p.grad)."""
+    """-> (dx or None, [per layer: (dW [Co,Ci], db, dgamma, dbeta)]; None where the gradient went straight into p.grad).
+    A layer whose input comes from a BatchNorm with running statistics (eval mode) and whose input-gradient GEMM is the
+    fused one with fewer than BNEVAL_EPILOGUE_BELOW outputs runs that BatchNorm's backward in the GEMM's epilogue
+    (ops.train_gemm_bneval): the layer below then gets its dy directly and has no BatchNorm pass of its own."""
     grads = [None] * len(layers)
     widest = max(c.weight.shape[0] for c, _, _ in layers)
     accs = torch.zeros((len(layers), 2, widest), dtype=torch.float64, device=dz.device)    # one fill for the block's reductions
     stats_done = False           # the reductions of this layer's BatchNorm backward were fused into the GEMM that produced dz
+    bn_done = None               # this layer's whole BatchNorm backward was: dz is already dy; (dgamma, dbeta, direct flags)
     for li in range(len(layers) - 1, -1, -1):
         conv, bn, relu = layers[li]
         x, x_stats, y, st, _, am = saved[li]
         dgamma = dbeta = None
         g_direct = beta_direct = False
-        if st is not None:
+        if bn_done is not None:
+            dy = dz
+            dgamma, dbeta, g_direct, beta_direct = bn_done
+        elif st is not None:
             dgamma, g_direct = _grad_sink(bn.weight, bn.weight.shape)
             dbeta, beta_direct = _grad_sink(bn.bias, bn.bias.shape)
-            dy = ops.bn_act_backward(y, st, dz, relu, argmax=am, K=pool_K if am is not None else 1, dgamma=dgamma, dbeta=dbeta,
-                                     acc=accs[li, :, :y.shape[1]], acc_ready=stats_done)
+            K = pool_K if am is not None else 1
+            if st.running:           # fixed statistics: no batch coupling, one pass
+                dy = ops.bn_eval_backward(y, st, dz, relu, argmax=am, K=K, dgamma=dgamma, dbeta=dbeta, acc=accs[li, :, :y.shape[1]])
+            else:
+                dy = ops.bn_act_backward(y, st, dz, relu, argmax=am, K=K, dgamma=dgamma, dbeta=dbeta,
+                                         acc=accs[li, :, :y.shape[1]], acc_ready=stats_done)
         else:
             dy = dz
-        stats_done = False
+        stats_done, bn_done = False, None
         w = _w2d(conv)
         dw, w_direct = _grad_sink(conv.weight, w.shape)
         db, b_direct = _grad_sink(conv.bias, (w.shape[0],)) if conv.bias is not None else (None, False)
         ops.grad_weight(dy, x, dw, db, x_stats=x_stats)      # x_stats: x is the previous layer's y, activated on load
         grads[li] = (None if w_direct else dw, None if b_direct else db, None if g_direct else dgamma, None if beta_direct else dbeta)
-        if (li > 0 and x_stats is not None and FUSED_BN and FUSED_BN_BWD and ops.mlp_mode() == "bf16x3"
-                and ops.train_gemm_supported(w.shape[0], w.shape[1])):
+        fused_t = (li > 0 and x_stats is not None and FUSED_BN and ops.mlp_mode() == "bf16x3"
+                   and ops.train_gemm_supported(w.shape[0], w.shape[1]))
+        if fused_t and x_stats.running and w.shape[1] < BNEVAL_EPILOGUE_BELOW:
+            # x is the pre-normalisation output of the layer below, whose BatchNorm has fixed statistics: its backward
+            # (dy = scale*g, dgamma, dbeta) happens in this GEMM's epilogue
+            bn_below = layers[li - 1][1]
+            gb, gb_direct = _grad_sink(bn_below.weight, bn_below.weight.shape)
+            bb, bb_direct = _grad_sink(bn_below.bias, bn_below.bias.shape)
+            dz = ops.train_gemm_bneval(dy, w, x, x_stats, accs[li - 1, :, :w.shape[1]], dgamma=gb, dbeta=bb,
+                                       packed=arena.lookup(conv.weight, True) if arena is not None else None)
+            bn_done = (gb, bb, gb_direct, bb_direct)
+        elif fused_t and not x_stats.running and FUSED_BN_BWD:
             # the layer below kept only its pre-normalisation output (x here): the input-gradient GEMM also accumulates the
             # two reductions of THAT layer's BatchNorm backward in its epilogue, saving a pass over dz and x
             dz = ops.train_gemm_bnbwd(dy, w, x, x_stats, accs[li - 1, :, :w.shape[1]],
@@ -336,7 +383,7 @@ class SegHeadFn(torch.autograd.Function):
         ctx.arena = arena = getattr(net, "_pn_arena", None)
         z1, saved = mlp_forward(feat.contiguous().view(B * N, C), layers, arena=arena)
         p = float(net.drop1.p)
-        if p > 0.0 or mask is not None:
+        if _dropout_on(net.drop1, mask):
             zd, mask = ops.dropout(z1, p, seed_offset=seed_offset, mask=mask)
         else:
             zd, mask = z1, None
@@ -382,11 +429,11 @@ class ClsHeadFn(torch.autograd.Function):
             z, saved = mlp_forward(cur, [(fc, bn, True)])
             p = float(drop.p)
             mask = masks[i] if masks is not None else None
-            if p > 0.0 or mask is not None:
+            if _dropout_on(drop, mask):
                 so = None if mask is not None else seed_offset + torch.tensor([0, 7919 * (i + 1)], dtype=torch.int64, device=x.device)
                 cur, mask = ops.dropout(z, p, seed_offset=so, mask=mask)
             else:
-                cur = z
+                cur, mask = z, None
             stages.append((saved, mask, p))
         logits = _gemm(cur, _w2d(net.fc3), net.fc3.bias.detach())
         logp = ops.log_softmax(logits)
@@ -415,7 +462,7 @@ class ClsHeadFn(torch.autograd.Function):
 
 def cls_head_train(net, global_feat: torch.Tensor, dropout_masks=None, seed_offset=None) -> torch.Tensor:
     """global_feat [B, 1024] -> log-probabilities [B, classes] with grad_fn."""
-    if dropout_masks is None and seed_offset is None:
+    if dropout_masks is None and seed_offset is None and (_dropout_on(net.drop1) or _dropout_on(net.drop2)):
         seed_offset = dropout_seed(global_feat.device)
     params = [net.fc1.weight, net.fc1.bias, net.bn1.weight, net.bn1.bias, net.fc2.weight, net.fc2.bias, net.bn2.weight,
               net.bn2.bias, net.fc3.weight, net.fc3.bias]
@@ -478,13 +525,13 @@ class LogSoftmaxFn(torch.autograd.Function):
 
 
 class BatchNormActFn(torch.autograd.Function):
-    """A BatchNorm (batch statistics) + optional ReLU on rows that does not directly follow its linear layer (PointNetCls:
-    relu(bn2(dropout(fc2(x)))), pointnet.py:148)."""
+    """A BatchNorm + optional ReLU on rows that does not directly follow its linear layer (PointNetCls:
+    relu(bn2(dropout(fc2(x)))), pointnet.py:148); batch or running statistics as the module's mode says."""
 
     @staticmethod
     def forward(ctx, bn, relu, x, gamma, beta):
         x = x.contiguous()
-        st = ops.bn_batch_stats(x, bn)
+        st = ops.running_stats(bn) if ops.uses_running_stats(bn) else ops.bn_batch_stats(x, bn)
         ctx.bn, ctx.relu, ctx.st = bn, relu, st
         ctx.save_for_backward(x)
         return ops.bn_act(x, st, relu)
@@ -492,7 +539,8 @@ class BatchNormActFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dz):
         (x,) = ctx.saved_tensors
-        dy, dgamma, dbeta = ops.bn_act_backward(x, ctx.st, dz.contiguous(), ctx.relu)
+        bwd = ops.bn_eval_backward if ctx.st.running else ops.bn_act_backward
+        dy, dgamma, dbeta = bwd(x, ctx.st, dz.contiguous(), ctx.relu)
         return None, None, dy, dgamma, dbeta
 
 
@@ -514,7 +562,7 @@ def pointnet_cls_train(net, x: torch.Tensor, dropout_mask=None):
     g, _, _, trans_feat = pointnet_encoder_train(net.feat, x.permute(0, 2, 1))
     h = mlp_rows_train([(net.fc1, net.bn1, True), (net.fc2, None, False)], g)
     p = float(net.dropout.p)
-    if p > 0.0 or dropout_mask is not None:
+    if _dropout_on(net.dropout, dropout_mask):
         h = DropoutFn.apply(h, p, None if dropout_mask is not None else dropout_seed(x.device), dropout_mask)
     h = BatchNormActFn.apply(net.bn2, True, h, net.bn2.weight, net.bn2.bias)
     logits = mlp_rows_train([(net.fc3, None, False)], h)
@@ -542,7 +590,7 @@ def pointnet_densecls_train(net, point_cloud: torch.Tensor, label: torch.Tensor,
     # classification head: fc1-bnc1-relu, fc2-dropout-bnc2-relu, fc3 (raw logits, :213-215)
     h = mlp_rows_train([(net.fc1, net.bnc1, True), (net.fc2, None, False)], out_max)
     p = float(net.dropout.p)
-    if p > 0.0 or dropout_mask is not None:
+    if _dropout_on(net.dropout, dropout_mask):
         h = DropoutFn.apply(h, p, None if dropout_mask is not None else dropout_seed(h.device), dropout_mask)
     h = BatchNormActFn.apply(net.bnc2, True, h, net.bnc2.weight, net.bnc2.bias)
     cls_logits = mlp_rows_train([(net.fc3, None, False)], h)
@@ -755,7 +803,7 @@ def _semseg_forward_train(net, points: torch.Tensor, fps_starts=None, dropout_ma
         up = fs[4]
         for i in (3, 2, 1, 0):
             up = feature_propagation_train(fp[i], xs[i], xs[i + 1], fs[i] if i > 0 else None, up, geometry=fp_geo[i])
-        if dropout_mask is None and seed_offset is None and net.drop1.p > 0:
+        if dropout_mask is None and seed_offset is None and _dropout_on(net.drop1):
             seed_offset = dropout_seed(points.device)
         params = [net.conv1.weight, net.conv1.bias, net.bn1.weight, net.bn1.bias, net.conv2.weight, net.conv2.bias]
         return SegHeadFn.apply(net, up.permute(0, 2, 1), dropout_mask, seed_offset, *params)[0]
@@ -798,7 +846,7 @@ def _semseg_forward_train(net, points: torch.Tensor, fps_starts=None, dropout_ma
     for i in (3, 2, 1, 0):
         user.wait_event(fp_ready[i])
         up = feature_propagation_train(fp[i], xs[i], xs[i + 1], fs[i] if i > 0 else None, up, geometry=fp_geo[i])
-    if dropout_mask is None and seed_offset is None and net.drop1.p > 0:
+    if dropout_mask is None and seed_offset is None and _dropout_on(net.drop1):
         seed_offset = dropout_seed(points.device)
     params = [net.conv1.weight, net.conv1.bias, net.bn1.weight, net.bn1.bias, net.conv2.weight, net.conv2.bias]
     return SegHeadFn.apply(net, up.permute(0, 2, 1), dropout_mask, seed_offset, *params)[0]
@@ -807,7 +855,7 @@ def _semseg_forward_train(net, points: torch.Tensor, fps_starts=None, dropout_ma
 def seg_head_train(net, l0_points: torch.Tensor, dropout_mask=None, seed_offset=None):
     """conv1-bn1-relu-drop1-conv2-log_softmax of the part-segmentation nets in train() mode (pointnet2.py:99-104):
     l0_points [B,128,N] -> (log_probs [B,N,k], feat [B,128,N]), both with grad_fn."""
-    if dropout_mask is None and seed_offset is None and net.drop1.p > 0:
+    if dropout_mask is None and seed_offset is None and _dropout_on(net.drop1):
         seed_offset = dropout_seed(l0_points.device)
     params = [net.conv1.weight, net.conv1.bias, net.bn1.weight, net.bn1.bias, net.conv2.weight, net.conv2.bias]
     logp, feat = SegHeadFn.apply(net, l0_points.permute(0, 2, 1), dropout_mask, seed_offset, *params)
@@ -961,6 +1009,14 @@ class SegMetrics:
 
 
 # ------------------------------------------------------------------------------------------------
+def _mode_modules(net) -> List[torch.nn.Module]:
+    return [m for m in net.modules() if isinstance(m, (torch.nn.modules.batchnorm._BatchNorm, torch.nn.Dropout))]
+
+
+def _modes(modules) -> Tuple[bool, ...]:
+    return tuple(m.training for m in modules)
+
+
 class GraphedTrainStep:
     """One training iteration of PointNet2SemSeg as ONE CUDA-graph replay + the gradient exchange + the Adam launch.
 
@@ -991,6 +1047,7 @@ class GraphedTrainStep:
         self._calls = 0
         self._bn_buffers = [b for m in self.net.modules() if isinstance(m, torch.nn.modules.batchnorm._BatchNorm)
                             for b in (m.running_mean, m.running_var, m.num_batches_tracked) if b is not None]
+        self._mode_modules = _mode_modules(self.net)
 
     @staticmethod
     def _starts(st, p):
@@ -1075,7 +1132,8 @@ class GraphedTrainStep:
 
         if not self.net.training:
             raise RuntimeError("GraphedTrainStep: call net.train() first")
-        key = (tuple(points.shape), points.device)
+        # a graph bakes in which BatchNorm layers use batch statistics and which dropouts apply: one capture per mode set
+        key = (tuple(points.shape), points.device, _modes(self._mode_modules))
         st = self._graphs.get(key)
         if st is None:
             st = self._graphs[key] = self._build(points, target)
@@ -1121,6 +1179,7 @@ class GraphedStep:
         self._graphs = {}
         self._bn_buffers = [b for m in self.net.modules() if isinstance(m, torch.nn.modules.batchnorm._BatchNorm)
                             for b in (m.running_mean, m.running_var, m.num_batches_tracked) if b is not None]
+        self._mode_modules = _mode_modules(self.net)
 
     def _fb(self, st):
         loss = self.loss_fn(self.net, st["x"], st["target"])
@@ -1156,7 +1215,7 @@ class GraphedStep:
 
         if not self.net.training:
             raise RuntimeError("GraphedStep: call net.train() first")
-        key = (tuple(points.shape), tuple(target.shape), points.device)
+        key = (tuple(points.shape), tuple(target.shape), points.device, _modes(self._mode_modules))
         st = self._graphs.get(key)
         if st is None:
             st = self._graphs[key] = self._build(points, target)
