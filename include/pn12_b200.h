@@ -96,6 +96,18 @@ int pn_fps_f32(const float* xyz, int64_t sB, int64_t sN, int64_t sC, int B, int 
  * out is contiguous [B,N,M].  Provided for API completeness; the hot path never materialises it. */
 int pn_square_distance_f32(const float* src, int64_t aB, int64_t aN, int64_t aC, const float* dst, int64_t bB,
                            int64_t bN, int64_t bC, int B, int N, int M, float* out, pn_stream_t stream);
+/* Backward of square_distance (model/pointnet_util.py:19-40; dist = -2 src dst^T + |src|^2 + |dst|^2) for g = dL/ddist [B,N,M]
+ * (batch stride gB >= 0, row stride gN >= 0, unit column stride; 16-byte aligned rows take the vector path):
+ *   dsrc[b,n] = 2 (sum_m g[b,n,m]) src[b,n] - 2 sum_m g[b,n,m] dst[b,m]
+ *   ddst[b,m] = 2 (sum_n g[b,n,m]) dst[b,m] - 2 sum_n g[b,n,m] src[b,n]
+ * the two terms formed apart and subtracted last, as torch's autograd adds the sum and matmul backwards.  g is read once:
+ * row and column sums come from the same pass (fp32, column sums accumulated with atomics, so the last bits depend on
+ * the order).  src / dst via element strides like pn_square_distance_f32; dsrc [B,N,3] / ddst [B,M,3] contiguous,
+ * written; either may be NULL (that side is skipped).  workspace: 16-byte aligned fp32 scratch of 4*B*(N+M) floats,
+ * zeroed here.  Limits: B <= 65535, N <= 4194240. */
+int pn_square_distance_bwd_f32(const float* g, int64_t gB, int64_t gN, const float* src, int64_t aB, int64_t aN, int64_t aC,
+                               const float* dst, int64_t bB, int64_t bN, int64_t bC, int B, int N, int M, float* workspace,
+                               float* dsrc, float* ddst, pn_stream_t stream);
 
 /* query_ball_point (model/pointnet_util.py:87-107).
  * out_idx [B,S,nsample]: the first nsample indices j (ascending) with NOT(sqdist(new_xyz_s, xyz_j) >
@@ -504,6 +516,19 @@ int pn_scan_sample_f32(const float* points, const uint32_t* raw_label, const int
  * *total (fp64, device, overwritten) = their sum; the reference divides by B.  Clouds via strides, D <= 8 coordinates. */
 int pn_chamfer_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN, int64_t bC,
                    int B, int N, int M, int D, float* per_point, double* total, pn_stream_t stream);
+/* pn_chamfer_f32 that also writes argmin [B,N] (int32, device) = the index m of the nearest p2 point, the first of equal
+ * minima (torch's min(dim) on the CPU), for the backward pass; per_point and *total are pn_chamfer_f32's. */
+int pn_chamfer_argmin_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN,
+                          int64_t bC, int B, int N, int M, int D, float* per_point, double* total, int32_t* argmin,
+                          pn_stream_t stream);
+/* Backward of chamfer_batch / chamfer_non_batch (model/chamfer.py:7-53: norm -> min -> sum): per p1 point, r = p1[b,n] -
+ * p2[b,a] with a = argmin[b,n] of pn_chamfer_argmin_f32, d = ||r|| recomputed in the forward's rounding sequence,
+ * c = (*g_total) * scale / d, and 0 where d == 0 (torch's norm backward).  dp1 [B,N,D] = c r (written);
+ * dp2[b,a] -= c r into a contiguous [B,M,D] buffer the caller zeroed (fp32 atomics).  Either output may be NULL.
+ * g_total: the fp32 gradient of the loss (device); scale = 1/B for chamfer_batch, 1 for chamfer_non_batch.  D <= 8. */
+int pn_chamfer_bwd_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN, int64_t bC,
+                       int B, int N, int M, int D, const int32_t* argmin, const float* g_total, float scale, float* dp1,
+                       float* dp2, pn_stream_t stream);
 /* SemKITTI_2_Common.__call__ (data_utils/kitti_utils.py:97-110): y[r, j] = max(x[r, src0[j]], x[r, src1[j]]) for j < n_out
  * (src1[j] == src0[j] for classes that are not merged); src0 / src1 are device int32 [n_out], indices < n_in. */
 int pn_class_merge_f32(const float* x, int64_t ldx, int64_t rows, int n_in, int n_out, const int* src0, const int* src1,

@@ -44,6 +44,7 @@ _SIGNATURES = {
     "pn_device_check": [C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)],
     "pn_fps_f32": [vp, i64, i64, i64, i32, i32, i32, vp, vp, _optsp, vp],
     "pn_square_distance_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, vp, vp],
+    "pn_square_distance_bwd_f32": [vp, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, vp, vp, vp, vp],
     "pn_ball_query_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, f32, i32, vp, vp],
     "pn_ball_grid_build_f32": [vp, i64, i64, i64, i32, i32, f32, vp, C.c_size_t, vp],
     "pn_ball_query_grid_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, f32, i32, vp, C.c_size_t, i32, vp, vp,
@@ -105,6 +106,8 @@ _SIGNATURES = {
     "pn_scan_filter_f32": [vp, vp, vp, i32, i64, vp, i32, i32, f32, f32, f32, f32, vp, vp, vp, C.c_size_t, vp],
     "pn_scan_sample_f32": [vp, vp, vp, i32, vp, i32, vp, vp, i32, vp, vp, f32, f32, vp, vp, vp, vp],
     "pn_chamfer_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp],
+    "pn_chamfer_argmin_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp],
+    "pn_chamfer_bwd_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp],
     "pn_class_merge_f32": [vp, i64, i64, i32, i32, vp, vp, vp, vp],
     "pn_seg_metrics_accumulate": [vp, i32, i64, vp, vp, vp, vp, vp],
 }

@@ -24,6 +24,9 @@
 //             pn_group_bwd_f32, pn_three_interpolate_bwd_f32    scatter-add through the gathers
 //   step      pn_adam_f32                         torch.optim.Adam (L2 weight decay) on one flat parameter buffer
 //   metrics   pn_seg_metrics_f32 + pn_seg_metrics_accumulate     pcdseg.py:72-83 without host round trips
+//   function-level gradients (model/pointnet_util.py, model/chamfer.py)
+//             pn_square_distance_bwd_f32          one read of dL/ddist: row and column sums, then 2 (sum g) x - 2 sum g y
+//             pn_chamfer_argmin_f32, pn_chamfer_bwd_f32    nearest points kept by the forward, norm backward of each pair
 //
 // All of these are HBM-bound streaming / reduction kernels except pn_grad_weight_f32 (CUDA-core SGEMM with a long K).
 #include <math_constants.h>
@@ -1116,12 +1119,15 @@ PN_EXPORT int pn_seg_metrics_accumulate(const int64_t* counts, int C, int64_t po
 // Row f-4 helpers.
 // chamfer_batch / chamfer_non_batch (model/chamfer.py:7-53): sum over b, n of min_m ||p1[b,n] - p2[b,m]||_2, divided by B.
 // One thread per p1 point, p2 staged through shared memory in tiles; the minimum is taken over squared distances
-// (sqrt is monotonic) and the root drawn once per point; block sums in fp64.
+// (sqrt is monotonic) and the root drawn once per point; block sums in fp64.  ARGMIN: also the index of the nearest p2
+// point (the first of equal minima, like torch's min(dim) on the CPU) for the backward pass.
 namespace pn {
 constexpr int CH_TILE = 256, CH_MAXD = 8;
+template <bool ARGMIN>
 __global__ void __launch_bounds__(CH_TILE)
 chamfer_kernel(const float* __restrict__ p1, int64_t aB, int64_t aN, int64_t aC, const float* __restrict__ p2, int64_t bB,
-               int64_t bN, int64_t bC, int N, int M, int D, float* __restrict__ per_point, double* __restrict__ total) {
+               int64_t bN, int64_t bC, int N, int M, int D, float* __restrict__ per_point, double* __restrict__ total,
+               int32_t* __restrict__ argmin) {
     __shared__ float tile[CH_TILE][CH_MAXD];
     __shared__ double red[CH_TILE / 32];
     const int b = blockIdx.y;
@@ -1130,6 +1136,7 @@ chamfer_kernel(const float* __restrict__ p1, int64_t aB, int64_t aN, int64_t aC,
 #pragma unroll
     for (int c = 0; c < CH_MAXD; ++c) q[c] = (n < N && c < D) ? p1[b * aB + (int64_t)n * aN + c * aC] : 0.0f;
     float best = CUDART_INF_F;
+    int best_m = 0;
     for (int m0 = 0; m0 < M; m0 += CH_TILE) {
         const int m = m0 + threadIdx.x;
 #pragma unroll
@@ -1143,12 +1150,22 @@ chamfer_kernel(const float* __restrict__ p1, int64_t aB, int64_t aN, int64_t aC,
                 const float t = q[c] - tile[j][c];
                 d = fmaf(t, t, d);
             }
-            best = fminf(best, d);
+            if constexpr (ARGMIN) {
+                if (d < best) {          // strict: the first minimum stays
+                    best = d;
+                    best_m = m0 + j;
+                }
+            } else {
+                best = fminf(best, d);
+            }
         }
         __syncthreads();
     }
     const float dist = n < N ? sqrtf(best) : 0.0f;
     if (n < N && per_point) per_point[(int64_t)b * N + n] = dist;
+    if constexpr (ARGMIN) {
+        if (n < N) argmin[(int64_t)b * N + n] = best_m;
+    }
     double s = (double)dist;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
@@ -1171,6 +1188,175 @@ __global__ void class_merge_kernel(const float* __restrict__ x, int64_t ldx, int
         y[e] = fmaxf(x[r * ldx + src0[j]], x[r * ldx + src1[j]]);
     }
 }
+
+// Backward of chamfer_batch / chamfer_non_batch: per p1 point, r = p1[n] - p2[a(n)] with the nearest p2 point a(n) of the
+// forward, d = ||r|| in the forward's rounding sequence, c = g*scale / d (0 where d == 0, as torch's norm backward);
+// dp1[n] = c*r (written), dp2[a(n)] -= c*r (fp32 atomics).
+__global__ void chamfer_bwd_kernel(const float* __restrict__ p1, int64_t aB, int64_t aN, int64_t aC, const float* __restrict__ p2,
+                                   int64_t bB, int64_t bN, int64_t bC, int N, int M, int D, int64_t total,
+                                   const int32_t* __restrict__ argmin, const float* __restrict__ g, float scale,
+                                   float* __restrict__ dp1, float* __restrict__ dp2) {
+    const float gs = *g * scale;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t b = i / N, n = i % N;
+        const int a = argmin[i];
+        float t[CH_MAXD];
+        float d = 0.0f;
+#pragma unroll
+        for (int c = 0; c < CH_MAXD; ++c) {
+            t[c] = c < D ? p1[b * aB + n * aN + c * aC] - p2[b * bB + (int64_t)a * bN + c * bC] : 0.0f;
+            d = fmaf(t[c], t[c], d);
+        }
+        const float dist = sqrtf(d);
+        const float coef = dist > 0.0f ? gs / dist : 0.0f;
+#pragma unroll
+        for (int c = 0; c < CH_MAXD; ++c) {
+            if (c >= D) break;
+            if (dp1) dp1[i * D + c] = coef * t[c];
+            if (dp2) atomicAdd(dp2 + (b * M + a) * D + c, -(coef * t[c]));
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Backward of square_distance (model/pointnet_util.py:19-40), dist = -2 src dst^T + |src|^2 + |dst|^2, g = dL/ddist [B,N,M]:
+//   dsrc[n] = 2 (sum_m g[n,m]) src[n] - 2 sum_m g[n,m] dst[m],   ddst[m] = 2 (sum_n g[n,m]) dst[m] - 2 sum_n g[n,m] src[n].
+// HBM-bound: g is read exactly once.  A CTA owns SDB_ROWS rows (SDB_RT per warp) and a chunk of columns, which its warps
+// stream in steps of 128 columns (a float4 per lane and row).  Row sums (sum g, sum g*dst) stay in registers for the whole
+// chunk; column sums (sum g, sum g*src) of a step are summed over the warp's rows in registers, then over the CTA's warps
+// in shared memory (double-buffered: one barrier per step), and leave as ONE vector red.global.add per column and CTA.
+// Both land in a small fp32 workspace, rows [B,N,4] and columns [B,M,4]; sqdist_bwd_finish_kernel forms the gradients
+// from it, with the reference's two terms kept apart and subtracted last (as torch's matmul + sum backward add them).
+constexpr int SDB_WARPS = 8, SDB_RT = 8, SDB_ROWS = SDB_WARPS * SDB_RT, SDB_STEP = 128;
+
+__device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float c, float d) {
+    asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+}
+
+template <bool VEC, bool ROWS, bool COLS>
+__global__ void __launch_bounds__(SDB_WARPS * 32, 2)
+sqdist_bwd_kernel(const float* __restrict__ g, int64_t gB, int64_t gN, const float* __restrict__ src, int64_t aB, int64_t aN,
+                  int64_t aC, const float* __restrict__ dst, int64_t bB, int64_t bN, int64_t bC, int N, int M, int chunk,
+                  float* __restrict__ rws, float* __restrict__ cws) {
+    __shared__ float4 part[COLS ? 2 : 1][SDB_WARPS][SDB_STEP];
+    const int b = blockIdx.z, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int r0 = blockIdx.y * SDB_ROWS + warp * SDB_RT;
+    const int m_begin = blockIdx.x * chunk, m_end = min(M, m_begin + chunk);
+    const float* __restrict__ gb = g + (int64_t)b * gB;
+    float sx[SDB_RT], sy[SDB_RT], sz[SDB_RT];                 // the warp's src rows (column sums only)
+    float rs[SDB_RT], rx[SDB_RT], ry[SDB_RT], rz[SDB_RT];     // row sums: sum g, sum g*dst
+#pragma unroll
+    for (int r = 0; r < SDB_RT; ++r) {
+        const int n = r0 + r;
+        const float* s = src + (int64_t)b * aB + (int64_t)n * aN;
+        sx[r] = COLS && n < N ? s[0] : 0.0f;
+        sy[r] = COLS && n < N ? s[aC] : 0.0f;
+        sz[r] = COLS && n < N ? s[2 * aC] : 0.0f;
+        rs[r] = rx[r] = ry[r] = rz[r] = 0.0f;
+    }
+    int buf = 0;
+    for (int c0 = m_begin; c0 < m_end; c0 += SDB_STEP) {
+        const int m = c0 + lane * 4;
+        float dx[4], dy[4], dz[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const float* q = dst + (int64_t)b * bB + (int64_t)(m + j) * bN;
+            const bool ok = ROWS && m + j < m_end;
+            dx[j] = ok ? q[0] : 0.0f;
+            dy[j] = ok ? q[bC] : 0.0f;
+            dz[j] = ok ? q[2 * bC] : 0.0f;
+        }
+        float v[SDB_RT][4];
+#pragma unroll
+        for (int r = 0; r < SDB_RT; ++r) {
+            const int n = r0 + r;
+            const float* row = gb + (int64_t)n * gN + m;
+            if (VEC && n < N && m + 3 < m_end) {
+                const float4 t = __ldcs(reinterpret_cast<const float4*>(row));
+                v[r][0] = t.x, v[r][1] = t.y, v[r][2] = t.z, v[r][3] = t.w;
+            } else {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) v[r][j] = n < N && m + j < m_end ? __ldcs(row + j) : 0.0f;
+            }
+        }
+        float cs[4], cx[4], cy[4], cz[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) cs[j] = cx[j] = cy[j] = cz[j] = 0.0f;
+#pragma unroll
+        for (int r = 0; r < SDB_RT; ++r) {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const float e = v[r][j];
+                if (ROWS) {
+                    rs[r] += e;
+                    rx[r] = fmaf(e, dx[j], rx[r]);
+                    ry[r] = fmaf(e, dy[j], ry[r]);
+                    rz[r] = fmaf(e, dz[j], rz[r]);
+                }
+                if (COLS) {
+                    cs[j] += e;
+                    cx[j] = fmaf(e, sx[r], cx[j]);
+                    cy[j] = fmaf(e, sy[r], cy[j]);
+                    cz[j] = fmaf(e, sz[r], cz[j]);
+                }
+            }
+        }
+        if (COLS) {
+            // slot j*32 + lane holds column m + j: conflict-free stores here and loads below
+#pragma unroll
+            for (int j = 0; j < 4; ++j) part[buf][warp][j * 32 + lane] = make_float4(cs[j], cx[j], cy[j], cz[j]);
+            __syncthreads();
+            if (threadIdx.x < SDB_STEP) {
+                const int col = c0 + (threadIdx.x & 31) * 4 + (threadIdx.x >> 5);
+                float4 t = part[buf][0][threadIdx.x];
+#pragma unroll
+                for (int w = 1; w < SDB_WARPS; ++w) {
+                    const float4 u = part[buf][w][threadIdx.x];
+                    t.x += u.x, t.y += u.y, t.z += u.z, t.w += u.w;
+                }
+                if (col < m_end) red_add_v4(cws + ((int64_t)b * M + col) * 4, t.x, t.y, t.z, t.w);
+            }
+            buf ^= 1;   // the other buffer was last read before this step's barrier
+        }
+    }
+    if (ROWS) {
+#pragma unroll
+        for (int r = 0; r < SDB_RT; ++r) {
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                rs[r] += __shfl_xor_sync(0xffffffffu, rs[r], o);
+                rx[r] += __shfl_xor_sync(0xffffffffu, rx[r], o);
+                ry[r] += __shfl_xor_sync(0xffffffffu, ry[r], o);
+                rz[r] += __shfl_xor_sync(0xffffffffu, rz[r], o);
+            }
+            if (lane == r && r0 + r < N) red_add_v4(rws + ((int64_t)b * N + r0 + r) * 4, rs[r], rx[r], ry[r], rz[r]);
+        }
+    }
+}
+
+// out[p] = 2 (sum e) x[p] - 2 (sum e*y) from the workspace records {sum e, sum e*y_x, sum e*y_y, sum e*y_z}, for the
+// B*N src points (rws -> dsrc) then the B*M dst points (cws -> ddst); a NULL output is skipped.
+__global__ void sqdist_bwd_finish_kernel(const float* __restrict__ src, int64_t aB, int64_t aN, int64_t aC,
+                                         const float* __restrict__ dst, int64_t bB, int64_t bN, int64_t bC, int B, int N, int M,
+                                         const float4* __restrict__ rws, const float4* __restrict__ cws, float* __restrict__ dsrc,
+                                         float* __restrict__ ddst) {
+    const int64_t nsrc = (int64_t)B * N, total = nsrc + (int64_t)B * M;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const bool is_src = i < nsrc;
+        float* out = is_src ? dsrc : ddst;
+        if (!out) continue;
+        const int64_t j = is_src ? i : i - nsrc;
+        const int P = is_src ? N : M;
+        const int64_t b = j / P, p = j % P;
+        const float* x = is_src ? src + b * aB + p * aN : dst + b * bB + p * bN;
+        const int64_t xc = is_src ? aC : bC;
+        const float4 w = is_src ? rws[j] : cws[j];
+        const float s2 = 2.0f * w.x;
+        out[j * 3 + 0] = __fsub_rn(__fmul_rn(s2, x[0]), 2.0f * w.y);
+        out[j * 3 + 1] = __fsub_rn(__fmul_rn(s2, x[xc]), 2.0f * w.z);
+        out[j * 3 + 2] = __fsub_rn(__fmul_rn(s2, x[2 * xc]), 2.0f * w.w);
+    }
+}
 }  // namespace pn
 
 PN_EXPORT int pn_chamfer_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN,
@@ -1184,7 +1370,7 @@ PN_EXPORT int pn_chamfer_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC
         return (int)e;
     }
     dim3 grid((unsigned)ceil_div(N, CH_TILE), (unsigned)B);
-    chamfer_kernel<<<grid, CH_TILE, 0, st>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, per_point, total);
+    chamfer_kernel<false><<<grid, CH_TILE, 0, st>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, per_point, total, nullptr);
     return finish_launch("pn_chamfer_f32");
 }
 
@@ -1194,4 +1380,70 @@ PN_EXPORT int pn_class_merge_f32(const float* x, int64_t ldx, int64_t rows, int 
     PN_REQUIRE(rows > 0 && n_in > 0 && n_out > 0 && ldx >= n_in, PN_ERR_BAD_ARG, "pn_class_merge_f32: bad shape");
     class_merge_kernel<<<ew_blocks(rows * n_out, 256), 256, 0, (cudaStream_t)stream>>>(x, ldx, rows, n_out, src0, src1, y);
     return finish_launch("pn_class_merge_f32");
+}
+
+PN_EXPORT int pn_chamfer_argmin_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN,
+                                    int64_t bC, int B, int N, int M, int D, float* per_point, double* total, int32_t* argmin,
+                                    pn_stream_t stream) {
+    PN_REQUIRE(p1 && p2 && total && argmin, PN_ERR_BAD_ARG, "pn_chamfer_argmin_f32: null pointer");
+    PN_REQUIRE(B > 0 && B <= 65535 && N > 0 && M > 0 && D > 0 && D <= CH_MAXD, PN_ERR_BAD_ARG,
+               "pn_chamfer_argmin_f32: bad sizes (D <= 8)");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(total, 0, sizeof(double), st);
+    if (e != cudaSuccess) {
+        set_error("pn_chamfer_argmin_f32: %s", cudaGetErrorString(e));
+        return (int)e;
+    }
+    dim3 grid((unsigned)ceil_div(N, CH_TILE), (unsigned)B);
+    chamfer_kernel<true><<<grid, CH_TILE, 0, st>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, per_point, total, argmin);
+    return finish_launch("pn_chamfer_argmin_f32");
+}
+
+PN_EXPORT int pn_chamfer_bwd_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN,
+                                 int64_t bC, int B, int N, int M, int D, const int32_t* argmin, const float* g_total, float scale,
+                                 float* dp1, float* dp2, pn_stream_t stream) {
+    PN_REQUIRE(p1 && p2 && argmin && g_total && (dp1 || dp2), PN_ERR_BAD_ARG, "pn_chamfer_bwd_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && M > 0 && D > 0 && D <= CH_MAXD, PN_ERR_BAD_ARG, "pn_chamfer_bwd_f32: bad sizes (D <= 8)");
+    const int64_t total = (int64_t)B * N;
+    chamfer_bwd_kernel<<<ew_blocks(total, 256), 256, 0, (cudaStream_t)stream>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, total,
+                                                                               argmin, g_total, scale, dp1, dp2);
+    return finish_launch("pn_chamfer_bwd_f32");
+}
+
+PN_EXPORT int pn_square_distance_bwd_f32(const float* g, int64_t gB, int64_t gN, const float* src, int64_t aB, int64_t aN,
+                                         int64_t aC, const float* dst, int64_t bB, int64_t bN, int64_t bC, int B, int N, int M,
+                                         float* workspace, float* dsrc, float* ddst, pn_stream_t stream) {
+    PN_REQUIRE(g && src && dst && workspace && (dsrc || ddst), PN_ERR_BAD_ARG, "pn_square_distance_bwd_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && M > 0, PN_ERR_BAD_ARG, "pn_square_distance_bwd_f32: B, N, M must be positive");
+    PN_REQUIRE(B <= 65535 && ceil_div(N, SDB_ROWS) <= 65535, PN_ERR_UNSUPPORTED,
+               "pn_square_distance_bwd_f32: B <= 65535 and N <= %d", 65535 * SDB_ROWS);
+    PN_REQUIRE(gB >= 0 && gN >= 0, PN_ERR_BAD_ARG, "pn_square_distance_bwd_f32: negative stride of g");
+    PN_REQUIRE(((uintptr_t)workspace & 15) == 0, PN_ERR_BAD_ARG, "pn_square_distance_bwd_f32: workspace must be 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    float* rws = workspace;                       // [B,N,4]
+    float* cws = workspace + (int64_t)B * N * 4;  // [B,M,4]
+    cudaError_t e = cudaMemsetAsync(workspace, 0, sizeof(float) * 4 * ((size_t)B * N + (size_t)B * M), st);
+    if (e != cudaSuccess) {
+        set_error("pn_square_distance_bwd_f32: %s", cudaGetErrorString(e));
+        return (int)e;
+    }
+    // columns per CTA: enough CTAs for four per SM where the shape allows, whole 128-column steps
+    const int64_t row_tiles = ceil_div(N, SDB_ROWS) * B;
+    const int64_t steps = ceil_div(M, SDB_STEP);
+    int64_t chunks = ceil_div((int64_t)sm_count() * 4, row_tiles);
+    if (chunks > steps) chunks = steps;
+    if (chunks > 65535) chunks = 65535;
+    const int chunk = (int)(ceil_div(steps, chunks) * SDB_STEP);
+    dim3 grid((unsigned)ceil_div(M, chunk), (unsigned)ceil_div(N, SDB_ROWS), (unsigned)B);
+    const bool vec = ((uintptr_t)g & 15) == 0 && gN % 4 == 0 && (B == 1 || gB % 4 == 0);
+    const bool rows = dsrc != nullptr, cols = ddst != nullptr;
+    auto kern = vec ? (rows ? (cols ? sqdist_bwd_kernel<true, true, true> : sqdist_bwd_kernel<true, true, false>)
+                            : sqdist_bwd_kernel<true, false, true>)
+                    : (rows ? (cols ? sqdist_bwd_kernel<false, true, true> : sqdist_bwd_kernel<false, true, false>)
+                            : sqdist_bwd_kernel<false, false, true>);
+    kern<<<grid, SDB_WARPS * 32, 0, st>>>(g, gB, gN, src, aB, aN, aC, dst, bB, bN, bC, N, M, chunk, rws, cws);
+    sqdist_bwd_finish_kernel<<<ew_blocks((int64_t)B * (N + (int64_t)M), 256), 256, 0, st>>>(
+        src, aB, aN, aC, dst, bB, bN, bC, B, N, M, reinterpret_cast<const float4*>(rws), reinterpret_cast<const float4*>(cws),
+        dsrc, ddst);
+    return finish_launch("pn_square_distance_bwd_f32");
 }

@@ -27,6 +27,8 @@ views of that storage, so chaining modules costs no transposes.
 eval(): BatchNorm is folded into the conv weights from the running statistics and the fused tensor-core chains run.
 train(): PointNetSetAbstraction and PointNetFeaturePropagation normalise with batch statistics and return tensors with a
 grad_fn (pointnet12_b200/train.py: forward and backward on our kernels), and so does PointNetSetAbstractionMsg.
+The functions (square_distance, index_points, sample_and_group(_all)) return results with a grad_fn when grad mode is on
+and a floating-point input requires a gradient, like the reference's torch expressions; index outputs carry none.
 CPU tensors raise: there is no CPU fallback.
 """
 from __future__ import annotations
@@ -41,13 +43,26 @@ from .. import ops
 
 # ------------------------------------------------------------------------------------------------
 # L1 primitives
+def grad_path(*inputs) -> bool:
+    """Whether grad mode is on and one of the floating-point tensor inputs requires a gradient: then the function-level API
+    returns results with a grad_fn (pointnet12_b200/train.py), otherwise it makes the forward-only launches."""
+    return torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.is_floating_point() and t.requires_grad
+                                           for t in inputs)
+
+
 def square_distance(src: torch.Tensor, dst: torch.Tensor) -> torch.Tensor:
     """[B,N,3] x [B,M,3] -> [B,N,M] with the reference's |a|^2 + |b|^2 - 2ab rounding sequence."""
+    if grad_path(src, dst):
+        from ..train import SquareDistanceFn
+        return SquareDistanceFn.apply(src, dst)
     return ops.square_distance(src, dst)
 
 
 def index_points(points: torch.Tensor, idx: torch.Tensor) -> torch.Tensor:
     """points [B,N,C], idx [B,S] or [B,S,K] -> [B,S,C] / [B,S,K,C]."""
+    if grad_path(points):
+        from ..train import GatherPointsFn
+        return GatherPointsFn.apply(points, idx)
     return ops.index_points(points, idx)
 
 
@@ -84,6 +99,9 @@ def draw_fps_starts(batch: int, level_sizes: Sequence[int], device) -> List[torc
 def sample_and_group(npoint: int, radius: float, nsample: int, xyz: torch.Tensor, points: Optional[torch.Tensor],
                      returnfps: bool = False, start_idx: Optional[torch.Tensor] = None):
     """-> new_xyz [B,npoint,3], new_points [B,npoint,nsample,3+D] (xyz relative to the centroid first)."""
+    if grad_path(xyz, points):
+        from ..train import sample_and_group_train
+        return sample_and_group_train(npoint, radius, nsample, xyz, points, returnfps, start_idx)
     fps_idx = farthest_point_sample(xyz, npoint, start_idx)
     new_xyz = ops.index_points(xyz, fps_idx)
     idx = ops.ball_query(radius, nsample, xyz, new_xyz)
@@ -98,6 +116,9 @@ def sample_and_group_all(xyz: torch.Tensor, points: Optional[torch.Tensor]):
     B, N, _ = xyz.shape
     new_xyz = torch.zeros((B, 1, 3), dtype=torch.float32, device=xyz.device)
     everyone = torch.arange(N, dtype=torch.int64, device=xyz.device).expand(B, 1, N).contiguous()
+    if grad_path(xyz, points):
+        from ..train import GroupPointsFn
+        return new_xyz, GroupPointsFn.apply(xyz, points, new_xyz, everyone, False)
     return new_xyz, ops.group(xyz, points, new_xyz, everyone, msg_order=False)   # x - 0 == x exactly
 
 
@@ -260,10 +281,7 @@ def autograd_path(module: nn.Module, *inputs) -> bool:
     """Whether a module runs on the autograd blocks of pointnet12_b200/train.py: in training mode, and in eval mode when grad
     mode is on and one of its floating-point inputs requires a gradient -- there BatchNorm normalises with its running
     statistics and dropout is the identity, as in the torch modules.  Otherwise the fused eval forward runs (no grad_fn)."""
-    if module.training:
-        return True
-    return torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.is_floating_point() and t.requires_grad
-                                           for t in inputs)
+    return module.training or grad_path(*inputs)
 
 
 def _mlp_rows(rows: torch.Tensor, layers) -> torch.Tensor:

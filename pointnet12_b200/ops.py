@@ -307,6 +307,30 @@ def square_distance(src: torch.Tensor, dst: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def square_distance_backward(g: torch.Tensor, src: torch.Tensor, dst: torch.Tensor, need_src: bool = True,
+                             need_dst: bool = True) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """Backward of square_distance (pn_square_distance_bwd_f32): g [B, N, M] = dL/ddist (any batch and row strides; a
+    view whose columns are not contiguous is copied first), src [B, N, 3], dst [B, M, 3] (any strides) -> (dsrc [B, N, 3]
+    or None, ddst [B, M, 3] or None), computed for the sides asked for."""
+    src, dst = _cloud(src, "src", 3), _cloud(dst, "dst", 3)
+    B, N, _ = src.shape
+    M = dst.shape[1]
+    g = _f32(g, "g")
+    if tuple(g.shape) != (B, N, M):
+        raise ValueError(f"g must have shape ({B}, {N}, {M}), got {tuple(g.shape)}")
+    if not (need_src or need_dst):
+        return None, None
+    if g.stride(2) != 1 and M > 1:
+        g = g.contiguous()
+    dsrc = torch.empty((B, N, 3), dtype=torch.float32, device=src.device) if need_src else None
+    ddst = torch.empty((B, M, 3), dtype=torch.float32, device=src.device) if need_dst else None
+    ws = torch.empty((4 * B * (N + M),), dtype=torch.float32, device=src.device)
+    with _on_device(src):
+        nv.call("pn_square_distance_bwd_f32", g.data_ptr(), g.stride(0), g.stride(1), src.data_ptr(), *src.stride(),
+                dst.data_ptr(), *dst.stride(), B, N, M, ws.data_ptr(), _p(dsrc), _p(ddst), _stream())
+    return dsrc, ddst
+
+
 GRID_MIN_POINTS = 4096     # below this the ordered scan of pn_ball_query_f32 is already short
 
 
@@ -411,6 +435,51 @@ def group(xyz: torch.Tensor, feat: Optional[torch.Tensor], new_xyz: torch.Tensor
         nv.call("pn_group_f32", xyz.data_ptr(), *xyz.stride(), _p(feat), *fs, D, new_xyz.data_ptr(), *new_xyz.stride(),
                 idx.data_ptr(), B, N, S, K, int(msg_order), out.data_ptr(), ld, _stream())
     return out
+
+
+def _chamfer_clouds(p1: torch.Tensor, p2: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    p1, p2 = _cloud(p1, "p1"), _cloud(p2, "p2")
+    if p1.shape[0] != p2.shape[0] or p1.shape[2] != p2.shape[2]:
+        raise ValueError(f"p1 {tuple(p1.shape)} and p2 {tuple(p2.shape)} must agree on the batch size and the coordinates")
+    return p1, p2
+
+
+def chamfer_argmin(p1: torch.Tensor, p2: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
+    """model/chamfer.py:7-53 with the nearest points (pn_chamfer_argmin_f32): p1 [B, N, D], p2 [B, M, D] (any strides,
+    D <= 8) -> (total float64 [1] = sum over b, n of min_m ||p1[b,n] - p2[b,m]||, argmin int32 [B, N], the first of equal
+    minima)."""
+    p1, p2 = _chamfer_clouds(p1, p2)
+    B, N, D = p1.shape
+    total = torch.empty((1,), dtype=torch.float64, device=p1.device)
+    argmin = torch.empty((B, N), dtype=torch.int32, device=p1.device)
+    with _on_device(p1):
+        nv.call("pn_chamfer_argmin_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, p2.shape[1], D, None,
+                total.data_ptr(), argmin.data_ptr(), _stream())
+    return total, argmin
+
+
+def chamfer_backward(p1: torch.Tensor, p2: torch.Tensor, argmin: torch.Tensor, g_total: torch.Tensor, scale: float,
+                     need_p1: bool = True, need_p2: bool = True) -> Tuple[Optional[torch.Tensor], Optional[torch.Tensor]]:
+    """Backward of the chamfer sum (pn_chamfer_bwd_f32): argmin of chamfer_argmin, g_total the loss gradient (a one-element
+    device tensor) -> (dp1 [B, N, D] or None, dp2 [B, M, D] or None) of scale * g_total * sum_n ||p1[n] - p2[argmin[n]]||."""
+    p1, p2 = _chamfer_clouds(p1, p2)
+    B, N, D = p1.shape
+    M = p2.shape[1]
+    _need_cuda(argmin, "argmin")
+    if argmin.dtype != torch.int32 or tuple(argmin.shape) != (B, N):
+        raise ValueError(f"argmin must be an int32 [{B}, {N}] tensor")
+    argmin = argmin.contiguous()
+    g = _f32(g_total, "g_total").reshape(-1)
+    if g.numel() != 1:
+        raise ValueError("g_total must have one element")
+    if not (need_p1 or need_p2):
+        return None, None
+    dp1 = torch.empty((B, N, D), dtype=torch.float32, device=p1.device) if need_p1 else None
+    dp2 = torch.zeros((B, M, D), dtype=torch.float32, device=p1.device) if need_p2 else None
+    with _on_device(p1):
+        nv.call("pn_chamfer_bwd_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, M, D, argmin.data_ptr(),
+                g.contiguous().data_ptr(), float(scale), _p(dp1), _p(dp2), _stream())
+    return dp1, dp2
 
 
 def _rows(x: torch.Tensor, name: str) -> Tuple[torch.Tensor, int, int, int]:

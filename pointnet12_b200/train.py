@@ -29,6 +29,7 @@ import os
 from typing import List, Optional, Sequence, Tuple
 
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import ops
 
@@ -641,18 +642,104 @@ def pointnet_seg_train(net, x: torch.Tensor):
 # ------------------------------------------------------------------------------------------------
 # train-mode forwards called by the modules (model/pointnet_util.py, model/pointnet2.py)
 class GatherPointsFn(torch.autograd.Function):
-    """new_xyz = index_points(xyz, fps_idx) of sample_and_group (pointnet_util.py:117) with its gradient w.r.t. xyz: the
-    scatter-add of pn_group_bwd_f32 through fps_idx seen as groups of one point."""
+    """index_points(points, idx) (pointnet_util.py:43-60) for idx [B, ...] with its gradient w.r.t. points: the scatter-add of
+    pn_group_bwd_f32 through idx seen as groups of one point, so repeated indices accumulate.  new_xyz = index_points(xyz,
+    fps_idx) of sample_and_group (:117) is one use."""
 
     @staticmethod
-    def forward(ctx, xyz_pm, fps_idx):
-        ctx.fps_idx, ctx.N = fps_idx, xyz_pm.shape[1]
-        return ops.index_points(xyz_pm, fps_idx)
+    def forward(ctx, points, idx):
+        ctx.idx, ctx.N = idx, points.shape[1]
+        return ops.index_points(points, idx)
 
     @staticmethod
-    def backward(ctx, dnew):
-        B, S = ctx.fps_idx.shape
-        return ops.group_backward(_rows_of(dnew, 3), 0, 3, ctx.fps_idx.view(B, S, 1), ctx.N), None
+    @once_differentiable
+    def backward(ctx, dout):
+        B, C = ctx.idx.shape[0], dout.shape[-1]
+        flat = ctx.idx.reshape(B, -1, 1)
+        if flat.shape[1] == 0:
+            return torch.zeros((B, ctx.N, C), dtype=torch.float32, device=dout.device), None
+        return ops.group_backward(_rows_of(dout, C), 0, C, flat, ctx.N), None
+
+
+class GroupPointsFn(torch.autograd.Function):
+    """new_points of sample_and_group (pointnet_util.py:127-131) = [xyz[idx] - new_xyz, points[idx]], or of
+    sample_and_group_all (:151-156, recentred=False: xyz[idx] as it is), with the gradients w.r.t. xyz and new_xyz
+    (pn_group_bwd_xyz_f32 on the xyz columns) and w.r.t. points (pn_group_bwd_f32 on the feature columns)."""
+
+    @staticmethod
+    def forward(ctx, xyz_pm, pts_pm, new_xyz, idx, recentred):
+        ctx.idx, ctx.N, ctx.recentred = idx, xyz_pm.shape[1], recentred
+        ctx.D = pts_pm.shape[2] if pts_pm is not None else 0
+        return ops.group(xyz_pm, pts_pm, new_xyz, idx, msg_order=False)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, dout):
+        rows = _rows_of(dout, 3 + ctx.D)
+        dxyz = dnew = dpts = None
+        if ctx.needs_input_grad[0] or ctx.needs_input_grad[2]:
+            dxyz, dnew = ops.group_backward_xyz(rows, 0, ctx.idx, ctx.N, recentred=ctx.recentred and ctx.needs_input_grad[2])
+        if ctx.D and ctx.needs_input_grad[1]:
+            dpts = ops.group_backward(rows, 3, ctx.D, ctx.idx, ctx.N)
+        return dxyz if ctx.needs_input_grad[0] else None, dpts, dnew, None, None
+
+
+class SquareDistanceFn(torch.autograd.Function):
+    """square_distance (pointnet_util.py:19-40) with the gradients w.r.t. src and dst (pn_square_distance_bwd_f32: one read
+    of the incoming [B, N, M] gradient)."""
+
+    @staticmethod
+    def forward(ctx, src, dst):
+        ctx.save_for_backward(src, dst)
+        return ops.square_distance(src, dst)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        src, dst = ctx.saved_tensors
+        return ops.square_distance_backward(g, src, dst, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+
+
+class ChamferFn(torch.autograd.Function):
+    """chamfer_batch (divisor = B) / chamfer_non_batch (divisor = 1) of model/chamfer.py:7-53 with the gradients w.r.t. both
+    clouds: the forward keeps each p1 point's nearest p2 point (pn_chamfer_argmin_f32), the backward differentiates the norm
+    of that pair (pn_chamfer_bwd_f32).  The value is the forward-only path's: the fp64 sum divided by the divisor, in fp32."""
+
+    @staticmethod
+    def forward(ctx, p1, p2, divisor):
+        total, ctx.argmin = ops.chamfer_argmin(p1, p2)
+        ctx.save_for_backward(p1, p2)
+        ctx.scale = 1.0 / divisor
+        return (total[0] / divisor).to(torch.float32)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        p1, p2 = ctx.saved_tensors
+        dp1, dp2 = ops.chamfer_backward(p1, p2, ctx.argmin, g, ctx.scale, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        return dp1, dp2, None
+
+
+def sample_and_group_train(npoint, radius, nsample, xyz: torch.Tensor, points: Optional[torch.Tensor], returnfps=False,
+                           start_idx=None):
+    """sample_and_group (pointnet_util.py:110-137) with gradients w.r.t. xyz and points: sampling and ball query run on the
+    detached coordinates (index outputs carry no gradient, as in the reference); the gathers and the recentring are
+    differentiated.  Same draws and indices as the forward-only path."""
+    from .model.pointnet_util import farthest_point_sample
+
+    with torch.no_grad():
+        xyz_d = xyz.detach()
+        fps_idx = farthest_point_sample(xyz_d, npoint, start_idx)
+        new_xyz = ops.index_points(xyz_d, fps_idx)
+        idx = ops.ball_query(radius, nsample, xyz_d, new_xyz)
+    grad_xyz = _wants_grad(xyz)
+    if grad_xyz:
+        new_xyz = GatherPointsFn.apply(xyz, fps_idx)
+    new_points = GroupPointsFn.apply(xyz, points, new_xyz, idx, True)
+    if returnfps:
+        grouped_xyz = GatherPointsFn.apply(xyz, idx) if grad_xyz else ops.index_points(xyz, idx)
+        return new_xyz, new_points, grouped_xyz, fps_idx
+    return new_xyz, new_points
 
 
 def _wants_grad(t: Optional[torch.Tensor]) -> bool:
