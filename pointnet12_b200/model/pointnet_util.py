@@ -88,10 +88,19 @@ def query_ball_point(radius: float, nsample: int, xyz: torch.Tensor, new_xyz: to
     return ops.ball_query(radius, nsample, xyz, new_xyz)
 
 
+# The HostDraws log (pointnet12_b200/train.py) of a CUDA-graph training runner while it warms up and captures, else None.
+draw_log = None
+
+
 def draw_fps_starts(batch: int, level_sizes: Sequence[int], device) -> List[torch.Tensor]:
     """All FPS start-index draws of one forward, made up front in call order on the CPU generator (the very
     torch.randint calls of pointnet_util.py:75, so torch.manual_seed reproduces the reference), staged in one
-    pinned buffer and sent with a single asynchronous copy: the host never waits for the device mid-forward."""
+    pinned buffer and sent with a single asynchronous copy: the host never waits for the device mid-forward.
+    While a graph runner records (`draw_log`), nothing is drawn: the starts are views of its control buffer, which the
+    runner fills with these same draws before every replay."""
+    if draw_log is not None:
+        n = len(level_sizes)
+        return list(draw_log.take(("fps", int(batch), tuple(int(s) for s in level_sizes)), n * batch).view(n, batch).unbind(0))
     draws = torch.stack([torch.randint(0, n, (batch,), dtype=torch.long) for n in level_sizes]).pin_memory()
     return list(draws.to(device, non_blocking=True).unbind(0))
 
@@ -455,7 +464,9 @@ class PointNetFeaturePropagation(nn.Module):
         B, N, _ = x1.shape
         if x2.shape[1] == 1:   # a single coarse point: broadcast it (reference :292-293)
             idx = torch.zeros((B, N, 3), dtype=torch.int64, device=x1.device)
-            return idx, torch.tensor([1.0, 0.0, 0.0], device=x1.device).expand(B, N, 3).contiguous()
+            w = torch.zeros((B, N, 3), dtype=torch.float32, device=x1.device)
+            w[:, :, 0] = 1.0             # weights (1, 0, 0) made on the device: no host copy, so a CUDA graph can capture it
+            return idx, w
         return ops.three_nn(x1, x2, order=order, background=background)
 
     def fold_first_layer(self, p2, head=None):

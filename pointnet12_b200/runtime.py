@@ -311,6 +311,29 @@ class GraphedSemSeg:
         return results
 
 
+class PinnedRing:
+    """Pinned int64 host buffers that stage values for a graph's static device buffer, used in turn: `next()` returns the
+    next buffer once the copy that last read it has run; `send(dst)` copies it to `dst` with one asynchronous copy on the
+    current stream."""
+
+    def __init__(self, shape, depth: int):
+        self.bufs = [torch.zeros(shape, dtype=torch.int64).pin_memory() for _ in range(depth)]
+        self.events = [None] * depth
+        self.slot = 0
+
+    def next(self) -> torch.Tensor:
+        self.slot = (self.slot + 1) % len(self.bufs)
+        if self.events[self.slot] is not None:
+            self.events[self.slot].synchronize()
+        return self.bufs[self.slot]
+
+    def send(self, dst: torch.Tensor) -> None:
+        dst.copy_(self.bufs[self.slot], non_blocking=True)
+        ev = torch.cuda.Event()
+        ev.record()
+        self.events[self.slot] = ev
+
+
 class GraphedModule:
     """CUDA-graph replay of any eval-mode network of this package, one batch at a time.  PointNetSeg / PointNetCls /
     PointNetDenseCls (model/pointnet.py) draw nothing on the host; the PointNet++ classification / part-segmentation nets
@@ -350,13 +373,12 @@ class GraphedModule:
         st = self._graphs.get(key)
         B = inputs[0].shape[0]
         if st is None:
-            st = {"in": [torch.empty(t.shape, dtype=t.dtype, device=dev) for t in inputs], "starts": None, "slot": 0}
+            st = {"in": [torch.empty(t.shape, dtype=t.dtype, device=dev) for t in inputs], "starts": None}
             sizes = self.net.fps_level_sizes(inputs[0].shape[2]) if hasattr(self.net, "fps_level_sizes") else []
             if sizes:
                 st["sizes"] = sizes
                 st["starts"] = torch.zeros((len(sizes), B), dtype=torch.int64, device=dev)
-                st["pinned"] = [torch.zeros((len(sizes), B), dtype=torch.int64).pin_memory() for _ in range(self.RING)]
-                st["events"] = [None] * self.RING
+                st["ring"] = PinnedRing((len(sizes), B), self.RING)
             for s, t in zip(st["in"], inputs):
                 s.copy_(t)
             side = torch.cuda.Stream(dev)
@@ -373,16 +395,10 @@ class GraphedModule:
             self._graphs[key] = st
             self._sig = self._signature()
         if st["starts"] is not None:
-            slot = st["slot"] = (st["slot"] + 1) % self.RING
-            if st["events"][slot] is not None:
-                st["events"][slot].synchronize()
-            pinned = st["pinned"][slot]
+            pinned = st["ring"].next()
             for i, n in enumerate(st["sizes"]):           # the reference's draws, same generator, same order
                 pinned[i] = torch.randint(0, n, (B,), dtype=torch.long)
-            st["starts"].copy_(pinned, non_blocking=True)
-            ev = torch.cuda.Event()
-            ev.record()
-            st["events"][slot] = ev
+            st["ring"].send(st["starts"])
         for s, t in zip(st["in"], inputs):
             s.copy_(t, non_blocking=True)
         st["graph"].replay()

@@ -25,6 +25,7 @@ atomics; `ops.set_mlp_mode("fp32")` puts every GEMM on the CUDA cores.
 """
 from __future__ import annotations
 
+import contextlib
 import os
 from typing import List, Optional, Sequence, Tuple
 
@@ -431,7 +432,10 @@ class ClsHeadFn(torch.autograd.Function):
             p = float(drop.p)
             mask = masks[i] if masks is not None else None
             if _dropout_on(drop, mask):
-                so = None if mask is not None else seed_offset + torch.tensor([0, 7919 * (i + 1)], dtype=torch.int64, device=x.device)
+                so = None
+                if mask is None:          # {seed, offset + 7919 (i + 1)}, formed on the device: no host copy under capture
+                    so = seed_offset.clone()
+                    so[1:].add_(7919 * (i + 1))
                 cur, mask = ops.dropout(z, p, seed_offset=so, mask=mask)
             else:
                 cur, mask = z, None
@@ -820,7 +824,12 @@ _SEED = {"next": 0}
 
 def dropout_seed(device) -> torch.Tensor:
     """{seed, offset} for the Philox stream of one dropout call: the seed comes from torch's CPU generator state
-    (so torch.manual_seed makes runs repeatable), the offset counts the calls."""
+    (so torch.manual_seed makes runs repeatable), the offset counts the calls.  While a graph runner records
+    (HostDraws), nothing is drawn and the counter stays: the pair is a view of the runner's control buffer."""
+    from .model import pointnet_util
+
+    if pointnet_util.draw_log is not None:
+        return pointnet_util.draw_log.take(("dropout",), 2)
     _SEED["next"] += 1
     return torch.tensor([torch.initial_seed() & 0x7FFFFFFFFFFFFFFF, _SEED["next"]], dtype=torch.int64).to(device, non_blocking=True)
 
@@ -1250,15 +1259,88 @@ class GraphedTrainStep:
         return st["loss"][p]
 
 
+class HostDraws:
+    """The host draws of one train-mode forward, logged for a CUDA-graph runner: the FPS start indices of the sampling levels
+    (model/pointnet_util.draw_fps_starts) and the dropout streams' {seed, offset} (dropout_seed).
+
+    While `recording()` is active those functions draw nothing: each call is logged with its kind and shape, in call order, and
+    gets views of its slice of ONE static int64 control buffer, `ctl` (zeros until the first pass has sized it).  Before every
+    replay the runner calls `draw_into(host_buffer)`, which repeats the logged draws exactly as the eager calls make them --
+    torch.randint(0, n, (B,)) per sampling level on the CPU default generator, the seed from torch.initial_seed(), the next value
+    of the dropout counter -- and sends the buffer to `ctl` with one copy.  So after the same torch.manual_seed a graphed loop
+    consumes the generator and the counter exactly as the eager loop does.  Every pass must make the same draws as the first."""
+
+    def __init__(self, device):
+        self.device = torch.device(device)
+        self.log = None         # [("fps", B, level sizes) | ("dropout",)] of the first pass
+        self.ctl = None
+        self._seen, self._used = [], 0
+
+    @contextlib.contextmanager
+    def recording(self):
+        """One recorded pass (a warm-up or the capture).  The CPU generator state and the dropout counter are restored on exit,
+        so the pass consumes neither."""
+        from .model import pointnet_util
+
+        rng, nxt, outer = torch.get_rng_state(), _SEED["next"], pointnet_util.draw_log
+        self._seen, self._used = [], 0
+        pointnet_util.draw_log = self
+        try:
+            yield self
+            if self.log is None:
+                self.log = self._seen
+                self.ctl = torch.zeros((self._used,), dtype=torch.int64, device=self.device)
+            elif self._seen != self.log:
+                raise RuntimeError(f"HostDraws: a pass drew {self._seen}, the first pass drew {self.log}")
+        finally:
+            pointnet_util.draw_log = outer
+            torch.set_rng_state(rng)
+            _SEED["next"] = nxt
+
+    def take(self, entry, n: int) -> torch.Tensor:
+        """Logs one draw call (`entry`) and returns its n values: a slice of `ctl`."""
+        i, o = len(self._seen), self._used
+        self._seen.append(entry)
+        self._used += n
+        if self.log is None:
+            return torch.zeros((n,), dtype=torch.int64, device=self.device)
+        if i >= len(self.log) or self.log[i] != entry:
+            raise RuntimeError(f"HostDraws: draw {i} is {entry}, the first pass drew {self.log[i] if i < len(self.log) else None}")
+        return self.ctl[o:o + n]
+
+    def draw_into(self, buf: torch.Tensor) -> None:
+        """The logged draws, made now on the host as the eager calls make them, in call order, into buf (int64, ctl's size)."""
+        o = 0
+        for entry in self.log:
+            if entry[0] == "fps":
+                _, B, sizes = entry
+                for n in sizes:
+                    torch.randint(0, n, (B,), dtype=torch.long, out=buf[o:o + B])
+                    o += B
+            else:
+                _SEED["next"] += 1
+                buf[o] = torch.initial_seed() & 0x7FFFFFFFFFFFFFFF
+                buf[o + 1] = _SEED["next"]
+                o += 2
+
+
 class GraphedStep:
-    """Generic CUDA-graph training iteration for nets whose train-mode forward draws nothing on the host (PointNetSeg: no
-    sampling, no dropout): forward + loss + backward are captured once per input shape and replayed; the gradient exchange and
-    Adam follow on the same stream.  loss_fn(net, points, target) -> scalar loss tensor with grad_fn.
+    """Generic CUDA-graph training iteration: forward + loss + backward are captured once per input shape and BatchNorm / Dropout
+    mode set and replayed; the gradient exchange and Adam follow on the same stream.  loss_fn(net, inputs, target) -> scalar loss
+    tensor with grad_fn, where `inputs` is the net's input tensor or, for nets with several inputs, a tuple of them; loss_fn gets
+    the graph's static copies in the same form.
 
         step = GraphedStep(net, FlatAdam(net.parameters(), ...),
                            lambda net, x, t: cross_entropy((out := net(x))[0], t) + feature_transform_reguliarzer(out[1]) * 0.001)
         loss = step(points, target)
-    """
+        loss = step((xyz, norm_plt, cls_label), target)          # PointNet2PartSegMsg_one_hot, PointNetDenseCls
+
+    Host draws in the forward -- the FPS start indices of the PointNet++ sampling levels, the dropouts' {seed, offset} -- are
+    logged while the runner warms up and captures (HostDraws); the graph reads them from a static control buffer, and before every
+    replay the runner makes the same draws on the host, as an eager iteration would, and sends them there with one asynchronous
+    copy from a pinned ring.  A net without such draws (PointNetSeg) has an empty log and nothing is staged."""
+
+    RING = 4
 
     def __init__(self, net, optimizer: "FlatAdam", loss_fn, group=None, warmup: int = 2):
         self.net = net.module if hasattr(net, "module") else net
@@ -1269,22 +1351,24 @@ class GraphedStep:
         self._mode_modules = _mode_modules(self.net)
 
     def _fb(self, st):
-        loss = self.loss_fn(self.net, st["x"], st["target"])
+        loss = self.loss_fn(self.net, st["x"] if st["tuple"] else st["x"][0], st["target"])
         self.opt.zero_grad()
         loss.backward()
         return loss
 
-    def _build(self, points, target):
+    def _build(self, xs, as_tuple, target):
         from . import _native as nv
+        from .runtime import PinnedRing
 
-        dev = points.device
-        st = {"x": points.clone(), "target": target.clone()}
+        dev = xs[0].device
+        st = {"x": tuple(t.clone() for t in xs), "tuple": as_tuple, "target": target.clone(), "draws": HostDraws(dev)}
         keep = [t.clone() for t in (self.opt.flat, *self._bn_buffers)]           # warm-up must not train
         side = torch.cuda.Stream(dev)
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):
-            for _ in range(self.warmup):
-                self._fb(st)
+            for _ in range(max(1, self.warmup)):          # (the first pass sizes the control buffer)
+                with st["draws"].recording():
+                    self._fb(st)
         torch.cuda.current_stream(dev).wait_stream(side)
         torch.cuda.synchronize(dev)
         with torch.no_grad():
@@ -1292,22 +1376,32 @@ class GraphedStep:
                 t.copy_(k)
         graph = torch.cuda.CUDAGraph()
         n0 = nv.launch_count
-        with torch.cuda.graph(graph):
+        with torch.cuda.graph(graph), st["draws"].recording():
             st["loss"] = self._fb(st)
         st["launches"], st["graph"] = nv.launch_count - n0, graph
+        st["ring"] = PinnedRing(st["draws"].ctl.shape, self.RING) if st["draws"].log else None
         return st
 
-    def __call__(self, points: torch.Tensor, target: torch.Tensor) -> torch.Tensor:
+    def __call__(self, inputs, target: torch.Tensor) -> torch.Tensor:
         from . import _native as nv
 
         if not self.net.training:
             raise RuntimeError("GraphedStep: call net.train() first")
-        key = (tuple(points.shape), tuple(target.shape), points.device, _modes(self._mode_modules))
+        as_tuple = isinstance(inputs, tuple)
+        xs = inputs if as_tuple else (inputs,)
+        # a graph bakes in the input shapes and dtypes and the draws of the modes it was captured with (a Dropout in .eval()
+        # draws no seed): one capture, with its own draw log, per key
+        key = (tuple((tuple(t.shape), t.dtype) for t in xs), as_tuple, tuple(target.shape), xs[0].device,
+               _modes(self._mode_modules))
         st = self._graphs.get(key)
         if st is None:
-            st = self._graphs[key] = self._build(points, target)
-        if points.data_ptr() != st["x"].data_ptr():
-            st["x"].copy_(points, non_blocking=True)
+            st = self._graphs[key] = self._build(xs, as_tuple, target)
+        if st["ring"] is not None:
+            st["draws"].draw_into(st["ring"].next())
+            st["ring"].send(st["draws"].ctl)
+        for s, t in zip(st["x"], xs):
+            if t.data_ptr() != s.data_ptr():
+                s.copy_(t, non_blocking=True)
         if target.data_ptr() != st["target"].data_ptr():
             st["target"].copy_(target, non_blocking=True)
         st["graph"].replay()
