@@ -448,6 +448,84 @@ int pn_three_interpolate_bwd_xyz_f32(const float* dx, int64_t ldx, int D1, int D
                                      const float* points2, int64_t p2B, int64_t p2S, int64_t p2C, const float* xyz1, int64_t aB,
                                      int64_t aN, int64_t aC, const float* xyz2, int64_t bB, int64_t bS, int64_t bC, int B, int N,
                                      int S, float* dpoints1, float* dpoints2, float* dxyz1, float* dxyz2, pn_stream_t stream);
+/* ---- Deterministic variants (torch.use_deterministic_algorithms) -------------------------------------------------------
+ * The same results as the entry points above, with every floating-point sum taken in an order that depends only on the
+ * shapes and the device's SM count: two calls on the same inputs give bitwise-equal outputs.  Column / slab / block partials go
+ * to a caller-provided workspace (16-byte aligned, at least the bytes the matching *_workspace_bytes helper returns; 0 there
+ * means bad sizes) and are added in block order; scatter-adds go through an inverse index (CSR) built by pn_csr_build and are
+ * pulled per destination in ascending slot order.  Accumulating outputs (sum, s1, dw, db, dgamma, ...) keep their semantics:
+ * the ordered total is added to them once. */
+size_t pn_bn_stats_workspace_bytes(int64_t rows, int C);
+int pn_bn_stats_det_f32(const float* y, int64_t ldy, int64_t rows, int C, double* sum, double* sumsq, void* workspace,
+                        size_t workspace_bytes, pn_stream_t stream);
+int pn_bn_bwd_stats_det_f32(const float* y, int64_t ldy, int64_t rows, int C, const float* dz, int64_t lddz,
+                            const int32_t* argmax, int K, const float* scale, const float* shift, const float* mean,
+                            const float* invstd, int relu, double* s1, double* s2, void* workspace, size_t workspace_bytes,
+                            pn_stream_t stream);
+/* (workspace: pn_bn_stats_workspace_bytes(rows, C)) */
+int pn_bn_eval_bwd_det_f32(const float* y, int64_t ldy, int64_t rows, int C, const float* dz, int64_t lddz,
+                           const int32_t* argmax, int K, const float* scale, const float* shift, const float* mean,
+                           const float* invstd, int relu, double* s1, double* s2, float* dy, int64_t lddy, float* dgamma,
+                           float* dbeta, void* workspace, size_t workspace_bytes, pn_stream_t stream);
+/* Weight gradients: workspace = one fp32 tile per row slab (about SMs x the tile for the tensor-core engine). */
+size_t pn_grad_weight_f32_workspace_bytes(int64_t rows, int cout, int cin);
+size_t pn_grad_weight_bf16x3_workspace_bytes(int64_t rows, int cout, int cin);
+int pn_grad_weight_det_f32(const float* dy, int64_t lddy, const float* x, int64_t ldx, int64_t rows, int cout, int cin,
+                           float* dw, int64_t lddw, float* db, void* workspace, size_t workspace_bytes, pn_stream_t stream);
+int pn_grad_weight_det_bf16x3(const float* dy, int64_t lddy, const float* x, int64_t ldx, int64_t rows, int cout, int cin,
+                              float* dw, int64_t lddw, float* db, void* workspace, size_t workspace_bytes, pn_stream_t stream);
+int pn_grad_weight_bn_det_bf16x3(const float* dy, int64_t lddy, const float* x, int64_t ldx, const float* x_scale,
+                                 const float* x_shift, int x_relu, int64_t rows, int cout, int cin, float* dw, int64_t lddw,
+                                 float* db, void* workspace, size_t workspace_bytes, pn_stream_t stream);
+/* Inverse index of a gather: slot i (of B * slots_per_batch) names destination key(i) = (i / slots_per_batch) * n_dst +
+ * clamp(idx[i], 0, n_dst - 1) (idx int32 or int64, idx_bits = 32 / 64).  offsets int32 [B*n_dst + 1]: the slots of key k are
+ * slots[offsets[k] .. offsets[k+1]), in ascending order (slots int32 [n_slots]).  A stable radix sort of the keys: no limit on
+ * how many slots one destination has.  workspace: pn_csr_workspace_bytes(n_slots, B * n_dst), 4-byte aligned. */
+size_t pn_csr_workspace_bytes(int64_t n_slots, int64_t n_keys);
+int pn_csr_build(const void* idx, int idx_bits, int64_t n_slots, int64_t slots_per_batch, int n_dst, int B, void* workspace,
+                 size_t workspace_bytes, int32_t* offsets, int32_t* slots, pn_stream_t stream);
+/* out[k, c] (contiguous [n_dst, D], written) = sum over the slots s of k in ascending order, sequentially in fp32 from 0, of
+ * (weight ? weight[s] : 1) * src[(s / div) * ld + col0 + c]  -- what np.add.at accumulates. */
+int pn_csr_pull_f32(const float* src, int64_t ld, int col0, int D, int div, const float* weight, const int32_t* offsets,
+                    const int32_t* slots, int64_t n_dst, float* out, pn_stream_t stream);
+/* pn_group_bwd_f32 through the CSR of idx (slots_per_batch = S*K, n_dst = N): dfeat [B,N,D] is written. */
+int pn_group_bwd_det_f32(const float* dgrouped, int64_t ldg, int col0, int D, const int32_t* offsets, const int32_t* slots, int B,
+                         int N, float* dfeat, pn_stream_t stream);
+/* pn_group_bwd_xyz_f32 through the same CSR: dxyz [B,N,3] is written. */
+int pn_group_bwd_xyz_det_f32(const float* dgrouped, int64_t ldg, int col0, const int64_t* idx, const int32_t* offsets,
+                             const int32_t* slots, int B, int N, int S, int K, float* dxyz, float* dnew_xyz, pn_stream_t stream);
+/* pn_three_interpolate_bwd_f32 through the CSR of the 3-NN idx (slots_per_batch = N*3, n_dst = S): dpoints2 is written. */
+int pn_three_interpolate_bwd_det_f32(const float* dx, int64_t ldx, int D1, int D2, const float* weight, const int32_t* offsets,
+                                     const int32_t* slots, int B, int N, int S, float* dpoints1, float* dpoints2,
+                                     pn_stream_t stream);
+/* pn_three_interpolate_bwd_xyz_f32 through the same CSR; workspace: fp32 [B*N*9] (the per-slot terms of dxyz2).  dpoints2
+ * and dxyz2 are written. */
+int pn_three_interpolate_bwd_xyz_det_f32(const float* dx, int64_t ldx, int D1, int D2, const int64_t* idx, const float* weight,
+                                         const float* points2, int64_t p2B, int64_t p2S, int64_t p2C, const float* xyz1,
+                                         int64_t aB, int64_t aN, int64_t aC, const float* xyz2, int64_t bB, int64_t bS,
+                                         int64_t bC, int B, int N, int S, const int32_t* offsets, const int32_t* slots,
+                                         float* workspace, float* dpoints1, float* dpoints2, float* dxyz1, float* dxyz2,
+                                         pn_stream_t stream);
+/* pn_cross_entropy_f32 with the loss summed per block and the blocks added in order; workspace replaces loss_sum. */
+size_t pn_cross_entropy_workspace_bytes(int64_t rows);
+int pn_cross_entropy_det_f32(const float* x, int64_t ldx, const int64_t* target, int64_t rows, int C, void* workspace,
+                             size_t workspace_bytes, float* loss, float* dx, int64_t lddx, float grad_scale, pn_stream_t stream);
+/* pn_chamfer_f32 (argmin NULL) or pn_chamfer_argmin_f32 with the total summed per block, blocks in order; total is written. */
+size_t pn_chamfer_workspace_bytes(int B, int N);
+int pn_chamfer_det_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN, int64_t bC,
+                       int B, int N, int M, int D, float* per_point, double* total, int32_t* argmin, void* workspace,
+                       size_t workspace_bytes, pn_stream_t stream);
+/* pn_chamfer_bwd_f32 through the CSR of argmin (int32, slots_per_batch = N, n_dst = M); workspace: fp32 [B*N*D].  dp2 is
+ * written. */
+int pn_chamfer_bwd_det_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN,
+                           int64_t bC, int B, int N, int M, int D, const int32_t* argmin, const float* g_total, float scale,
+                           const int32_t* offsets, const int32_t* slots, float* workspace, float* dp1, float* dp2,
+                           pn_stream_t stream);
+/* pn_square_distance_bwd_f32 with one workspace slot per column chunk (rows) and per row tile (columns), added in order. */
+size_t pn_square_distance_bwd_det_workspace_bytes(int B, int N, int M);
+int pn_square_distance_bwd_det_f32(const float* g, int64_t gB, int64_t gN, const float* src, int64_t aB, int64_t aN, int64_t aC,
+                                   const float* dst, int64_t bB, int64_t bN, int64_t bC, int B, int N, int M, void* workspace,
+                                   size_t workspace_bytes, float* dsrc, float* ddst, pn_stream_t stream);
 /* nn.Dropout(p) in training mode (pointnet2.py:172): y = x*keep/(1-p).  mask_in (bytes, dense [rows*C]) != NULL:
  * keep = mask_in -- also the backward pass.  Otherwise keep ~ Bernoulli(1-p) from a Philox4x32-10 stream keyed by
  * seed_offset[0] with counter offset seed_offset[1] (DEVICE memory, so a replayed CUDA graph sees fresh values) and

@@ -110,6 +110,37 @@ _SIGNATURES = {
     "pn_chamfer_bwd_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp],
     "pn_class_merge_f32": [vp, i64, i64, i32, i32, vp, vp, vp, vp],
     "pn_seg_metrics_accumulate": [vp, i32, i64, vp, vp, vp, vp, vp],
+    # deterministic variants (*_det_*): the default signature plus a workspace (pointer, bytes) or a prebuilt CSR
+    "pn_bn_stats_det_f32": [vp, i64, i64, i32, vp, vp, vp, C.c_size_t, vp],
+    "pn_bn_bwd_stats_det_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, C.c_size_t, vp],
+    "pn_bn_eval_bwd_det_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, vp, vp, C.c_size_t,
+                               vp],
+    "pn_grad_weight_det_f32": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp, C.c_size_t, vp],
+    "pn_grad_weight_det_bf16x3": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp, C.c_size_t, vp],
+    "pn_grad_weight_bn_det_bf16x3": [vp, i64, vp, i64, vp, vp, i32, i64, i32, i32, vp, i64, vp, vp, C.c_size_t, vp],
+    "pn_csr_build": [vp, i32, i64, i64, i32, i32, vp, C.c_size_t, vp, vp, vp],
+    "pn_csr_pull_f32": [vp, i64, i32, i32, i32, vp, vp, vp, i64, vp, vp],
+    "pn_group_bwd_det_f32": [vp, i64, i32, i32, vp, vp, i32, i32, vp, vp],
+    "pn_group_bwd_xyz_det_f32": [vp, i64, i32, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp],
+    "pn_three_interpolate_bwd_det_f32": [vp, i64, i32, i32, vp, vp, vp, i32, i32, i32, vp, vp, vp],
+    "pn_three_interpolate_bwd_xyz_det_f32": [vp, i64, i32, i32, vp, vp, vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64,
+                                             i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp],
+    "pn_cross_entropy_det_f32": [vp, i64, vp, i64, i32, vp, C.c_size_t, vp, vp, i64, f32, vp],
+    "pn_chamfer_det_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp, C.c_size_t, vp],
+    "pn_chamfer_bwd_det_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp, vp, vp, vp],
+    "pn_square_distance_bwd_det_f32": [vp, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, vp, C.c_size_t, vp, vp,
+                                       vp],
+}
+
+# size_t helpers of the deterministic variants: name -> argtypes
+_SIZE_HELPERS = {
+    "pn_bn_stats_workspace_bytes": [i64, i32],
+    "pn_grad_weight_f32_workspace_bytes": [i64, i32, i32],
+    "pn_grad_weight_bf16x3_workspace_bytes": [i64, i32, i32],
+    "pn_csr_workspace_bytes": [i64, i64],
+    "pn_cross_entropy_workspace_bytes": [i64],
+    "pn_chamfer_workspace_bytes": [i32, i32],
+    "pn_square_distance_bwd_det_workspace_bytes": [i32, i32, i32],
 }
 
 
@@ -148,6 +179,10 @@ def lib():
         handle.pn_train_gemm_scratch_bytes.restype = C.c_size_t
         handle.pn_scan_workspace_bytes.argtypes = [i32, i64]
         handle.pn_scan_workspace_bytes.restype = C.c_size_t
+        for name, argtypes in _SIZE_HELPERS.items():
+            fn = getattr(handle, name)
+            fn.argtypes = argtypes
+            fn.restype = C.c_size_t
         _lib = handle
     return _lib
 

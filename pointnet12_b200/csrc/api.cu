@@ -16,7 +16,7 @@ void set_error(const char* fmt, ...) {
 
 }  // namespace pn
 
-PN_EXPORT int pn_version(void) { return 402; /* 0.4.2: function-level gradients: pn_square_distance_bwd_f32, pn_chamfer_argmin_f32, pn_chamfer_bwd_f32; 0.4.1: sampling on clusters of three and 48 points per thread; 3-NN block workspace in pairs (opaque, size changed); 0.4.0: per-call pn_launch_opts replace the process-wide setters; dynamic tile scheduling */ }
+PN_EXPORT int pn_version(void) { return 403; /* 0.4.3: deterministic variants of every floating-point reduction for torch.use_deterministic_algorithms: pn_csr_build / pn_csr_pull_f32 (inverse index + ordered pull), the *_det_* entry points and their *_workspace_bytes helpers; 0.4.2: function-level gradients: pn_square_distance_bwd_f32, pn_chamfer_argmin_f32, pn_chamfer_bwd_f32; 0.4.1: sampling on clusters of three and 48 points per thread; 3-NN block workspace in pairs (opaque, size changed); 0.4.0: per-call pn_launch_opts replace the process-wide setters; dynamic tile scheduling */ }
 
 PN_EXPORT const char* pn_last_error_string(void) { return pn::g_err; }
 

@@ -33,6 +33,10 @@ inline int finish_launch(const char* what) {
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// Deterministic scatter-add (scatter.cu): out[d, :D] = the slots of d (CSR of pn_csr_build), added in slot order.
+int csr_pull(const float* src, int64_t ld, int col0, int D, int div, const float* weight, const int32_t* offsets,
+             const int32_t* slots, int64_t n_dst, float* out, cudaStream_t stream);
+
 // Layout of the per-cloud bucket workspace of pn_ball_grid_build_f32 (ball_grid.cu): bytes per cloud and the offset of the
 // cell-sorted float4 (x, y, z, original index) records, for kernels of other files that walk the cloud in bucket order.
 size_t ball_grid_cloud_bytes(int N);

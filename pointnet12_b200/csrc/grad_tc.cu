@@ -27,6 +27,9 @@ constexpr int IMG = TM * KC * 2;              // one bf16 image of a 128 x 32 op
 constexpr int STAGE = 4 * IMG;                // A hi, A lo, B hi, B lo
 constexpr int SMEM = NS * STAGE + 1024;
 
+// DET: dw / db point to a workspace of [gridDim.z] slabs of [cout, lddw] and of [gridDim.z, 2] rows of [cout] (the two
+// producer halves of a channel): the slab's tile and bias sums are stored there instead of added.
+template <bool DET = false>
 __global__ void __launch_bounds__(THREADS)
 grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ x, int64_t ldx, int64_t rows,
                       int64_t rows_per_split, int cout, int cin, float* __restrict__ dw, int64_t lddw,
@@ -143,6 +146,10 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
         tc::fence_after();
         const int row = (warp & 3) * 32 + lane;                       // a warp reads the TMEM lanes of its quarter
         const int co = co0 + row;
+        if (DET) {
+            dw += (int64_t)blockIdx.z * cout * lddw;
+            if (db) db += ((int64_t)blockIdx.z * 2 + half) * cout;
+        }
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
             const int col0 = (warp >> 2) * 64 + h * 32;
@@ -150,7 +157,11 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
             tc::ld32(tbase + ((unsigned)((warp & 3) * 32) << 16) + (unsigned)col0, r);
             if (co < cout) {
                 float* dst = dw + (int64_t)co * lddw + ci0 + col0;
-                if (vec_red && ci0 + col0 + 32 <= cin) {
+                if (DET) {
+#pragma unroll
+                    for (int j = 0; j < 32; ++j)
+                        if (ci0 + col0 + j < cin) dst[j] = __uint_as_float(r[j]);
+                } else if (vec_red && ci0 + col0 + 32 <= cin) {
                     // 16-byte vector reductions: a quarter of the atomic operations the row slabs send to the same tile
 #pragma unroll
                     for (int j = 0; j < 32; j += 4)
@@ -164,7 +175,10 @@ grad_weight_tc_kernel(const float* __restrict__ dy, int64_t lddy, const float* _
                 }
             }
         }
-        if (do_bias) atomicAdd(&db[co0 + m], bsum);
+        if (do_bias) {
+            if (DET) db[co0 + m] = bsum;
+            else atomicAdd(&db[co0 + m], bsum);
+        }
     }
     tc::fence_before();
     __syncthreads();
@@ -200,7 +214,8 @@ static int grad_weight_tc(const float* dy, int64_t lddy, const float* x, int64_t
         int dev = 0;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        cudaFuncSetAttribute(grad_weight_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
+        cudaFuncSetAttribute(grad_weight_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
+        cudaFuncSetAttribute(grad_weight_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
         if (sms <= 0) sms = 148;
     }
     const int64_t tiles = ceil_div(cout, TM) * ceil_div(cin, TN);
@@ -212,7 +227,81 @@ static int grad_weight_tc(const float* dy, int64_t lddy, const float* x, int64_t
     PN_REQUIRE(splits <= 65535, PN_ERR_UNSUPPORTED, "pn_grad_weight_bf16x3: too many row splits");
     dim3 grid((unsigned)ceil_div(cout, TM), (unsigned)ceil_div(cin, TN), (unsigned)splits);
     const int vec_red = ((uintptr_t)dw % 16 == 0) && (lddw % 4 == 0);
-    grad_weight_tc_kernel<<<grid, THREADS, SMEM, (cudaStream_t)stream>>>(dy, lddy, x, ldx, rows, rps, cout, cin, dw, lddw, db,
+    grad_weight_tc_kernel<false><<<grid, THREADS, SMEM, (cudaStream_t)stream>>>(dy, lddy, x, ldx, rows, rps, cout, cin, dw, lddw, db,
                                                                         vec_red, x_scale, x_shift, x_relu);
     return finish_launch("pn_grad_weight_bf16x3");
+}
+
+// ------------------------------------------------------------------------------------------------
+// Deterministic variants: every row slab stores its tile (and bias sums) in the caller's workspace, then the slabs are added
+// to dw / db in slab order (slab_sum_kernel, train.cu).  Same launch shape as the atomic variant.
+namespace pn {
+int grad_weight_slab_sum(const float* ws, int64_t splits, int64_t bias_parts, int cout, int cin, float* dw, int64_t lddw, float* db,
+                         cudaStream_t st);
+}
+
+static void grad_weight_tc_shape(int64_t rows, int cout, int cin, int64_t* splits, int64_t* rps) {
+    using namespace pn::gtc;
+    int dev = 0, sms = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (sms <= 0) sms = 148;
+    const int64_t tiles = pn::ceil_div(cout, TM) * pn::ceil_div(cin, TN);
+    int64_t sp = pn::ceil_div((int64_t)sms, tiles);
+    int64_t r = pn::ceil_div(pn::ceil_div(rows, sp), KC) * KC;
+    if (r < 4 * KC) r = 4 * KC;
+    *rps = r;
+    *splits = pn::ceil_div(rows, r);
+}
+
+PN_EXPORT size_t pn_grad_weight_bf16x3_workspace_bytes(int64_t rows, int cout, int cin) {
+    if (rows <= 0 || cout <= 0 || cin <= 0) return 0;
+    int64_t splits, rps;
+    grad_weight_tc_shape(rows, cout, cin, &splits, &rps);
+    return sizeof(float) * (size_t)splits * ((size_t)cout * cin + 2 * (size_t)cout);
+}
+
+static int grad_weight_tc_det(const char* name, const float* dy, int64_t lddy, const float* x, int64_t ldx, int64_t rows, int cout,
+                              int cin, float* dw, int64_t lddw, float* db, const float* x_scale, const float* x_shift, int x_relu,
+                              void* workspace, size_t workspace_bytes, pn_stream_t stream) {
+    using namespace pn;
+    using namespace pn::gtc;
+    PN_REQUIRE(dy && x && dw, PN_ERR_BAD_ARG, "%s: null pointer", name);
+    PN_REQUIRE(rows > 0 && cout > 0 && cin > 0 && lddy >= cout && ldx >= cin && lddw >= cin, PN_ERR_BAD_ARG, "%s: bad shape", name);
+    const size_t need = pn_grad_weight_bf16x3_workspace_bytes(rows, cout, cin);
+    PN_REQUIRE(workspace, PN_ERR_BAD_ARG, "%s: null workspace", name);
+    PN_REQUIRE(workspace_bytes >= need, PN_ERR_BAD_ARG, "%s: workspace of %zu bytes, need %zu", name, workspace_bytes, need);
+    PN_REQUIRE(((uintptr_t)workspace & 15) == 0, PN_ERR_BAD_ARG, "%s: workspace must be 16-byte aligned", name);
+    static bool attr = false;
+    if (!attr) {
+        cudaFuncSetAttribute(grad_weight_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
+        attr = true;
+    }
+    int64_t splits, rps;
+    grad_weight_tc_shape(rows, cout, cin, &splits, &rps);
+    PN_REQUIRE(splits <= 65535, PN_ERR_UNSUPPORTED, "%s: too many row splits", name);
+    float* ws = static_cast<float*>(workspace);
+    float* wsb = ws + splits * (int64_t)cout * cin;
+    dim3 grid((unsigned)ceil_div(cout, TM), (unsigned)ceil_div(cin, TN), (unsigned)splits);
+    cudaStream_t st = (cudaStream_t)stream;
+    grad_weight_tc_kernel<true><<<grid, THREADS, SMEM, st>>>(dy, lddy, x, ldx, rows, rps, cout, cin, ws, cin, db ? wsb : nullptr, 0,
+                                                             x_scale, x_shift, x_relu);
+    const int e = finish_launch(name);
+    if (e != PN_OK) return e;
+    return grad_weight_slab_sum(ws, splits, 2 * splits, cout, cin, dw, lddw, db, st);
+}
+
+PN_EXPORT int pn_grad_weight_det_bf16x3(const float* dy, int64_t lddy, const float* x, int64_t ldx, int64_t rows, int cout, int cin,
+                                        float* dw, int64_t lddw, float* db, void* workspace, size_t workspace_bytes,
+                                        pn_stream_t stream) {
+    return grad_weight_tc_det("pn_grad_weight_det_bf16x3", dy, lddy, x, ldx, rows, cout, cin, dw, lddw, db, nullptr, nullptr, 0,
+                              workspace, workspace_bytes, stream);
+}
+
+PN_EXPORT int pn_grad_weight_bn_det_bf16x3(const float* dy, int64_t lddy, const float* x, int64_t ldx, const float* x_scale,
+                                           const float* x_shift, int x_relu, int64_t rows, int cout, int cin, float* dw, int64_t lddw,
+                                           float* db, void* workspace, size_t workspace_bytes, pn_stream_t stream) {
+    PN_REQUIRE(x_scale && x_shift, PN_ERR_BAD_ARG, "pn_grad_weight_bn_det_bf16x3: null scale / shift");
+    return grad_weight_tc_det("pn_grad_weight_bn_det_bf16x3", dy, lddy, x, ldx, rows, cout, cin, dw, lddw, db, x_scale, x_shift,
+                              x_relu, workspace, workspace_bytes, stream);
 }

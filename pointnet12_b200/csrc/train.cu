@@ -53,7 +53,9 @@ static inline int sm_count() {
 // MODE 2: as 1 with dz routed from the pooled gradient: g = dpool[row/K] if argmax[row/K] == row%K.
 constexpr int ST_LANES = 16;
 
-template <int MODE>
+// DET: s1 / s2 are [gridDim.x, C] partial rows, one per block, written instead of added (col_partials_sum_kernel adds them in
+// block order).
+template <int MODE, bool DET = false>
 __global__ void __launch_bounds__(32 * ST_LANES)
 col_stats_kernel(const float* __restrict__ y, int64_t ldy, int64_t rows, int C, int64_t rows_per_block,
                  const float* __restrict__ dz, int64_t lddz, const int32_t* __restrict__ argmax, int K,
@@ -95,9 +97,28 @@ col_stats_kernel(const float* __restrict__ y, int64_t ldy, int64_t rows, int C, 
     if (ry == 0 && c < C) {
 #pragma unroll
         for (int i = 1; i < ST_LANES; ++i) { a1 += r1[i][lane]; a2 += r2[i][lane]; }
-        atomicAdd(&s1[c], a1);
-        atomicAdd(&s2[c], a2);
+        if (DET) {
+            s1[(int64_t)blockIdx.x * C + c] = a1;
+            s2[(int64_t)blockIdx.x * C + c] = a2;
+        } else {
+            atomicAdd(&s1[c], a1);
+            atomicAdd(&s2[c], a2);
+        }
     }
+}
+
+// s1[c] += sum_b part[b, c], s2[c] += sum_b part[blocks + b, c], b ascending: the deterministic end of the column reductions.
+__global__ void col_partials_sum_kernel(const double* __restrict__ part, int blocks, int C, double* __restrict__ s1,
+                                        double* __restrict__ s2) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    double a1 = 0.0, a2 = 0.0;
+    for (int b = 0; b < blocks; ++b) {
+        a1 += part[(int64_t)b * C + c];
+        a2 += part[(int64_t)(blocks + b) * C + c];
+    }
+    s1[c] += a1;
+    s2[c] += a2;
 }
 
 static inline void stats_grid(int64_t rows, int C, dim3* grid, int64_t* rows_per_block) {
@@ -246,7 +267,7 @@ __global__ void bn_bwd_apply_kernel(const float* __restrict__ y, int64_t ldy, in
 // do not depend on the batch, so dy = scale*g needs no column reduction first.  g = dz * [y*scale+shift > 0] (POOLED:
 // routed from dz[row/K] by the arg-max of bn_act_max, either layout); dy = scale*g; s1 += sum g, s2 += sum g*xhat with
 // xhat = (y-mean)*invstd (fp64 per block, one atomic per column per block).  Same block shape as col_stats_kernel.
-template <bool POOLED>
+template <bool POOLED, bool DET = false>
 __global__ void __launch_bounds__(32 * ST_LANES)
 bn_eval_bwd_kernel(const float* __restrict__ y, int64_t ldy, int64_t rows, int C, int64_t rows_per_block,
                    const float* __restrict__ dz, int64_t lddz, const int32_t* __restrict__ argmax, int K,
@@ -282,8 +303,13 @@ bn_eval_bwd_kernel(const float* __restrict__ y, int64_t ldy, int64_t rows, int C
     if (ry == 0 && c < C) {
 #pragma unroll
         for (int i = 1; i < ST_LANES; ++i) { a1 += r1[i][lane]; a2 += r2[i][lane]; }
-        atomicAdd(&s1[c], a1);
-        atomicAdd(&s2[c], a2);
+        if (DET) {      // partial rows as in col_stats_kernel
+            s1[(int64_t)blockIdx.x * C + c] = a1;
+            s2[(int64_t)blockIdx.x * C + c] = a2;
+        } else {
+            atomicAdd(&s1[c], a1);
+            atomicAdd(&s2[c], a2);
+        }
     }
 }
 
@@ -300,7 +326,9 @@ __global__ void bn_eval_bwd_finalize_kernel(const double* __restrict__ s1, const
 // dW[co,ci] += sum_r dy[r,co] * x[r,ci]; db[co] += sum_r dy[r,co].  Both operands are read along their rows
 // (channels contiguous), so a K step is BK rows of each: straight 16-byte loads into shared memory, no transpose.
 // grid = (co tiles, ci tiles, row splits); fp32 atomics into the pre-zeroed (or accumulating) dW.
-template <int BM, int BN, int BK, int TM, int TN>
+// DET: dw / db point to a workspace of [gridDim.z] slabs of [cout, lddw] / [cout]; each row split stores its partial tile
+// there (slab_sum_kernel adds the slabs in split order).
+template <int BM, int BN, int BK, int TM, int TN, bool DET = false>
 __global__ void __launch_bounds__((BM / TM) * (BN / TN))
 grad_weight_kernel(const float* __restrict__ dy, int64_t lddy, const float* __restrict__ x, int64_t ldx, int64_t rows,
                    int64_t rows_per_split, int cout, int cin, float* __restrict__ dw, int64_t lddw,
@@ -385,6 +413,10 @@ grad_weight_kernel(const float* __restrict__ dy, int64_t lddy, const float* __re
         }
         __syncthreads();
     }
+    if (DET) {
+        dw += (int64_t)blockIdx.z * cout * lddw;
+        if (db) db += (int64_t)blockIdx.z * cout;
+    }
 #pragma unroll
     for (int i = 0; i < TM; ++i) {
         const int co = co0 + ty * TM + i;
@@ -392,9 +424,34 @@ grad_weight_kernel(const float* __restrict__ dy, int64_t lddy, const float* __re
 #pragma unroll
         for (int j = 0; j < TN; ++j) {
             const int ci = ci0 + tx * TN + j;
-            if (ci < cin) atomicAdd(&dw[(int64_t)co * lddw + ci], acc[i][j]);
+            if (ci < cin) {
+                if (DET) dw[(int64_t)co * lddw + ci] = acc[i][j];
+                else atomicAdd(&dw[(int64_t)co * lddw + ci], acc[i][j]);
+            }
         }
-        if (do_bias) atomicAdd(&db[co], bsum[i]);
+        if (do_bias) {
+            if (DET) db[co] = bsum[i];
+            else atomicAdd(&db[co], bsum[i]);
+        }
+    }
+}
+
+// dw[co, ci] += sum_s ws[s, co, ci] and db[co] += sum_p wsb[p, co] in ascending slab order: the deterministic end of the
+// weight gradients (ws [splits, cout, cin], wsb [bias_parts, cout] right behind it).
+__global__ void slab_sum_kernel(const float* __restrict__ ws, int splits, int bias_parts, int cout, int cin,
+                                float* __restrict__ dw, int64_t lddw, float* __restrict__ db) {
+    const int64_t tile = (int64_t)cout * cin, total = tile + (db ? cout : 0);
+    const float* __restrict__ wsb = ws + (int64_t)splits * tile;
+    for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+        float acc = 0.0f;
+        if (e < tile) {
+            for (int s = 0; s < splits; ++s) acc += ws[s * tile + e];
+            dw[(e / cin) * lddw + e % cin] += acc;
+        } else {
+            const int64_t co = e - tile;
+            for (int p = 0; p < bias_parts; ++p) acc += wsb[p * (int64_t)cout + co];
+            db[co] += acc;
+        }
     }
 }
 
@@ -429,7 +486,8 @@ __global__ void group_bwd_kernel(const float* __restrict__ dg, int64_t ldg, int 
     }
 }
 
-// rows (b,n) of dx = [d points1 (D1) | d interpolated (D2)]
+// rows (b,n) of dx = [d points1 (D1) | d interpolated (D2)]; DP2 = false: dp1 only (the deterministic path pulls dp2)
+template <bool DP2 = true>
 __global__ void three_interpolate_bwd_kernel(const float* __restrict__ dx, int64_t ldx, int D1, int D2,
                                              const int64_t* __restrict__ idx, const float* __restrict__ weight, int N,
                                              int S, int64_t total, float* __restrict__ dp1, float* __restrict__ dp2) {
@@ -440,7 +498,7 @@ __global__ void three_interpolate_bwd_kernel(const float* __restrict__ dx, int64
         const float g = dx[row * ldx + c];
         if (c < D1) {
             dp1[row * D1 + c] = g;
-        } else {
+        } else if (DP2) {
             const int64_t b = row / N;
             const int cc = c - D1;
 #pragma unroll
@@ -456,7 +514,8 @@ __global__ void three_interpolate_bwd_kernel(const float* __restrict__ dx, int64
 // Coordinate gradient of the grouping (pointnet_util.py:127-131, :243-247; group-all :151-156).  The three xyz_rel
 // columns at col0 of row (b,s,k) go to dxyz[b, idx[b,s,k]] (a padded ball repeats its first hit: each repeat adds its own
 // share); the recentring subtracted new_xyz[b,s] from every row of the group, so dnew[b,s] = -sum_k (dnew = NULL: group-all,
-// not recentred).  One warp per group, lanes over k.
+// not recentred).  One warp per group, lanes over k.  SCATTER = false: dnew only (the deterministic path pulls dxyz).
+template <bool SCATTER = true>
 __global__ void __launch_bounds__(256)
 group_bwd_xyz_kernel(const float* __restrict__ dg, int64_t ldg, int col0, const int64_t* __restrict__ idx, int N, int S,
                      int K, int64_t groups, float* __restrict__ dxyz, float* __restrict__ dnew) {
@@ -469,12 +528,14 @@ group_bwd_xyz_kernel(const float* __restrict__ dg, int64_t ldg, int col0, const 
             const int64_t row = grp * K + k;
             const float* r = dg + row * ldg + col0;
             const float x = r[0], y = r[1], z = r[2];
-            int64_t j = idx[row];
-            j = j < 0 ? 0 : (j >= N ? N - 1 : j);
-            float* o = dxyz + (b * N + j) * 3;
-            atomicAdd(o, x);
-            atomicAdd(o + 1, y);
-            atomicAdd(o + 2, z);
+            if (SCATTER) {
+                int64_t j = idx[row];
+                j = j < 0 ? 0 : (j >= N ? N - 1 : j);
+                float* o = dxyz + (b * N + j) * 3;
+                atomicAdd(o, x);
+                atomicAdd(o + 1, y);
+                atomicAdd(o + 2, z);
+            }
             sx += x;
             sy += y;
             sz += z;
@@ -502,7 +563,8 @@ group_bwd_xyz_kernel(const float* __restrict__ dg, int64_t ldg, int col0, const 
 //   dL/dd_j = -(g_j - sum_k w_k g_k) / R * r_j^2, or 0 where d_j was clamped (the masked assignment stops the gradient)
 //   dxyz1[n] = sum_j dL/dd_j * 2(a - b_j),   dxyz2[idx_j] += -dL/dd_j * 2(a - b_j)
 // VEC: the dx row (from D1), the p2 rows and the dp2 rows are read / added as float4.
-template <bool VEC>
+// DET: nothing is added to dp2 (pulled afterwards) and dxyz2 is a [rows, 3, 3] workspace of the per-slot terms, written.
+template <bool VEC, bool DET = false>
 __global__ void __launch_bounds__(256)
 three_interpolate_bwd_xyz_kernel(const float* __restrict__ dx, int64_t ldx, int D1, int D2, const int64_t* __restrict__ idx,
                                  const float* __restrict__ weight, const float* __restrict__ p2, int64_t p2B, int64_t p2S,
@@ -536,7 +598,7 @@ three_interpolate_bwd_xyz_kernel(const float* __restrict__ dx, int64_t ldx, int 
                 for (int k = 0; k < 3; ++k) {
                     const float4 pv = *reinterpret_cast<const float4*>(q[k] + c);
                     dot[k] = fmaf(gv.x, pv.x, fmaf(gv.y, pv.y, fmaf(gv.z, pv.z, fmaf(gv.w, pv.w, dot[k]))));
-                    atomicAdd(reinterpret_cast<float4*>(o[k] + c), make_float4(gv.x * w[k], gv.y * w[k], gv.z * w[k], gv.w * w[k]));
+                    if (!DET) atomicAdd(reinterpret_cast<float4*>(o[k] + c), make_float4(gv.x * w[k], gv.y * w[k], gv.z * w[k], gv.w * w[k]));
                 }
             }
         } else {
@@ -546,7 +608,7 @@ three_interpolate_bwd_xyz_kernel(const float* __restrict__ dx, int64_t ldx, int 
 #pragma unroll
                 for (int k = 0; k < 3; ++k) {
                     dot[k] = fmaf(gv, q[k][c * p2C], dot[k]);
-                    atomicAdd(o[k] + c, gv * w[k]);
+                    if (!DET) atomicAdd(o[k] + c, gv * w[k]);
                 }
             }
         }
@@ -582,10 +644,17 @@ three_interpolate_bwd_xyz_kernel(const float* __restrict__ dx, int64_t ldx, int 
             gx += tx;
             gy += ty;
             gz += tz;
-            float* o2 = dxyz2 + (b * S + j[k]) * 3;
-            atomicAdd(o2, -tx);
-            atomicAdd(o2 + 1, -ty);
-            atomicAdd(o2 + 2, -tz);
+            if (DET) {
+                float* o2 = dxyz2 + (row * 3 + k) * 3;
+                o2[0] = -tx;
+                o2[1] = -ty;
+                o2[2] = -tz;
+            } else {
+                float* o2 = dxyz2 + (b * S + j[k]) * 3;
+                atomicAdd(o2, -tx);
+                atomicAdd(o2 + 1, -ty);
+                atomicAdd(o2 + 2, -tz);
+            }
         }
         dxyz1[row * 3] = gx;
         dxyz1[row * 3 + 1] = gy;
@@ -667,6 +736,8 @@ label_count_kernel(const int64_t* __restrict__ target, int64_t rows, double* __r
     if ((threadIdx.x & 31) == 0 && local) atomicAdd(count, (double)local);
 }
 
+// DET: loss_sum is a [gridDim.x] array of block partials, written (ordered_sum_kernel adds them in block order).
+template <bool DET = false>
 __global__ void __launch_bounds__(256)
 cross_entropy_kernel(const float* __restrict__ x, int64_t ldx, const int64_t* __restrict__ target, int64_t rows, int C,
                      double* __restrict__ loss_sum, const double* __restrict__ count, float* __restrict__ dx, int64_t lddx,
@@ -710,8 +781,18 @@ cross_entropy_kernel(const float* __restrict__ x, int64_t ldx, const int64_t* __
     if (threadIdx.x == 0) {
         double t = 0.0;
         for (int i = 0; i < (int)(blockDim.x >> 5); ++i) t += red[i];
-        atomicAdd(loss_sum, t);
+        if (DET) loss_sum[blockIdx.x] = t;
+        else atomicAdd(loss_sum, t);
     }
+}
+
+// *out = sum of part[0, n): one warp, lane l adds the partials l, l + 32, ... in order, then a fixed butterfly.
+__global__ void ordered_sum_kernel(const double* __restrict__ part, int64_t n, double* __restrict__ out) {
+    double t = 0.0;
+    for (int64_t i = threadIdx.x; i < n; i += 32) t += part[i];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+    if (threadIdx.x == 0) *out = t;
 }
 
 __global__ void loss_finalize_kernel(const double* __restrict__ loss_sum, const double* __restrict__ count,
@@ -1123,7 +1204,8 @@ PN_EXPORT int pn_seg_metrics_accumulate(const int64_t* counts, int C, int64_t po
 // point (the first of equal minima, like torch's min(dim) on the CPU) for the backward pass.
 namespace pn {
 constexpr int CH_TILE = 256, CH_MAXD = 8;
-template <bool ARGMIN>
+// DET: total is a [gridDim.y * gridDim.x] array of block partials, written.
+template <bool ARGMIN, bool DET = false>
 __global__ void __launch_bounds__(CH_TILE)
 chamfer_kernel(const float* __restrict__ p1, int64_t aB, int64_t aN, int64_t aC, const float* __restrict__ p2, int64_t bB,
                int64_t bN, int64_t bC, int N, int M, int D, float* __restrict__ per_point, double* __restrict__ total,
@@ -1174,7 +1256,8 @@ chamfer_kernel(const float* __restrict__ p1, int64_t aB, int64_t aN, int64_t aC,
     if (threadIdx.x == 0) {
         double t = 0.0;
         for (int i = 0; i < CH_TILE / 32; ++i) t += red[i];
-        atomicAdd(total, t);
+        if (DET) total[blockIdx.y * gridDim.x + blockIdx.x] = t;
+        else atomicAdd(total, t);
     }
 }
 
@@ -1191,7 +1274,8 @@ __global__ void class_merge_kernel(const float* __restrict__ x, int64_t ldx, int
 
 // Backward of chamfer_batch / chamfer_non_batch: per p1 point, r = p1[n] - p2[a(n)] with the nearest p2 point a(n) of the
 // forward, d = ||r|| in the forward's rounding sequence, c = g*scale / d (0 where d == 0, as torch's norm backward);
-// dp1[n] = c*r (written), dp2[a(n)] -= c*r (fp32 atomics).
+// dp1[n] = c*r (written), dp2[a(n)] -= c*r (fp32 atomics; DET: dp2 is a [B*N, D] workspace of the terms -c*r, written).
+template <bool DET = false>
 __global__ void chamfer_bwd_kernel(const float* __restrict__ p1, int64_t aB, int64_t aN, int64_t aC, const float* __restrict__ p2,
                                    int64_t bB, int64_t bN, int64_t bC, int N, int M, int D, int64_t total,
                                    const int32_t* __restrict__ argmin, const float* __restrict__ g, float scale,
@@ -1213,7 +1297,8 @@ __global__ void chamfer_bwd_kernel(const float* __restrict__ p1, int64_t aB, int
         for (int c = 0; c < CH_MAXD; ++c) {
             if (c >= D) break;
             if (dp1) dp1[i * D + c] = coef * t[c];
-            if (dp2) atomicAdd(dp2 + (b * M + a) * D + c, -(coef * t[c]));
+            if (DET) dp2[i * D + c] = -(coef * t[c]);
+            else if (dp2) atomicAdd(dp2 + (b * M + a) * D + c, -(coef * t[c]));
         }
     }
 }
@@ -1233,7 +1318,9 @@ __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float 
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
-template <bool VEC, bool ROWS, bool COLS>
+// DET: rws / cws are [gridDim.x, B, N, 4] / [gridDim.y, B, M, 4]: each CTA stores its sums in the slot of its column chunk /
+// row tile instead of adding them (sqdist_partials_sum_kernel adds the slots in order).
+template <bool VEC, bool ROWS, bool COLS, bool DET = false>
 __global__ void __launch_bounds__(SDB_WARPS * 32, 2)
 sqdist_bwd_kernel(const float* __restrict__ g, int64_t gB, int64_t gN, const float* __restrict__ src, int64_t aB, int64_t aN,
                   int64_t aC, const float* __restrict__ dst, int64_t bB, int64_t bN, int64_t bC, int N, int M, int chunk,
@@ -1314,7 +1401,10 @@ sqdist_bwd_kernel(const float* __restrict__ g, int64_t gB, int64_t gN, const flo
                     const float4 u = part[buf][w][threadIdx.x];
                     t.x += u.x, t.y += u.y, t.z += u.z, t.w += u.w;
                 }
-                if (col < m_end) red_add_v4(cws + ((int64_t)b * M + col) * 4, t.x, t.y, t.z, t.w);
+                if (col < m_end) {
+                    if (DET) *reinterpret_cast<float4*>(cws + (((int64_t)blockIdx.y * gridDim.z + b) * M + col) * 4) = t;
+                    else red_add_v4(cws + ((int64_t)b * M + col) * 4, t.x, t.y, t.z, t.w);
+                }
             }
             buf ^= 1;   // the other buffer was last read before this step's barrier
         }
@@ -1329,8 +1419,26 @@ sqdist_bwd_kernel(const float* __restrict__ g, int64_t gB, int64_t gN, const flo
                 ry[r] += __shfl_xor_sync(0xffffffffu, ry[r], o);
                 rz[r] += __shfl_xor_sync(0xffffffffu, rz[r], o);
             }
-            if (lane == r && r0 + r < N) red_add_v4(rws + ((int64_t)b * N + r0 + r) * 4, rs[r], rx[r], ry[r], rz[r]);
+            if (lane == r && r0 + r < N) {
+                if (DET)
+                    *reinterpret_cast<float4*>(rws + (((int64_t)blockIdx.x * gridDim.z + b) * N + r0 + r) * 4) =
+                        make_float4(rs[r], rx[r], ry[r], rz[r]);
+                else
+                    red_add_v4(rws + ((int64_t)b * N + r0 + r) * 4, rs[r], rx[r], ry[r], rz[r]);
+            }
         }
+    }
+}
+
+// out[i] = sum_s part[s * n + i] (s ascending), over the n records of [slots, n] float4 partials.
+__global__ void sqdist_partials_sum_kernel(const float4* __restrict__ part, int slots, int64_t n, float4* __restrict__ out) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        float4 t = part[i];
+        for (int s = 1; s < slots; ++s) {
+            const float4 u = part[s * n + i];
+            t.x += u.x, t.y += u.y, t.z += u.z, t.w += u.w;
+        }
+        out[i] = t;
     }
 }
 
@@ -1446,4 +1554,341 @@ PN_EXPORT int pn_square_distance_bwd_f32(const float* g, int64_t gB, int64_t gN,
         src, aB, aN, aC, dst, bB, bN, bC, B, N, M, reinterpret_cast<const float4*>(rws), reinterpret_cast<const float4*>(cws),
         dsrc, ddst);
     return finish_launch("pn_square_distance_bwd_f32");
+}
+
+// ------------------------------------------------------------------------------------------------
+// Deterministic variants (torch.use_deterministic_algorithms): the same arithmetic as the entry points above, with every
+// floating-point sum taken in an order fixed by the shapes and the SM count -- per-block / per-slab partials in a
+// caller-provided workspace, added in block order, and scatter-adds pulled through the CSR of pn_csr_build (scatter.cu).
+namespace pn {
+static inline size_t bn_det_bytes(int64_t rows, int C) {
+    dim3 grid;
+    int64_t rpb;
+    stats_grid(rows, C, &grid, &rpb);
+    return sizeof(double) * 2 * (size_t)grid.x * (size_t)C;
+}
+
+static inline void grad_weight_f32_shape(int64_t rows, int cout, int cin, int64_t* splits, int64_t* rps) {
+    const int64_t tiles = ceil_div(cout, 64) * ceil_div(cin, 64);
+    int64_t sp = ceil_div((int64_t)sm_count() * 4, tiles);
+    int64_t r = ceil_div(ceil_div(rows, sp), 16) * 16;
+    if (r < 64) r = 64;
+    *rps = r;
+    *splits = ceil_div(rows, r);
+}
+
+int grad_weight_slab_sum(const float* ws, int64_t splits, int64_t bias_parts, int cout, int cin, float* dw, int64_t lddw, float* db,
+                         cudaStream_t st);
+
+static inline void sqdist_bwd_shape(int B, int N, int M, int* chunk, dim3* grid) {
+    const int64_t row_tiles = ceil_div(N, SDB_ROWS) * B;
+    const int64_t steps = ceil_div(M, SDB_STEP);
+    int64_t chunks = ceil_div((int64_t)sm_count() * 4, row_tiles);
+    if (chunks > steps) chunks = steps;
+    if (chunks > 65535) chunks = 65535;
+    *chunk = (int)(ceil_div(steps, chunks) * SDB_STEP);
+    *grid = dim3((unsigned)ceil_div(M, *chunk), (unsigned)ceil_div(N, SDB_ROWS), (unsigned)B);
+}
+}  // namespace pn
+
+PN_EXPORT size_t pn_bn_stats_workspace_bytes(int64_t rows, int C) {
+    return rows > 0 && C > 0 ? bn_det_bytes(rows, C) : 0;
+}
+
+#define PN_DET_WS(name, need)                                                                                              \
+    PN_REQUIRE(workspace, PN_ERR_BAD_ARG, name ": null workspace");                                                          \
+    PN_REQUIRE(workspace_bytes >= (need), PN_ERR_BAD_ARG, name ": workspace of %zu bytes, need %zu", workspace_bytes,     \
+               (size_t)(need));                                                                                              \
+    PN_REQUIRE(((uintptr_t)workspace & 15) == 0, PN_ERR_BAD_ARG, name ": workspace must be 16-byte aligned")
+
+PN_EXPORT int pn_bn_stats_det_f32(const float* y, int64_t ldy, int64_t rows, int C, double* sum, double* sumsq, void* workspace,
+                                  size_t workspace_bytes, pn_stream_t stream) {
+    PN_REQUIRE(y && sum && sumsq, PN_ERR_BAD_ARG, "pn_bn_stats_det_f32: null pointer");
+    PN_REQUIRE(rows > 0 && C > 0 && ldy >= C, PN_ERR_BAD_ARG, "pn_bn_stats_det_f32: bad shape");
+    PN_DET_WS("pn_bn_stats_det_f32", bn_det_bytes(rows, C));
+    dim3 grid;
+    int64_t rpb;
+    stats_grid(rows, C, &grid, &rpb);
+    cudaStream_t st = (cudaStream_t)stream;
+    double* part = static_cast<double*>(workspace);
+    col_stats_kernel<0, true><<<grid, 32 * ST_LANES, 0, st>>>(y, ldy, rows, C, rpb, nullptr, 0, nullptr, 1, nullptr, nullptr, nullptr,
+                                                               nullptr, 0, part, part + (int64_t)grid.x * C);
+    col_partials_sum_kernel<<<(unsigned)ceil_div(C, 128), 128, 0, st>>>(part, (int)grid.x, C, sum, sumsq);
+    return finish_launch("pn_bn_stats_det_f32");
+}
+
+PN_EXPORT int pn_bn_bwd_stats_det_f32(const float* y, int64_t ldy, int64_t rows, int C, const float* dz, int64_t lddz,
+                                      const int32_t* argmax, int K, const float* scale, const float* shift, const float* mean,
+                                      const float* invstd, int relu, double* s1, double* s2, void* workspace,
+                                      size_t workspace_bytes, pn_stream_t stream) {
+    PN_REQUIRE(y && dz && scale && shift && mean && invstd && s1 && s2, PN_ERR_BAD_ARG, "pn_bn_bwd_stats_det_f32: null pointer");
+    PN_REQUIRE(rows > 0 && C > 0 && ldy >= C && lddz >= C, PN_ERR_BAD_ARG, "pn_bn_bwd_stats_det_f32: bad shape");
+    PN_REQUIRE(!argmax || (K > 0 && rows % K == 0), PN_ERR_BAD_ARG, "pn_bn_bwd_stats_det_f32: rows must be a multiple of K");
+    PN_DET_WS("pn_bn_bwd_stats_det_f32", bn_det_bytes(rows, C));
+    dim3 grid;
+    int64_t rpb;
+    stats_grid(rows, C, &grid, &rpb);
+    cudaStream_t st = (cudaStream_t)stream;
+    double* p1 = static_cast<double*>(workspace);
+    double* p2 = p1 + (int64_t)grid.x * C;
+    if (argmax)
+        col_stats_kernel<2, true><<<grid, 32 * ST_LANES, 0, st>>>(y, ldy, rows, C, rpb, dz, lddz, argmax, K, scale, shift, mean,
+                                                                   invstd, relu, p1, p2);
+    else
+        col_stats_kernel<1, true><<<grid, 32 * ST_LANES, 0, st>>>(y, ldy, rows, C, rpb, dz, lddz, nullptr, 1, scale, shift, mean,
+                                                                   invstd, relu, p1, p2);
+    col_partials_sum_kernel<<<(unsigned)ceil_div(C, 128), 128, 0, st>>>(p1, (int)grid.x, C, s1, s2);
+    return finish_launch("pn_bn_bwd_stats_det_f32");
+}
+
+PN_EXPORT int pn_bn_eval_bwd_det_f32(const float* y, int64_t ldy, int64_t rows, int C, const float* dz, int64_t lddz,
+                                     const int32_t* argmax, int K, const float* scale, const float* shift, const float* mean,
+                                     const float* invstd, int relu, double* s1, double* s2, float* dy, int64_t lddy, float* dgamma,
+                                     float* dbeta, void* workspace, size_t workspace_bytes, pn_stream_t stream) {
+    PN_REQUIRE(y && dz && scale && shift && mean && invstd && s1 && s2 && dy, PN_ERR_BAD_ARG,
+               "pn_bn_eval_bwd_det_f32: null pointer");
+    PN_REQUIRE(rows > 0 && C > 0 && ldy >= C && lddz >= C && lddy >= C, PN_ERR_BAD_ARG, "pn_bn_eval_bwd_det_f32: bad shape");
+    PN_REQUIRE(!argmax || (K > 0 && rows % K == 0), PN_ERR_BAD_ARG, "pn_bn_eval_bwd_det_f32: rows must be a multiple of K");
+    PN_DET_WS("pn_bn_eval_bwd_det_f32", bn_det_bytes(rows, C));
+    dim3 grid;
+    int64_t rpb;
+    stats_grid(rows, C, &grid, &rpb);
+    cudaStream_t st = (cudaStream_t)stream;
+    double* p1 = static_cast<double*>(workspace);
+    double* p2 = p1 + (int64_t)grid.x * C;
+    if (argmax)
+        bn_eval_bwd_kernel<true, true><<<grid, 32 * ST_LANES, 0, st>>>(y, ldy, rows, C, rpb, dz, lddz, argmax, K, scale, shift, mean,
+                                                                      invstd, relu, p1, p2, dy, lddy);
+    else
+        bn_eval_bwd_kernel<false, true><<<grid, 32 * ST_LANES, 0, st>>>(y, ldy, rows, C, rpb, dz, lddz, nullptr, 1, scale, shift,
+                                                                       mean, invstd, relu, p1, p2, dy, lddy);
+    col_partials_sum_kernel<<<(unsigned)ceil_div(C, 128), 128, 0, st>>>(p1, (int)grid.x, C, s1, s2);
+    if (dgamma || dbeta) bn_eval_bwd_finalize_kernel<<<(unsigned)ceil_div(C, 128), 128, 0, st>>>(s1, s2, C, dgamma, dbeta);
+    return finish_launch("pn_bn_eval_bwd_det_f32");
+}
+
+PN_EXPORT size_t pn_grad_weight_f32_workspace_bytes(int64_t rows, int cout, int cin) {
+    if (rows <= 0 || cout <= 0 || cin <= 0) return 0;
+    int64_t splits, rps;
+    grad_weight_f32_shape(rows, cout, cin, &splits, &rps);
+    return sizeof(float) * (size_t)splits * ((size_t)cout * cin + cout);
+}
+
+// Launch the deterministic slab sum of the weight gradients (also used by grad_tc.cu).
+int pn::grad_weight_slab_sum(const float* ws, int64_t splits, int64_t bias_parts, int cout, int cin, float* dw, int64_t lddw, float* db,
+                         cudaStream_t st) {
+    slab_sum_kernel<<<ew_blocks((int64_t)cout * cin + cout, 256), 256, 0, st>>>(ws, (int)splits, (int)bias_parts, cout, cin, dw, lddw,
+                                                                                db);
+    return finish_launch("grad weight slab sum");
+}
+
+PN_EXPORT int pn_grad_weight_det_f32(const float* dy, int64_t lddy, const float* x, int64_t ldx, int64_t rows, int cout, int cin,
+                                     float* dw, int64_t lddw, float* db, void* workspace, size_t workspace_bytes,
+                                     pn_stream_t stream) {
+    PN_REQUIRE(dy && x && dw, PN_ERR_BAD_ARG, "pn_grad_weight_det_f32: null pointer");
+    PN_REQUIRE(rows > 0 && cout > 0 && cin > 0 && lddy >= cout && ldx >= cin && lddw >= cin, PN_ERR_BAD_ARG,
+               "pn_grad_weight_det_f32: bad shape");
+    PN_DET_WS("pn_grad_weight_det_f32", pn_grad_weight_f32_workspace_bytes(rows, cout, cin));
+    int64_t splits, rps;
+    grad_weight_f32_shape(rows, cout, cin, &splits, &rps);
+    PN_REQUIRE(splits <= 65535, PN_ERR_UNSUPPORTED, "pn_grad_weight_det_f32: too many row splits");
+    int vec_ok = 0;
+    if (((uintptr_t)dy % 16 == 0) && (lddy % 4 == 0)) vec_ok |= 1;
+    if (((uintptr_t)x % 16 == 0) && (ldx % 4 == 0)) vec_ok |= 2;
+    cudaStream_t st = (cudaStream_t)stream;
+    float* ws = static_cast<float*>(workspace);
+    float* wsb = ws + splits * (int64_t)cout * cin;
+    dim3 grid((unsigned)ceil_div(cout, 64), (unsigned)ceil_div(cin, 64), (unsigned)splits);
+    grad_weight_kernel<64, 64, 16, 4, 4, true><<<grid, 256, 0, st>>>(dy, lddy, x, ldx, rows, rps, cout, cin, ws, cin,
+                                                                      db ? wsb : nullptr, vec_ok);
+    const int e = finish_launch("pn_grad_weight_det_f32");
+    if (e != PN_OK) return e;
+    return grad_weight_slab_sum(ws, splits, splits, cout, cin, dw, lddw, db, st);
+}
+
+PN_EXPORT int pn_group_bwd_det_f32(const float* dgrouped, int64_t ldg, int col0, int D, const int32_t* offsets,
+                                   const int32_t* slots, int B, int N, float* dfeat, pn_stream_t stream) {
+    PN_REQUIRE(dgrouped && offsets && slots && dfeat, PN_ERR_BAD_ARG, "pn_group_bwd_det_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && D > 0 && col0 >= 0 && ldg >= col0 + D, PN_ERR_BAD_ARG, "pn_group_bwd_det_f32: bad shape");
+    return csr_pull(dgrouped, ldg, col0, D, 1, nullptr, offsets, slots, (int64_t)B * N, dfeat, (cudaStream_t)stream);
+}
+
+PN_EXPORT int pn_group_bwd_xyz_det_f32(const float* dgrouped, int64_t ldg, int col0, const int64_t* idx, const int32_t* offsets,
+                                       const int32_t* slots, int B, int N, int S, int K, float* dxyz, float* dnew_xyz,
+                                       pn_stream_t stream) {
+    PN_REQUIRE(dgrouped && idx && offsets && slots && dxyz, PN_ERR_BAD_ARG, "pn_group_bwd_xyz_det_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && S > 0 && K > 0 && col0 >= 0 && ldg >= col0 + 3, PN_ERR_BAD_ARG,
+               "pn_group_bwd_xyz_det_f32: bad shape");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dnew_xyz) {
+        const int64_t groups = (int64_t)B * S;
+        group_bwd_xyz_kernel<false><<<ew_blocks(groups * 32, 256), 256, 0, st>>>(dgrouped, ldg, col0, idx, N, S, K, groups, dxyz,
+                                                                                 dnew_xyz);
+        const int e = finish_launch("pn_group_bwd_xyz_det_f32");
+        if (e != PN_OK) return e;
+    }
+    return csr_pull(dgrouped, ldg, col0, 3, 1, nullptr, offsets, slots, (int64_t)B * N, dxyz, st);
+}
+
+PN_EXPORT int pn_three_interpolate_bwd_det_f32(const float* dx, int64_t ldx, int D1, int D2, const float* weight,
+                                               const int32_t* offsets, const int32_t* slots, int B, int N, int S, float* dpoints1,
+                                               float* dpoints2, pn_stream_t stream) {
+    PN_REQUIRE(dx && weight && offsets && slots && dpoints2 && (D1 == 0 || dpoints1), PN_ERR_BAD_ARG,
+               "pn_three_interpolate_bwd_det_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && S > 0 && D1 >= 0 && D2 > 0 && ldx >= D1 + D2, PN_ERR_BAD_ARG,
+               "pn_three_interpolate_bwd_det_f32: bad shape");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (D1 > 0) {
+        const int64_t total = (int64_t)B * N * D1;
+        three_interpolate_bwd_kernel<false><<<ew_blocks(total, 256), 256, 0, st>>>(dx, ldx, D1, 0, nullptr, nullptr, N, S, total,
+                                                                                   dpoints1, nullptr);
+        const int e = finish_launch("pn_three_interpolate_bwd_det_f32");
+        if (e != PN_OK) return e;
+    }
+    return csr_pull(dx, ldx, D1, D2, 3, weight, offsets, slots, (int64_t)B * S, dpoints2, st);
+}
+
+PN_EXPORT int pn_three_interpolate_bwd_xyz_det_f32(const float* dx, int64_t ldx, int D1, int D2, const int64_t* idx,
+                                                   const float* weight, const float* points2, int64_t p2B, int64_t p2S, int64_t p2C,
+                                                   const float* xyz1, int64_t aB, int64_t aN, int64_t aC, const float* xyz2,
+                                                   int64_t bB, int64_t bS, int64_t bC, int B, int N, int S, const int32_t* offsets,
+                                                   const int32_t* slots, float* workspace, float* dpoints1, float* dpoints2,
+                                                   float* dxyz1, float* dxyz2, pn_stream_t stream) {
+    PN_REQUIRE(dx && idx && weight && points2 && xyz1 && xyz2 && offsets && slots && workspace && dpoints2 && dxyz1 && dxyz2 &&
+                   (D1 == 0 || dpoints1),
+               PN_ERR_BAD_ARG, "pn_three_interpolate_bwd_xyz_det_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && D1 >= 0 && D2 > 0 && ldx >= D1 + D2, PN_ERR_BAD_ARG,
+               "pn_three_interpolate_bwd_xyz_det_f32: bad shape");
+    PN_REQUIRE(S >= 3, PN_ERR_BAD_ARG, "pn_three_interpolate_bwd_xyz_det_f32: need S >= 3 (got %d)", S);
+    const int64_t rows = (int64_t)B * N;
+    const bool vec = D1 % 4 == 0 && D2 % 4 == 0 && ldx % 4 == 0 && p2C == 1 && p2S % 4 == 0 && p2B % 4 == 0 &&
+                     ((uintptr_t)dx & 15) == 0 && ((uintptr_t)points2 & 15) == 0 && ((uintptr_t)dpoints1 & 15) == 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned grid = (unsigned)ew_blocks(rows * 32, 256);
+    if (vec)
+        three_interpolate_bwd_xyz_kernel<true, true><<<grid, 256, 0, st>>>(dx, ldx, D1, D2, idx, weight, points2, p2B, p2S, p2C, xyz1,
+                                                                          aB, aN, aC, xyz2, bB, bS, bC, N, S, rows, dpoints1,
+                                                                          dpoints2, dxyz1, workspace);
+    else
+        three_interpolate_bwd_xyz_kernel<false, true><<<grid, 256, 0, st>>>(dx, ldx, D1, D2, idx, weight, points2, p2B, p2S, p2C,
+                                                                           xyz1, aB, aN, aC, xyz2, bB, bS, bC, N, S, rows, dpoints1,
+                                                                           dpoints2, dxyz1, workspace);
+    int e = finish_launch("pn_three_interpolate_bwd_xyz_det_f32");
+    if (e != PN_OK) return e;
+    e = csr_pull(dx, ldx, D1, D2, 3, weight, offsets, slots, (int64_t)B * S, dpoints2, st);
+    if (e != PN_OK) return e;
+    return csr_pull(workspace, 3, 0, 3, 1, nullptr, offsets, slots, (int64_t)B * S, dxyz2, st);
+}
+
+PN_EXPORT size_t pn_cross_entropy_workspace_bytes(int64_t rows) {
+    return rows > 0 ? sizeof(double) * (2 + (size_t)ew_blocks(rows, 256)) : 0;
+}
+
+PN_EXPORT int pn_cross_entropy_det_f32(const float* x, int64_t ldx, const int64_t* target, int64_t rows, int C, void* workspace,
+                                       size_t workspace_bytes, float* loss, float* dx, int64_t lddx, float grad_scale,
+                                       pn_stream_t stream) {
+    PN_REQUIRE(x && target && loss, PN_ERR_BAD_ARG, "pn_cross_entropy_det_f32: null pointer");
+    PN_REQUIRE(rows > 0 && C > 0 && ldx >= C && (!dx || lddx >= C), PN_ERR_BAD_ARG, "pn_cross_entropy_det_f32: bad shape");
+    PN_DET_WS("pn_cross_entropy_det_f32", pn_cross_entropy_workspace_bytes(rows));
+    cudaStream_t st = (cudaStream_t)stream;
+    double* ws = static_cast<double*>(workspace);     // [sum, count, block partials]
+    cudaError_t e = cudaMemsetAsync(ws, 0, 2 * sizeof(double), st);
+    if (e != cudaSuccess) {
+        set_error("pn_cross_entropy_det_f32: %s", cudaGetErrorString(e));
+        return (int)e;
+    }
+    const unsigned blocks = ew_blocks(rows, 256);
+    label_count_kernel<<<blocks, 256, 0, st>>>(target, rows, ws + 1);      // integers in fp64: exact in any order
+    cross_entropy_kernel<true><<<blocks, 256, 0, st>>>(x, ldx, target, rows, C, ws + 2, ws + 1, dx, lddx, grad_scale);
+    ordered_sum_kernel<<<1, 32, 0, st>>>(ws + 2, blocks, ws);
+    loss_finalize_kernel<<<1, 1, 0, st>>>(ws, ws + 1, loss);
+    return finish_launch("pn_cross_entropy_det_f32");
+}
+
+PN_EXPORT size_t pn_chamfer_workspace_bytes(int B, int N) {
+    return B > 0 && N > 0 ? sizeof(double) * (size_t)B * (size_t)ceil_div(N, CH_TILE) : 0;
+}
+
+PN_EXPORT int pn_chamfer_det_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN,
+                                 int64_t bC, int B, int N, int M, int D, float* per_point, double* total, int32_t* argmin,
+                                 void* workspace, size_t workspace_bytes, pn_stream_t stream) {
+    PN_REQUIRE(p1 && p2 && total, PN_ERR_BAD_ARG, "pn_chamfer_det_f32: null pointer");
+    PN_REQUIRE(B > 0 && B <= 65535 && N > 0 && M > 0 && D > 0 && D <= CH_MAXD, PN_ERR_BAD_ARG,
+               "pn_chamfer_det_f32: bad sizes (D <= 8)");
+    PN_DET_WS("pn_chamfer_det_f32", pn_chamfer_workspace_bytes(B, N));
+    cudaStream_t st = (cudaStream_t)stream;
+    double* part = static_cast<double*>(workspace);
+    dim3 grid((unsigned)ceil_div(N, CH_TILE), (unsigned)B);
+    if (argmin)
+        chamfer_kernel<true, true><<<grid, CH_TILE, 0, st>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, per_point, part, argmin);
+    else
+        chamfer_kernel<false, true><<<grid, CH_TILE, 0, st>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, per_point, part, nullptr);
+    ordered_sum_kernel<<<1, 32, 0, st>>>(part, (int64_t)grid.x * grid.y, total);
+    return finish_launch("pn_chamfer_det_f32");
+}
+
+PN_EXPORT int pn_chamfer_bwd_det_f32(const float* p1, int64_t aB, int64_t aN, int64_t aC, const float* p2, int64_t bB, int64_t bN,
+                                     int64_t bC, int B, int N, int M, int D, const int32_t* argmin, const float* g_total,
+                                     float scale, const int32_t* offsets, const int32_t* slots, float* workspace, float* dp1,
+                                     float* dp2, pn_stream_t stream) {
+    PN_REQUIRE(p1 && p2 && argmin && g_total && (dp1 || dp2), PN_ERR_BAD_ARG, "pn_chamfer_bwd_det_f32: null pointer");
+    PN_REQUIRE(!dp2 || (offsets && slots && workspace), PN_ERR_BAD_ARG, "pn_chamfer_bwd_det_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && M > 0 && D > 0 && D <= CH_MAXD, PN_ERR_BAD_ARG, "pn_chamfer_bwd_det_f32: bad sizes (D <= 8)");
+    const int64_t total = (int64_t)B * N;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!dp2) {      // nothing is scattered: the default kernel is deterministic already
+        chamfer_bwd_kernel<<<ew_blocks(total, 256), 256, 0, st>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, total, argmin, g_total,
+                                                                 scale, dp1, nullptr);
+        return finish_launch("pn_chamfer_bwd_det_f32");
+    }
+    chamfer_bwd_kernel<true><<<ew_blocks(total, 256), 256, 0, st>>>(p1, aB, aN, aC, p2, bB, bN, bC, N, M, D, total, argmin, g_total,
+                                                                   scale, dp1, workspace);
+    const int e = finish_launch("pn_chamfer_bwd_det_f32");
+    if (e != PN_OK) return e;
+    return csr_pull(workspace, D, 0, D, 1, nullptr, offsets, slots, (int64_t)B * M, dp2, st);
+}
+
+PN_EXPORT size_t pn_square_distance_bwd_det_workspace_bytes(int B, int N, int M) {
+    if (B <= 0 || N <= 0 || M <= 0) return 0;
+    int chunk;
+    dim3 grid;
+    sqdist_bwd_shape(B, N, M, &chunk, &grid);
+    return sizeof(float) * 4 * ((size_t)(1 + grid.x) * B * N + (size_t)(1 + grid.y) * B * M);
+}
+
+PN_EXPORT int pn_square_distance_bwd_det_f32(const float* g, int64_t gB, int64_t gN, const float* src, int64_t aB, int64_t aN,
+                                             int64_t aC, const float* dst, int64_t bB, int64_t bN, int64_t bC, int B, int N, int M,
+                                             void* workspace, size_t workspace_bytes, float* dsrc, float* ddst, pn_stream_t stream) {
+    PN_REQUIRE(g && src && dst && (dsrc || ddst), PN_ERR_BAD_ARG, "pn_square_distance_bwd_det_f32: null pointer");
+    PN_REQUIRE(B > 0 && N > 0 && M > 0, PN_ERR_BAD_ARG, "pn_square_distance_bwd_det_f32: B, N, M must be positive");
+    PN_REQUIRE(B <= 65535 && ceil_div(N, SDB_ROWS) <= 65535, PN_ERR_UNSUPPORTED,
+               "pn_square_distance_bwd_det_f32: B <= 65535 and N <= %d", 65535 * SDB_ROWS);
+    PN_REQUIRE(gB >= 0 && gN >= 0, PN_ERR_BAD_ARG, "pn_square_distance_bwd_det_f32: negative stride of g");
+    PN_DET_WS("pn_square_distance_bwd_det_f32", pn_square_distance_bwd_det_workspace_bytes(B, N, M));
+    int chunk;
+    dim3 grid;
+    sqdist_bwd_shape(B, N, M, &chunk, &grid);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t nr = (int64_t)B * N, nc = (int64_t)B * M;
+    float* rws = static_cast<float*>(workspace);       // [B,N,4] sums, then [B,M,4] sums, then the per-CTA slots
+    float* cws = rws + nr * 4;
+    float* rpart = cws + nc * 4;                        // [grid.x, B, N, 4]
+    float* cpart = rpart + (int64_t)grid.x * nr * 4;    // [grid.y, B, M, 4]
+    const bool vec = ((uintptr_t)g & 15) == 0 && gN % 4 == 0 && (B == 1 || gB % 4 == 0);
+    const bool rows = dsrc != nullptr, cols = ddst != nullptr;
+    auto kern = vec ? (rows ? (cols ? sqdist_bwd_kernel<true, true, true, true> : sqdist_bwd_kernel<true, true, false, true>)
+                            : sqdist_bwd_kernel<true, false, true, true>)
+                    : (rows ? (cols ? sqdist_bwd_kernel<false, true, true, true> : sqdist_bwd_kernel<false, true, false, true>)
+                            : sqdist_bwd_kernel<false, false, true, true>);
+    kern<<<grid, SDB_WARPS * 32, 0, st>>>(g, gB, gN, src, aB, aN, aC, dst, bB, bN, bC, N, M, chunk, rpart, cpart);
+    if (rows)
+        sqdist_partials_sum_kernel<<<ew_blocks(nr, 256), 256, 0, st>>>(reinterpret_cast<const float4*>(rpart), (int)grid.x, nr,
+                                                                       reinterpret_cast<float4*>(rws));
+    if (cols)
+        sqdist_partials_sum_kernel<<<ew_blocks(nc, 256), 256, 0, st>>>(reinterpret_cast<const float4*>(cpart), (int)grid.y, nc,
+                                                                       reinterpret_cast<float4*>(cws));
+    sqdist_bwd_finish_kernel<<<ew_blocks(nr + nc, 256), 256, 0, st>>>(src, aB, aN, aC, dst, bB, bN, bC, B, N, M,
+                                                                     reinterpret_cast<const float4*>(rws),
+                                                                     reinterpret_cast<const float4*>(cws), dsrc, ddst);
+    return finish_launch("pn_square_distance_bwd_det_f32");
 }

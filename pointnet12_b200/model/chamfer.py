@@ -20,6 +20,12 @@ def _chamfer_sum(p1: torch.Tensor, p2: torch.Tensor) -> torch.Tensor:
     assert p1.size(0) == p2.size(0) and p1.size(2) == p2.size(2)
     B, N, D = p1.shape
     total = torch.empty((1,), dtype=torch.float64, device=p1.device)
+    if ops.deterministic():
+        ws = ops._workspace(nv.lib().pn_chamfer_workspace_bytes(B, N), p1.device)
+        with ops._on_device(p1):
+            nv.call("pn_chamfer_det_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, p2.shape[1], D, None,
+                    total.data_ptr(), None, ws.data_ptr(), ws.numel(), ops._stream())
+        return total[0]
     with ops._on_device(p1):
         nv.call("pn_chamfer_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, p2.shape[1], D, None,
                 total.data_ptr(), ops._stream())

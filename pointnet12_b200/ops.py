@@ -52,6 +52,49 @@ def _p(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
 
+def deterministic() -> bool:
+    """True when torch.are_deterministic_algorithms_enabled() (warn_only=True included).  The training and gradient wrappers
+    below read it at every launch and then take the deterministic variants of their kernels (*_det_* entry points: partial
+    sums added in a fixed order instead of floating-point atomics, scatter-adds pulled through the inverse index of csr()),
+    so that two runs from the same state give bitwise-equal results.  Torch's flag is the only switch."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _workspace(nbytes: int, device) -> torch.Tensor:
+    """A uint8 scratch buffer for a *_det_* entry point (the caching allocator aligns it to at least 512 bytes)."""
+    if nbytes <= 0:
+        raise ValueError("bad sizes for a deterministic workspace")
+    return torch.empty((int(nbytes),), dtype=torch.uint8, device=device)
+
+
+class Csr:
+    """Inverse index of a gather (pn_csr_build): the slots of destination k of batch b (key b * n_dst + k) are
+    slots[offsets[key] : offsets[key + 1]], in ascending order.  It depends on the index only, so one serves every gradient
+    through the same gather."""
+
+    __slots__ = ("offsets", "slots", "n_dst")
+
+
+def csr(idx: torch.Tensor, n_dst: int) -> Csr:
+    """idx int64 or int32 [B, ...] with values in [0, n_dst) (clamped like the gathers) -> Csr."""
+    _need_cuda(idx, "idx")
+    if idx.dtype not in (torch.int32, torch.int64):
+        idx = idx.long()
+    idx = idx if idx.is_contiguous() else idx.contiguous()
+    B = idx.shape[0]
+    per_batch = idx[0].numel()
+    n = B * per_batch
+    out = Csr()
+    out.n_dst = int(n_dst)
+    out.offsets = torch.empty((B * int(n_dst) + 1,), dtype=torch.int32, device=idx.device)
+    out.slots = torch.empty((max(n, 1),), dtype=torch.int32, device=idx.device)
+    ws = _workspace(nv.lib().pn_csr_workspace_bytes(n, B * int(n_dst)), idx.device)
+    with _on_device(idx):
+        nv.call("pn_csr_build", idx.data_ptr(), 64 if idx.dtype == torch.int64 else 32, n, per_batch, int(n_dst), B, ws.data_ptr(),
+                ws.numel(), out.offsets.data_ptr(), out.slots.data_ptr(), _stream())
+    return out
+
+
 class _on_device:
     """Make the tensor's device current for the duration of a launch (no-op in the common case)."""
 
@@ -324,6 +367,12 @@ def square_distance_backward(g: torch.Tensor, src: torch.Tensor, dst: torch.Tens
         g = g.contiguous()
     dsrc = torch.empty((B, N, 3), dtype=torch.float32, device=src.device) if need_src else None
     ddst = torch.empty((B, M, 3), dtype=torch.float32, device=src.device) if need_dst else None
+    if deterministic():
+        ws = _workspace(nv.lib().pn_square_distance_bwd_det_workspace_bytes(B, N, M), src.device)
+        with _on_device(src):
+            nv.call("pn_square_distance_bwd_det_f32", g.data_ptr(), g.stride(0), g.stride(1), src.data_ptr(), *src.stride(),
+                    dst.data_ptr(), *dst.stride(), B, N, M, ws.data_ptr(), ws.numel(), _p(dsrc), _p(ddst), _stream())
+        return dsrc, ddst
     ws = torch.empty((4 * B * (N + M),), dtype=torch.float32, device=src.device)
     with _on_device(src):
         nv.call("pn_square_distance_bwd_f32", g.data_ptr(), g.stride(0), g.stride(1), src.data_ptr(), *src.stride(),
@@ -452,6 +501,12 @@ def chamfer_argmin(p1: torch.Tensor, p2: torch.Tensor) -> Tuple[torch.Tensor, to
     B, N, D = p1.shape
     total = torch.empty((1,), dtype=torch.float64, device=p1.device)
     argmin = torch.empty((B, N), dtype=torch.int32, device=p1.device)
+    if deterministic():
+        ws = _workspace(nv.lib().pn_chamfer_workspace_bytes(B, N), p1.device)
+        with _on_device(p1):
+            nv.call("pn_chamfer_det_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, p2.shape[1], D, None,
+                    total.data_ptr(), argmin.data_ptr(), ws.data_ptr(), ws.numel(), _stream())
+        return total, argmin
     with _on_device(p1):
         nv.call("pn_chamfer_argmin_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, p2.shape[1], D, None,
                 total.data_ptr(), argmin.data_ptr(), _stream())
@@ -475,6 +530,15 @@ def chamfer_backward(p1: torch.Tensor, p2: torch.Tensor, argmin: torch.Tensor, g
     if not (need_p1 or need_p2):
         return None, None
     dp1 = torch.empty((B, N, D), dtype=torch.float32, device=p1.device) if need_p1 else None
+    if deterministic():
+        dp2 = torch.empty((B, M, D), dtype=torch.float32, device=p1.device) if need_p2 else None
+        inv = csr(argmin, M) if need_p2 else None
+        terms = torch.empty((B * N * D,), dtype=torch.float32, device=p1.device) if need_p2 else None
+        with _on_device(p1):
+            nv.call("pn_chamfer_bwd_det_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, M, D,
+                    argmin.data_ptr(), g.contiguous().data_ptr(), float(scale), _p(inv.offsets) if inv else None,
+                    _p(inv.slots) if inv else None, _p(terms), _p(dp1), _p(dp2), _stream())
+        return dp1, dp2
     dp2 = torch.zeros((B, M, D), dtype=torch.float32, device=p1.device) if need_p2 else None
     with _on_device(p1):
         nv.call("pn_chamfer_bwd_f32", p1.data_ptr(), *p1.stride(), p2.data_ptr(), *p2.stride(), B, N, M, D, argmin.data_ptr(),
@@ -938,7 +1002,7 @@ def bn_batch_stats(y: torch.Tensor, bn, momentum_update: bool = True) -> BatchSt
     st.rows = rows
     track = momentum_update and bn.track_running_stats and bn.running_mean is not None
     with _on_device(y):
-        nv.call("pn_bn_stats_f32", y.data_ptr(), _ld(y), rows, Cc, acc[0].data_ptr(), acc[1].data_ptr(), _stream())
+        _col_stats(y, acc)
         nv.call("pn_bn_finalize_f32", acc[0].data_ptr(), acc[1].data_ptr(), rows, Cc, _p(bn.weight), _p(bn.bias),
                 float(bn.eps), float(bn.momentum if bn.momentum is not None else 0.1),
                 bn.running_mean.data_ptr() if track else None, bn.running_var.data_ptr() if track else None,
@@ -947,6 +1011,17 @@ def bn_batch_stats(y: torch.Tensor, bn, momentum_update: bool = True) -> BatchSt
     if track:      # written through raw pointers: tell torch (the eval path refolds BatchNorm when a version changes)
         torch.autograd.graph.increment_version([b for b in (bn.running_mean, bn.running_var, bn.num_batches_tracked) if b is not None])
     return st
+
+
+def _col_stats(y: torch.Tensor, acc: torch.Tensor) -> None:
+    """acc[0] += column sums of y, acc[1] += of y*y (pn_bn_stats_f32, or its deterministic variant)."""
+    rows, Cc = y.shape
+    if deterministic():
+        ws = _workspace(nv.lib().pn_bn_stats_workspace_bytes(rows, Cc), y.device)
+        nv.call("pn_bn_stats_det_f32", y.data_ptr(), _ld(y), rows, Cc, acc[0].data_ptr(), acc[1].data_ptr(), ws.data_ptr(),
+                ws.numel(), _stream())
+    else:
+        nv.call("pn_bn_stats_f32", y.data_ptr(), _ld(y), rows, Cc, acc[0].data_ptr(), acc[1].data_ptr(), _stream())
 
 
 def bn_finalize(acc: torch.Tensor, rows: int, bn) -> BatchStats:
@@ -978,7 +1053,8 @@ def train_gemm(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], i
                packed: Optional[torch.Tensor] = None) -> torch.Tensor:
     """pn_train_gemm_bf16x3: y = f(x) @ W^T + bias with f = the normalise(+ReLU) of the layer that produced x (in_stats:
     its BatchStats; None = identity), column sums of y / y*y added to stats_acc (float64 [2, cout], zeroed by the caller).
-    W = w [cout, cin], or w^T for w [cin, cout] when transposed."""
+    W = w [cout, cin], or w^T for w [cin, cout] when transposed.  Deterministic mode: the GEMM without the column sums
+    (its epilogue adds them with atomics), then the deterministic column statistics of y."""
     x = _rowmat(x, "x")
     rows, cin = x.shape
     w = _f32(w, "w").contiguous()
@@ -989,12 +1065,16 @@ def train_gemm(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], i
     # packed: the weight image already converted by pn_train_pack_many (train.PackedWeights); else converted by this call
     scratch = packed if packed is not None else torch.empty((int(nv.lib().pn_train_gemm_scratch_bytes(cin, cout)),),
                                                             dtype=torch.uint8, device=x.device)
+    det_stats = stats_acc is not None and deterministic()
+    fused_acc = None if det_stats else stats_acc
     with _on_device(x):
         nv.call("pn_train_gemm_bf16x3", x.data_ptr(), _ld(x), rows, cin, _p(in_stats.scale) if in_stats is not None else None,
                 _p(in_stats.shift) if in_stats is not None else None, int(in_relu), None if packed is not None else w.data_ptr(),
                 int(transposed), _p(bias), cout,
-                y.data_ptr(), cout, _p(stats_acc[0]) if stats_acc is not None else None,
-                _p(stats_acc[1]) if stats_acc is not None else None, scratch.data_ptr(), _stream(), tag=(rows, cin, cout))
+                y.data_ptr(), cout, _p(fused_acc[0]) if fused_acc is not None else None,
+                _p(fused_acc[1]) if fused_acc is not None else None, scratch.data_ptr(), _stream(), tag=(rows, cin, cout))
+        if det_stats:
+            _col_stats(y, stats_acc)
     return y
 
 
@@ -1002,7 +1082,12 @@ def train_gemm_bnbwd(dy: torch.Tensor, w: torch.Tensor, prev_y: torch.Tensor, pr
                      transposed: bool = True, packed: Optional[torch.Tensor] = None) -> torch.Tensor:
     """pn_train_gemm_bnbwd_bf16x3: dz = dy @ W (w [cout_layer, cin_layer] given as stored, transposed=True) plus, in the
     epilogue, the two reductions of the BatchNorm backward of the layer BELOW (pre-normalisation output prev_y, statistics
-    prev_st) into acc (float64 [2, C], zeroed): bn_act_backward(..., acc=acc, acc_ready=True) then skips its own pass."""
+    prev_st) into acc (float64 [2, C], zeroed): bn_act_backward(..., acc=acc, acc_ready=True) then skips its own pass.
+    Deterministic mode: the plain GEMM, then the deterministic reductions of pn_bn_bwd_stats_det_f32."""
+    if deterministic():
+        dz = train_gemm(dy, w, None, transposed=transposed, packed=packed)
+        _bn_bwd_stats(prev_y, prev_st, dz, True, None, 1, acc)
+        return dz
     dy = _rowmat(dy, "dy")
     rows, cin = dy.shape
     w = _f32(w, "w").contiguous()
@@ -1027,7 +1112,11 @@ def train_gemm_bneval(dy: torch.Tensor, w: torch.Tensor, prev_y: torch.Tensor, p
     """pn_train_gemm_bneval_bf16x3: the input-gradient GEMM dy @ W of a layer whose input came from a BatchNorm with FIXED
     statistics prev_st (running_stats) applied to prev_y, with that BatchNorm's backward in the epilogue: returns the layer
     below's dy = scale * g (what bn_eval_backward would return for dz = dy @ W), adds its affine gradients to dgamma / dbeta.
-    acc: float64 [2, C] scratch, ZEROED."""
+    acc: float64 [2, C] scratch, ZEROED.  Deterministic mode: the plain GEMM, then bn_eval_backward's deterministic pass."""
+    if deterministic():
+        dz = train_gemm(dy, w, None, transposed=transposed, packed=packed)
+        return bn_eval_backward(prev_y, prev_st, dz, True, dgamma=dgamma, dbeta=dbeta, acc=acc) if dgamma is not None else \
+            bn_eval_backward(prev_y, prev_st, dz, True, acc=acc)[0]
     dy = _rowmat(dy, "dy")
     rows, cin = dy.shape
     w = _f32(w, "w").contiguous()
@@ -1089,9 +1178,22 @@ def bn_act_backward(y: torch.Tensor, st: BatchStats, dz: torch.Tensor, relu: boo
               st.shift.data_ptr(), st.mean.data_ptr(), st.invstd.data_ptr(), int(relu), acc[0].data_ptr(), acc[1].data_ptr())
     with _on_device(y):
         if not acc_ready:        # (acc_ready: the reductions were accumulated by the epilogue of train_gemm_bnbwd)
-            nv.call("pn_bn_bwd_stats_f32", *common, _stream())
+            _bn_bwd_stats(y, st, dz, relu, argmax, K, acc)
         nv.call("pn_bn_bwd_apply_f32", *common, dy.data_ptr(), Cc, dgamma.data_ptr(), dbeta.data_ptr(), _stream())
     return (dy, dgamma, dbeta) if fresh else dy
+
+
+def _bn_bwd_stats(y, st, dz, relu, argmax, K, acc) -> None:
+    """The two reductions of the batch-statistics BatchNorm backward into acc (pn_bn_bwd_stats_f32 or its deterministic
+    variant)."""
+    rows, Cc = y.shape
+    args = (y.data_ptr(), _ld(y), rows, Cc, dz.data_ptr(), _ld(dz), _p(argmax), int(K), st.scale.data_ptr(), st.shift.data_ptr(),
+            st.mean.data_ptr(), st.invstd.data_ptr(), int(relu), acc[0].data_ptr(), acc[1].data_ptr())
+    if deterministic():
+        ws = _workspace(nv.lib().pn_bn_stats_workspace_bytes(rows, Cc), y.device)
+        nv.call("pn_bn_bwd_stats_det_f32", *args, ws.data_ptr(), ws.numel(), _stream())
+    else:
+        nv.call("pn_bn_bwd_stats_f32", *args, _stream())
 
 
 def bn_eval_backward(y: torch.Tensor, st: BatchStats, dz: torch.Tensor, relu: bool = True,
@@ -1108,10 +1210,15 @@ def bn_eval_backward(y: torch.Tensor, st: BatchStats, dz: torch.Tensor, relu: bo
     if fresh:
         dgb = torch.zeros((2, Cc), dtype=torch.float32, device=y.device)
         dgamma, dbeta = dgb[0], dgb[1]
+    args = (y.data_ptr(), _ld(y), rows, Cc, dz.data_ptr(), _ld(dz), _p(argmax), int(K), st.scale.data_ptr(), st.shift.data_ptr(),
+            st.mean.data_ptr(), st.invstd.data_ptr(), int(relu), acc[0].data_ptr(), acc[1].data_ptr(), dy.data_ptr(), Cc,
+            dgamma.data_ptr(), dbeta.data_ptr())
     with _on_device(y):
-        nv.call("pn_bn_eval_bwd_f32", y.data_ptr(), _ld(y), rows, Cc, dz.data_ptr(), _ld(dz), _p(argmax), int(K),
-                st.scale.data_ptr(), st.shift.data_ptr(), st.mean.data_ptr(), st.invstd.data_ptr(), int(relu),
-                acc[0].data_ptr(), acc[1].data_ptr(), dy.data_ptr(), Cc, dgamma.data_ptr(), dbeta.data_ptr(), _stream())
+        if deterministic():
+            ws = _workspace(nv.lib().pn_bn_stats_workspace_bytes(rows, Cc), y.device)
+            nv.call("pn_bn_eval_bwd_det_f32", *args, ws.data_ptr(), ws.numel(), _stream())
+        else:
+            nv.call("pn_bn_eval_bwd_f32", *args, _stream())
     return (dy, dgamma, dbeta) if fresh else dy
 
 
@@ -1130,6 +1237,20 @@ def grad_weight(dy: torch.Tensor, x: torch.Tensor, dw: torch.Tensor, db: Optiona
         raise ValueError("grad_weight: shape mismatch")
     if engine == "auto":
         engine = "tc" if (mlp_mode() == "bf16x3" and cout * cin >= GRAD_TC_MIN_TILE) else "fp32"
+    if deterministic():
+        size = nv.lib().pn_grad_weight_f32_workspace_bytes if engine == "fp32" and x_stats is None else \
+            nv.lib().pn_grad_weight_bf16x3_workspace_bytes
+        ws = _workspace(size(rows, cout, cin), dy.device)
+        with _on_device(dy):
+            if x_stats is not None:
+                nv.call("pn_grad_weight_bn_det_bf16x3", dy.data_ptr(), _ld(dy), x.data_ptr(), _ld(x), x_stats.scale.data_ptr(),
+                        x_stats.shift.data_ptr(), int(x_relu), rows, cout, cin, dw.data_ptr(), cin, _p(db), ws.data_ptr(),
+                        ws.numel(), _stream())
+            else:
+                name = {"tc": "pn_grad_weight_det_bf16x3", "fp32": "pn_grad_weight_det_f32"}[engine]
+                nv.call(name, dy.data_ptr(), _ld(dy), x.data_ptr(), _ld(x), rows, cout, cin, dw.data_ptr(), cin, _p(db),
+                        ws.data_ptr(), ws.numel(), _stream())
+        return
     if x_stats is not None:
         # x is the PRE-normalisation output of the previous layer: its normalise + ReLU is applied on load (tensor cores only)
         with _on_device(dy):
@@ -1150,11 +1271,20 @@ def transpose(w: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def group_backward(dgrouped: torch.Tensor, col0: int, D: int, idx: torch.Tensor, N: int) -> torch.Tensor:
-    """dgrouped [B*S*K, >= col0+D] -> dfeat [B, N, D] (scatter-add through the ball-query indices)."""
+def group_backward(dgrouped: torch.Tensor, col0: int, D: int, idx: torch.Tensor, N: int,
+                   inv: Optional[Csr] = None) -> torch.Tensor:
+    """dgrouped [B*S*K, >= col0+D] -> dfeat [B, N, D] (scatter-add through the ball-query indices).  Deterministic mode: pulled
+    through inv = csr(idx, N) (built here when not given)."""
     dgrouped = _rowmat(dgrouped, "dgrouped")
     idx = _i64(idx, "idx")
     B, S, K = idx.shape
+    if deterministic():
+        inv = inv if inv is not None else csr(idx, N)
+        dfeat = torch.empty((B, N, D), dtype=torch.float32, device=dgrouped.device)
+        with _on_device(dgrouped):
+            nv.call("pn_group_bwd_det_f32", dgrouped.data_ptr(), _ld(dgrouped), int(col0), int(D), inv.offsets.data_ptr(),
+                    inv.slots.data_ptr(), B, int(N), dfeat.data_ptr(), _stream())
+        return dfeat
     dfeat = torch.zeros((B, N, D), dtype=torch.float32, device=dgrouped.device)
     with _on_device(dgrouped):
         nv.call("pn_group_bwd_f32", dgrouped.data_ptr(), _ld(dgrouped), int(col0), int(D), idx.data_ptr(), B, N, S, K,
@@ -1162,13 +1292,22 @@ def group_backward(dgrouped: torch.Tensor, col0: int, D: int, idx: torch.Tensor,
     return dfeat
 
 
-def three_interpolate_backward(dx: torch.Tensor, D1: int, D2: int, idx: torch.Tensor, weight: torch.Tensor, S: int):
-    """dx [B*N, D1+D2] -> (dpoints1 [B,N,D1] or None, dpoints2 [B,S,D2])."""
+def three_interpolate_backward(dx: torch.Tensor, D1: int, D2: int, idx: torch.Tensor, weight: torch.Tensor, S: int,
+                               inv: Optional[Csr] = None):
+    """dx [B*N, D1+D2] -> (dpoints1 [B,N,D1] or None, dpoints2 [B,S,D2]).  Deterministic mode: dpoints2 pulled through
+    inv = csr(idx, S)."""
     dx = _rowmat(dx, "dx")
     idx = _i64(idx, "idx")
     weight = _f32(weight, "weight").contiguous()
     B, N, _ = idx.shape
     dp1 = torch.empty((B, N, D1), dtype=torch.float32, device=dx.device) if D1 else None
+    if deterministic():
+        inv = inv if inv is not None else csr(idx, S)
+        dp2 = torch.empty((B, S, D2), dtype=torch.float32, device=dx.device)
+        with _on_device(dx):
+            nv.call("pn_three_interpolate_bwd_det_f32", dx.data_ptr(), _ld(dx), int(D1), int(D2), weight.data_ptr(),
+                    inv.offsets.data_ptr(), inv.slots.data_ptr(), B, N, int(S), _p(dp1), dp2.data_ptr(), _stream())
+        return dp1, dp2
     dp2 = torch.zeros((B, S, D2), dtype=torch.float32, device=dx.device)
     with _on_device(dx):
         nv.call("pn_three_interpolate_bwd_f32", dx.data_ptr(), _ld(dx), int(D1), int(D2), idx.data_ptr(), weight.data_ptr(),
@@ -1176,12 +1315,21 @@ def three_interpolate_backward(dx: torch.Tensor, D1: int, D2: int, idx: torch.Te
     return dp1, dp2
 
 
-def group_backward_xyz(dgrouped: torch.Tensor, col0: int, idx: torch.Tensor, N: int, recentred: bool = True):
+def group_backward_xyz(dgrouped: torch.Tensor, col0: int, idx: torch.Tensor, N: int, recentred: bool = True,
+                       inv: Optional[Csr] = None):
     """Coordinate gradient of the grouping: dgrouped [B*S*K, >= col0+3] with the xyz_rel columns at col0 -> (dxyz [B,N,3],
     dnew_xyz [B,S,3] = -sum over each group, or None when the group was not recentred (group-all))."""
     dgrouped = _rowmat(dgrouped, "dgrouped")
     idx = _i64(idx, "idx")
     B, S, K = idx.shape
+    if deterministic():          # dxyz pulled through inv = csr(idx, N)
+        inv = inv if inv is not None else csr(idx, N)
+        dxyz = torch.empty((B, N, 3), dtype=torch.float32, device=dgrouped.device)
+        dnew = torch.empty((B, S, 3), dtype=torch.float32, device=dgrouped.device) if recentred else None
+        with _on_device(dgrouped):
+            nv.call("pn_group_bwd_xyz_det_f32", dgrouped.data_ptr(), _ld(dgrouped), int(col0), idx.data_ptr(),
+                    inv.offsets.data_ptr(), inv.slots.data_ptr(), B, int(N), S, K, dxyz.data_ptr(), _p(dnew), _stream())
+        return dxyz, dnew
     dxyz = torch.zeros((B, N, 3), dtype=torch.float32, device=dgrouped.device)
     dnew = torch.empty((B, S, 3), dtype=torch.float32, device=dgrouped.device) if recentred else None
     with _on_device(dgrouped):
@@ -1191,7 +1339,7 @@ def group_backward_xyz(dgrouped: torch.Tensor, col0: int, idx: torch.Tensor, N: 
 
 
 def three_interpolate_backward_xyz(dx: torch.Tensor, D1: int, D2: int, idx: torch.Tensor, weight: torch.Tensor,
-                                   points2: torch.Tensor, xyz1: torch.Tensor, xyz2: torch.Tensor):
+                                   points2: torch.Tensor, xyz1: torch.Tensor, xyz2: torch.Tensor, inv: Optional[Csr] = None):
     """three_interpolate_backward plus the gradient through the 3-NN weights: points2 [B,S,D2], xyz1 [B,N,3], xyz2 [B,S,3]
     (the forward's inputs, any strides) -> (dpoints1 [B,N,D1] or None, dpoints2 [B,S,D2], dxyz1 [B,N,3], dxyz2 [B,S,3]).
     Needs S >= 3."""
@@ -1203,6 +1351,18 @@ def three_interpolate_backward_xyz(dx: torch.Tensor, D1: int, D2: int, idx: torc
     B, N, _ = idx.shape
     S = points2.shape[1]
     dp1 = torch.empty((B, N, D1), dtype=torch.float32, device=dx.device) if D1 else None
+    if deterministic():          # dpoints2 and dxyz2 pulled through inv = csr(idx, S)
+        inv = inv if inv is not None else csr(idx, S)
+        dp2 = torch.empty((B, S, D2), dtype=torch.float32, device=dx.device)
+        dxyz1 = torch.empty((B, N, 3), dtype=torch.float32, device=dx.device)
+        dxyz2 = torch.empty((B, S, 3), dtype=torch.float32, device=dx.device)
+        terms = torch.empty((B * N * 9,), dtype=torch.float32, device=dx.device)
+        with _on_device(dx):
+            nv.call("pn_three_interpolate_bwd_xyz_det_f32", dx.data_ptr(), _ld(dx), int(D1), int(D2), idx.data_ptr(),
+                    weight.data_ptr(), points2.data_ptr(), *points2.stride(), xyz1.data_ptr(), *xyz1.stride(), xyz2.data_ptr(),
+                    *xyz2.stride(), B, N, S, inv.offsets.data_ptr(), inv.slots.data_ptr(), terms.data_ptr(), _p(dp1),
+                    dp2.data_ptr(), dxyz1.data_ptr(), dxyz2.data_ptr(), _stream())
+        return dp1, dp2, dxyz1, dxyz2
     dp2 = torch.zeros((B, S, D2), dtype=torch.float32, device=dx.device)
     dxyz1 = torch.empty((B, N, 3), dtype=torch.float32, device=dx.device)
     dxyz2 = torch.zeros((B, S, 3), dtype=torch.float32, device=dx.device)
@@ -1241,6 +1401,14 @@ def cross_entropy(x: torch.Tensor, target: torch.Tensor, want_grad: bool = True,
     rows, Cc = x.shape
     if target.numel() != rows:
         raise ValueError("target must hold one label per row")
+    if deterministic():
+        ws = _workspace(nv.lib().pn_cross_entropy_workspace_bytes(rows), x.device)
+        loss = torch.empty((), dtype=torch.float32, device=x.device)
+        dx = torch.empty((rows, Cc), dtype=torch.float32, device=x.device) if want_grad else None
+        with _on_device(x):
+            nv.call("pn_cross_entropy_det_f32", x.data_ptr(), _ld(x), target.data_ptr(), rows, Cc, ws.data_ptr(), ws.numel(),
+                    loss.data_ptr(), _p(dx), Cc, float(grad_scale), _stream())
+        return loss, dx
     scratch = torch.empty((2,), dtype=torch.float64, device=x.device)
     loss = torch.empty((), dtype=torch.float32, device=x.device)
     dx = torch.empty((rows, Cc), dtype=torch.float32, device=x.device) if want_grad else None

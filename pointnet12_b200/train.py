@@ -327,10 +327,11 @@ class SetAbstractionFn(torch.autograd.Function):
                                   arena=ctx.arena)
         # the feature channels sit behind the three xyz columns (SSG order) or in front of them (MSG order)
         msg = ctx.branch is not None
-        dpts = ops.group_backward(dx0, 0 if msg else 3, D, ctx.idx, N) if need_dpts else None
+        inv = ops.csr(ctx.idx, N) if ops.deterministic() and need_dpts and need_xyz else None    # one inverse index for both
+        dpts = ops.group_backward(dx0, 0 if msg else 3, D, ctx.idx, N, inv=inv) if need_dpts else None
         dxyz = dnew = None
         if need_xyz:
-            dxyz, dnew = ops.group_backward_xyz(dx0, D if msg else 0, ctx.idx, N, recentred=ctx.needs_input_grad[4])
+            dxyz, dnew = ops.group_backward_xyz(dx0, D if msg else 0, ctx.idx, N, recentred=ctx.needs_input_grad[4], inv=inv)
         ctx.saved = None
         return (None, None, dxyz if ctx.needs_input_grad[2] else None, dpts, dnew, None, *_layer_grads(layers, grads))
 
@@ -681,10 +682,13 @@ class GroupPointsFn(torch.autograd.Function):
     def backward(ctx, dout):
         rows = _rows_of(dout, 3 + ctx.D)
         dxyz = dnew = dpts = None
-        if ctx.needs_input_grad[0] or ctx.needs_input_grad[2]:
-            dxyz, dnew = ops.group_backward_xyz(rows, 0, ctx.idx, ctx.N, recentred=ctx.recentred and ctx.needs_input_grad[2])
-        if ctx.D and ctx.needs_input_grad[1]:
-            dpts = ops.group_backward(rows, 3, ctx.D, ctx.idx, ctx.N)
+        need_xyz, need_pts = ctx.needs_input_grad[0] or ctx.needs_input_grad[2], ctx.D and ctx.needs_input_grad[1]
+        inv = ops.csr(ctx.idx, ctx.N) if ops.deterministic() and need_xyz and need_pts else None    # one inverse index for both
+        if need_xyz:
+            dxyz, dnew = ops.group_backward_xyz(rows, 0, ctx.idx, ctx.N, recentred=ctx.recentred and ctx.needs_input_grad[2],
+                                                inv=inv)
+        if need_pts:
+            dpts = ops.group_backward(rows, 3, ctx.D, ctx.idx, ctx.N, inv=inv)
         return dxyz if ctx.needs_input_grad[0] else None, dpts, dnew, None, None
 
 
@@ -1229,7 +1233,8 @@ class GraphedTrainStep:
         if not self.net.training:
             raise RuntimeError("GraphedTrainStep: call net.train() first")
         # a graph bakes in which BatchNorm layers use batch statistics and which dropouts apply: one capture per mode set
-        key = (tuple(points.shape), points.device, _modes(self._mode_modules))
+        # ... and which kernels run: torch.use_deterministic_algorithms selects the deterministic variants at capture time
+        key = (tuple(points.shape), points.device, _modes(self._mode_modules), ops.deterministic())
         st = self._graphs.get(key)
         if st is None:
             st = self._graphs[key] = self._build(points, target)
@@ -1392,7 +1397,7 @@ class GraphedStep:
         # a graph bakes in the input shapes and dtypes and the draws of the modes it was captured with (a Dropout in .eval()
         # draws no seed): one capture, with its own draw log, per key
         key = (tuple((tuple(t.shape), t.dtype) for t in xs), as_tuple, tuple(target.shape), xs[0].device,
-               _modes(self._mode_modules))
+               _modes(self._mode_modules), ops.deterministic())
         st = self._graphs.get(key)
         if st is None:
             st = self._graphs[key] = self._build(xs, as_tuple, target)
