@@ -21,6 +21,10 @@
  *   - Return value: 0 on success; negative pn_status on bad arguments; positive = cudaError_t of
  *     the launch.  pn_last_error_string() describes the last failure on the calling thread.
  *     Nothing is printed and nothing throws.
+ *   - pointnet12_b200/_native.py builds its ctypes bindings by reading the declarations below, so they use only
+ *     int, int32_t, int64_t, size_t and float by value, pointers (bound as void*), typedefs and structs of these (array
+ *     fields sized by an integer #define), enums, and the return types int, size_t and const char*; any other spelling
+ *     makes that module's import fail.
  */
 #ifndef PN12_B200_H
 #define PN12_B200_H

@@ -16,140 +16,79 @@ HEADER = os.path.join(os.path.dirname(PKG), "include", "pn12_b200.h")
 
 _lib = None
 
-vp, i64, i32, f32 = C.c_void_p, C.c_int64, C.c_int, C.c_float
-
-MLP_MAX_LAYERS = 6
-
-
-class MlpDesc(C.Structure):
-    """pn_mlp_desc of include/pn12_b200.h."""
-    _fields_ = [("nlayers", C.c_int), ("cin", C.c_int * MLP_MAX_LAYERS), ("cout", C.c_int * MLP_MAX_LAYERS),
-                ("relu", C.c_int * MLP_MAX_LAYERS)]
+# The C spellings include/pn12_b200.h may use.  Every pointer is passed as c_void_p: the header's types cannot tell host
+# from device pointers, and c_void_p takes an integer address (data_ptr()) as well as a byref() or a ctypes array.
+_SCALARS = {"int": C.c_int, "int32_t": C.c_int, "int64_t": C.c_int64, "size_t": C.c_size_t, "float": C.c_float}
+_RETURNS = {"int": C.c_int, "size_t": C.c_size_t, "const char*": C.c_char_p}
 
 
-_descp = C.POINTER(MlpDesc)
+def _spelling(t: str) -> str:
+    return re.sub(r"\s*\*", "*", " ".join(t.split()))
 
 
-class LaunchOpts(C.Structure):
-    """pn_launch_opts of include/pn12_b200.h: per-call launch options (all zeros = defaults)."""
-    _fields_ = [("mlp_passes", C.c_int), ("mlp_engine", C.c_int), ("reserved_sms", C.c_int), ("fps_cluster", C.c_int),
-                ("fps_threads", C.c_int), ("fps_exchange", C.c_int), ("tile_counter", C.c_void_p), ("mlp_debug", C.c_void_p)]
+def parse_header(text: str):
+    """(integer #defines, structs: name -> ctypes.Structure, functions: name -> (argtypes, restype)) of a header written
+    in the small C grammar of include/pn12_b200.h.  Anything outside it raises a ValueError naming the declaration."""
+    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
+    text = re.sub(r"#ifdef __cplusplus.*?#endif", "", text, flags=re.S)
+    consts = {k: int(v) for k, v in re.findall(r"^\s*#\s*define\s+(\w+)\s+(-?\d+)\s*$", text, flags=re.M)}
+    text = re.sub(r"^\s*#.*$", "", text, flags=re.M)
+    decl_re = r"[^;{}]*(?:\{[^{}]*\}[^;{}]*)?;"
+    rest = re.sub(decl_re, "", text).strip()
+    if rest:
+        raise ValueError(f"cannot parse declaration: {rest}")
+    types, structs, functions = dict(_SCALARS), {}, {}
+
+    def var(s: str, decl: str):  # "T name" or "T name[N]" -> (name, ctype, spelling of T)
+        m = re.fullmatch(r"(.*?)\s*\b(\w+)\s*(?:\[\s*(\w+)\s*\])?", s.strip())
+        spelling = _spelling(m.group(1)) if m else ""
+        t = C.c_void_p if "*" in spelling else types.get(spelling)
+        if t is None:
+            raise ValueError(f"unsupported type in {s.strip()!r} of: {decl}")
+        if m.group(3):
+            n = int(m.group(3)) if m.group(3).isdigit() else consts.get(m.group(3))
+            if n is None:
+                raise ValueError(f"unknown array bound {m.group(3)!r} in: {decl}")
+            t = t * n
+        return m.group(2), t, spelling
+
+    for decl in (" ".join(d[:-1].split()) for d in re.findall(decl_re, text)):
+        if not decl or re.fullmatch(r"enum \w+ \{[^{}]*\}", decl):
+            continue
+        if m := re.fullmatch(r"typedef struct (\w+) \{([^{}]*)\} \1", decl):
+            fields = []
+            for field in (f for f in m.group(2).split(";") if f.strip()):
+                first, *more = field.split(",")
+                name, t, spelling = var(first, decl)
+                if more and "*" in spelling:
+                    raise ValueError(f"one pointer field per declaration in: {decl}")
+                fields += [(name, t)] + [var(f"{spelling} {v}", decl)[:2] for v in more]
+            structs[m.group(1)] = type(m.group(1), (C.Structure,), {"_fields_": fields})
+        elif m := re.fullmatch(r"typedef ([^{}\[\]]+)", decl):
+            name, t, _ = var(m.group(1), decl)
+            types[name] = t
+        elif m := re.fullmatch(r"(.+?) ?\b(pn_\w+) ?\(([^\[\]]*)\)", decl):
+            restype = _RETURNS.get(_spelling(m.group(1)))
+            if restype is None:
+                raise ValueError(f"unsupported return type in: {decl}")
+            params = [] if m.group(3).strip() == "void" else m.group(3).split(",")
+            functions[m.group(2)] = ([var(p, decl)[1] for p in params], restype)
+        else:
+            raise ValueError(f"cannot parse declaration: {decl}")
+    return consts, structs, functions
 
 
-_optsp = C.POINTER(LaunchOpts)
-
-# name -> argtypes, mirroring include/pn12_b200.h
-_SIGNATURES = {
-    "pn_version": [],
-    "pn_device_check": [C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)],
-    "pn_fps_f32": [vp, i64, i64, i64, i32, i32, i32, vp, vp, _optsp, vp],
-    "pn_square_distance_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, vp, vp],
-    "pn_square_distance_bwd_f32": [vp, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, vp, vp, vp, vp],
-    "pn_ball_query_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, f32, i32, vp, vp],
-    "pn_ball_grid_build_f32": [vp, i64, i64, i64, i32, i32, f32, vp, C.c_size_t, vp],
-    "pn_ball_query_grid_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, f32, i32, vp, C.c_size_t, i32, vp, vp,
-                               vp],
-    "pn_fps_progress_f32": [vp, i64, i64, i64, i32, i32, i32, vp, vp, vp, _optsp, vp],
-    "pn_fps_sorted_f32": [vp, i64, i64, i64, vp, C.c_size_t, i32, i32, i32, vp, vp, vp, _optsp, vp],
-    "pn_fps_launch_info": [i32, i32, i32, _optsp, C.POINTER(i32), C.POINTER(C.c_size_t)],
-    "pn_ball_query_stream_f32": [vp, i64, i64, i64, vp, i32, i32, i32, i32, f32, i32, vp, C.c_size_t, i32, C.c_size_t, vp, vp,
-                                 vp],
-    "pn_index_points_f32": [vp, i64, i64, i64, i32, i32, i32, vp, i64, vp, vp],
-    "pn_group_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, vp, i64, i64, i64, vp, i32, i32, i32, i32, i32, vp,
-                     i64, vp],
-    "pn_linear_f32": [vp, i64, i64, vp, i64, vp, i64, i32, i32, i64, i32, i32, vp, i64, i64, vp],
-    "pn_group_max_f32": [vp, i64, i64, i32, i32, vp, i64, vp],
-    "pn_three_nn_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, vp, vp, vp],
-    "pn_three_nn_blocks_build_f32": [vp, i64, i64, i64, i32, i32, vp, C.c_size_t, vp],
-    "pn_three_nn_blocks_f32": [vp, i64, i64, i64, vp, i64, i64, vp, C.c_size_t, i32, i32, i32, i32, vp, vp, vp],
-    "pn_three_interpolate_f32": [vp, i64, i64, i64, i32, vp, i64, i64, i64, i32, i32, vp, vp, i32, i32, vp, i64, i64,
-                                 vp],
-    "pn_log_softmax_f32": [vp, i64, i64, i32, vp, i64, vp],
-    "pn_argmax_labels_u8": [vp, i64, i64, i32, vp, vp],
-    "pn_mlp_pack_bf16x3": [_descp, C.POINTER(vp), C.POINTER(vp), vp, vp],
-    "pn_mlp_pack_t_bf16x3": [_descp, C.POINTER(vp), C.POINTER(vp), C.POINTER(i32), vp, vp],
-    "pn_mlp_rows_bf16x3": [_descp, vp, vp, i64, i64, i32, vp, i64, _optsp, vp],
-    "pn_sa_mlp_max_bf16x3": [_descp, vp, vp, i64, i64, i64, vp, i64, i64, i64, i32, vp, i64, i64, i64, vp, i32, i32, i32,
-                             i32, i32, vp, i64, _optsp, vp],
-    "pn_sa_mlp_bf16x3": [_descp, vp, vp, i64, i64, i64, vp, i64, i64, i64, i32, vp, i64, i64, i64, vp, i32, i32, i32,
-                         i32, i32, i32, vp, i64, _optsp, vp],
-    "pn_fp_mlp_bf16x3": [_descp, vp, vp, i64, i64, i64, i32, vp, i64, i64, i64, i32, i32, vp, vp, i32, vp, i64, i64, vp,
-                         i64, i32, i32, i32, vp, i64, _optsp, vp],
-    "pn_ball_grid_order": [vp, i32, C.POINTER(vp), C.POINTER(i64), C.POINTER(i64)],
-    "pn_bn_stats_f32": [vp, i64, i64, i32, vp, vp, vp],
-    "pn_bn_finalize_f32": [vp, vp, i64, i32, vp, vp, f32, f32, vp, vp, vp, vp, vp, vp, vp, vp],
-    "pn_bn_act_f32": [vp, i64, i64, i32, vp, vp, i32, vp, i64, vp],
-    "pn_bn_act_max_f32": [vp, i64, i64, i32, i32, vp, vp, i32, vp, i64, vp, vp],
-    "pn_bn_bwd_stats_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp],
-    "pn_bn_bwd_apply_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, vp, vp],
-    "pn_bn_eval_bwd_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, vp, vp],
-    "pn_grad_weight_f32": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp],
-    "pn_grad_weight_bf16x3": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp],
-    "pn_grad_weight_bn_bf16x3": [vp, i64, vp, i64, vp, vp, i32, i64, i32, i32, vp, i64, vp, vp],
-    "pn_train_gemm_supported": [i32, i32],
-    "pn_train_pack_many": [vp, i32, i32, i32, vp],
-    "pn_train_gemm_bf16x3": [vp, i64, i64, i32, vp, vp, i32, vp, i32, vp, i32, vp, i64, vp, vp, vp, vp],
-    "pn_train_gemm_bnbwd_bf16x3": [vp, i64, i64, i32, vp, i32, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp],
-    "pn_train_gemm_bneval_bf16x3": [vp, i64, i64, i32, vp, i32, i32, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
-    "pn_transpose_f32": [vp, i32, i32, vp, vp],
-    "pn_group_bwd_f32": [vp, i64, i32, i32, vp, i32, i32, i32, i32, vp, vp],
-    "pn_three_interpolate_bwd_f32": [vp, i64, i32, i32, vp, vp, i32, i32, i32, vp, vp, vp],
-    "pn_group_bwd_xyz_f32": [vp, i64, i32, vp, i32, i32, i32, i32, vp, vp, vp],
-    "pn_three_interpolate_bwd_xyz_f32": [vp, i64, i32, i32, vp, vp, vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64,
-                                         i32, i32, i32, vp, vp, vp, vp, vp],
-    "pn_dropout_f32": [vp, i64, i64, i32, f32, vp, vp, vp, vp, i64, vp],
-    "pn_cross_entropy_f32": [vp, i64, vp, i64, i32, vp, vp, vp, i64, f32, vp],
-    "pn_log_softmax_bwd_f32": [vp, i64, vp, i64, i64, i32, vp, i64, vp],
-    "pn_adam_f32": [vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, i64, f32, vp],
-    "pn_adam_dev_f32": [vp, vp, vp, vp, i64, vp, vp, f32, f32, f32, f32, f32, vp],
-    "pn_seg_metrics_f32": [vp, i64, vp, i64, i32, vp, vp, vp],
-    "pn_scan_filter_f32": [vp, vp, vp, i32, i64, vp, i32, i32, f32, f32, f32, f32, vp, vp, vp, C.c_size_t, vp],
-    "pn_scan_sample_f32": [vp, vp, vp, i32, vp, i32, vp, vp, i32, vp, vp, f32, f32, vp, vp, vp, vp],
-    "pn_chamfer_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp],
-    "pn_chamfer_argmin_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp],
-    "pn_chamfer_bwd_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp],
-    "pn_class_merge_f32": [vp, i64, i64, i32, i32, vp, vp, vp, vp],
-    "pn_seg_metrics_accumulate": [vp, i32, i64, vp, vp, vp, vp, vp],
-    # deterministic variants (*_det_*): the default signature plus a workspace (pointer, bytes) or a prebuilt CSR
-    "pn_bn_stats_det_f32": [vp, i64, i64, i32, vp, vp, vp, C.c_size_t, vp],
-    "pn_bn_bwd_stats_det_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, C.c_size_t, vp],
-    "pn_bn_eval_bwd_det_f32": [vp, i64, i64, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp, i64, vp, vp, vp, C.c_size_t,
-                               vp],
-    "pn_grad_weight_det_f32": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp, C.c_size_t, vp],
-    "pn_grad_weight_det_bf16x3": [vp, i64, vp, i64, i64, i32, i32, vp, i64, vp, vp, C.c_size_t, vp],
-    "pn_grad_weight_bn_det_bf16x3": [vp, i64, vp, i64, vp, vp, i32, i64, i32, i32, vp, i64, vp, vp, C.c_size_t, vp],
-    "pn_csr_build": [vp, i32, i64, i64, i32, i32, vp, C.c_size_t, vp, vp, vp],
-    "pn_csr_pull_f32": [vp, i64, i32, i32, i32, vp, vp, vp, i64, vp, vp],
-    "pn_group_bwd_det_f32": [vp, i64, i32, i32, vp, vp, i32, i32, vp, vp],
-    "pn_group_bwd_xyz_det_f32": [vp, i64, i32, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp],
-    "pn_three_interpolate_bwd_det_f32": [vp, i64, i32, i32, vp, vp, vp, i32, i32, i32, vp, vp, vp],
-    "pn_three_interpolate_bwd_xyz_det_f32": [vp, i64, i32, i32, vp, vp, vp, i64, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64,
-                                             i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp],
-    "pn_cross_entropy_det_f32": [vp, i64, vp, i64, i32, vp, C.c_size_t, vp, vp, i64, f32, vp],
-    "pn_chamfer_det_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, vp, vp, C.c_size_t, vp],
-    "pn_chamfer_bwd_det_f32": [vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp, vp, vp, vp],
-    "pn_square_distance_bwd_det_f32": [vp, i64, i64, vp, i64, i64, i64, vp, i64, i64, i64, i32, i32, i32, vp, C.c_size_t, vp, vp,
-                                       vp],
-}
-
-# size_t helpers of the deterministic variants: name -> argtypes
-_SIZE_HELPERS = {
-    "pn_bn_stats_workspace_bytes": [i64, i32],
-    "pn_grad_weight_f32_workspace_bytes": [i64, i32, i32],
-    "pn_grad_weight_bf16x3_workspace_bytes": [i64, i32, i32],
-    "pn_csr_workspace_bytes": [i64, i64],
-    "pn_cross_entropy_workspace_bytes": [i64],
-    "pn_chamfer_workspace_bytes": [i32, i32],
-    "pn_square_distance_bwd_det_workspace_bytes": [i32, i32, i32],
-}
+with open(HEADER) as _f:
+    _CONSTS, _STRUCTS, _FUNCTIONS = parse_header(_f.read())
+MLP_MAX_LAYERS = _CONSTS["PN_MLP_MAX_LAYERS"]
+LaunchOpts = _STRUCTS["pn_launch_opts"]           # per-call launch options (all zeros = defaults)
+MlpDesc = _STRUCTS["pn_mlp_desc"]
+TrainPackItem = _STRUCTS["pn_train_pack_item"]
 
 
 def declared_symbols() -> list:
     """Every function name include/pn12_b200.h declares (used by the export test)."""
-    with open(HEADER) as f:
-        text = f.read()
-    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
-    return sorted(set(re.findall(r"\b(pn_[a-z0-9_]+)\s*\(", text)))
+    return sorted(_FUNCTIONS)
 
 
 def lib():
@@ -161,28 +100,9 @@ def lib():
                 f"{LIB_PATH} is missing: build it with `python -m pointnet12_b200.build` "
                 "(nvcc, sm_100a). pointnet12_b200 has no CPU or PyTorch fallback.")
         handle = C.CDLL(LIB_PATH)
-        handle.pn_last_error_string.restype = C.c_char_p
-        handle.pn_last_error_string.argtypes = []
-        for name, argtypes in _SIGNATURES.items():
+        for name, (argtypes, restype) in _FUNCTIONS.items():
             fn = getattr(handle, name)
-            fn.argtypes = argtypes
-            fn.restype = i32
-        handle.pn_mlp_blob_bytes.argtypes = [_descp]
-        handle.pn_mlp_blob_bytes.restype = C.c_size_t
-        handle.pn_mlp_resident_groups.argtypes = [_descp]
-        handle.pn_mlp_resident_groups.restype = C.c_int
-        handle.pn_ball_grid_bytes.argtypes = [i32, i32]
-        handle.pn_ball_grid_bytes.restype = C.c_size_t
-        handle.pn_three_nn_blocks_bytes.argtypes = [i32, i32]
-        handle.pn_three_nn_blocks_bytes.restype = C.c_size_t
-        handle.pn_train_gemm_scratch_bytes.argtypes = [i32, i32]
-        handle.pn_train_gemm_scratch_bytes.restype = C.c_size_t
-        handle.pn_scan_workspace_bytes.argtypes = [i32, i64]
-        handle.pn_scan_workspace_bytes.restype = C.c_size_t
-        for name, argtypes in _SIZE_HELPERS.items():
-            fn = getattr(handle, name)
-            fn.argtypes = argtypes
-            fn.restype = C.c_size_t
+            fn.argtypes, fn.restype = argtypes, restype
         _lib = handle
     return _lib
 

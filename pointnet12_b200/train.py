@@ -48,8 +48,6 @@ class PackedWeights:
     parameter's storage has moved since (the GEMM then converts the weight itself)."""
 
     def __init__(self, convs):
-        import numpy as np
-
         from . import _native as nv
 
         items, self.slots, total = [], {}, 0
@@ -67,11 +65,11 @@ class PackedWeights:
             return
         dev = items[0][0].device
         self.arena = torch.empty((total,), dtype=torch.uint8, device=dev)
-        table = np.zeros(self.n, dtype=[("w", "<u8"), ("out", "<u8"), ("cin", "<i4"), ("cout", "<i4"), ("tr", "<i4"), ("res", "<i4")])
+        table = (nv.TrainPackItem * self.n)()
         for i, (w, off, nbytes, cin, cout, tr) in enumerate(items):
-            table[i] = (w.data_ptr(), self.arena.data_ptr() + off, cin, cout, int(tr), 0)
+            table[i] = nv.TrainPackItem(w.data_ptr(), self.arena.data_ptr() + off, cin, cout, int(tr), 0)
             self.slots[(w.data_ptr(), tr)] = self.arena[off:off + nbytes]
-        self.table = torch.from_numpy(table.view(np.uint8).copy()).to(dev)
+        self.table = torch.frombuffer(bytearray(table), dtype=torch.uint8).to(dev)
         self.max_cin, self.max_cout = max(i[3] for i in items), max(i[4] for i in items)
         self._ptrs = [(w, w.data_ptr()) for w, *_ in items]
 

@@ -20,8 +20,6 @@ def test_library_exports_every_declared_symbol():
     missing = [s for s in declared if not hasattr(lib, s)]
     assert not missing, f"libpn12_b200.so does not export {missing}"
     assert lib.pn_version() >= 100
-    # every bound signature is a declared symbol (no stale bindings)
-    assert set(nv._SIGNATURES) <= set(declared)
 
 
 def test_argument_validation_needs_no_gpu():
