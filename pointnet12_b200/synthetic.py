@@ -88,6 +88,127 @@ def modelnet_batch(batch: int, n_points: int = 1024, seed: int = 4000) -> np.nda
     return np.ascontiguousarray(pts.transpose(0, 2, 1), dtype=np.float32)
 
 
+# ------------------------------------------------------------------------------------------------ clouds at the geometry edges
+# Inputs built to reach the decisions where the sampling, ball-query and 3-NN kernels can go wrong: ties between DISTINCT
+# points, points exactly on the radius, sampling that runs out of distinct points, zero extent along an axis, large |p|^2 in
+# the expansion formula and points beyond the reference's initial FPS distance of 1e10 (pointnet_util.py:74).
+LATTICE_STEP = 2.0 ** -5
+
+
+def lattice_batch(batch: int, n_points: int, side: int = 29, seed: int = 0) -> np.ndarray:
+    """[B, 4, N]: N distinct sites of the integer lattice {-side//2 .. side-1-side//2}^3 scaled by 2^-5, in shuffled index
+    order; the 4th channel is uniform in [-1, 1).  Every coordinate is k / 32 with |k| < 32, so the reference's distance
+    formulas are exact in fp32 (equal to float64): ties between distinct points are real, and r**2 is exact for r = k / 32."""
+    if n_points > side ** 3:
+        raise ValueError(f"a {side}^3 lattice has fewer than {n_points} sites")
+    rng = np.random.default_rng(seed)
+    out = np.empty((batch, 4, n_points), dtype=np.float32)
+    for b in range(batch):
+        site = rng.choice(side ** 3, n_points, replace=False)
+        ijk = np.stack([site % side, site // side % side, site // side ** 2], axis=0) - side // 2
+        out[b, :3] = ijk * LATTICE_STEP
+        out[b, 3] = rng.uniform(-1.0, 1.0, n_points)
+    return out
+
+
+def few_distinct_batch(batch: int, n_points: int, distinct: int, seed: int = 0) -> np.ndarray:
+    """[B, 4, N]: `distinct` different points (uniform in [-1, 1)^4) resampled to N, each of them present at least once."""
+    rng = np.random.default_rng(seed)
+    out = np.empty((batch, 4, n_points), dtype=np.float32)
+    for b in range(batch):
+        base = rng.uniform(-1.0, 1.0, (4, distinct)).astype(np.float32)
+        pick = np.concatenate([np.arange(distinct), rng.integers(0, distinct, n_points - distinct)])
+        out[b] = base[:, rng.permutation(pick)]
+    return out
+
+
+def flat_batch(batch: int, n_points: int, axes: str = "z", config: int = 30) -> np.ndarray:
+    """kitti_batch with the coordinates named in `axes` ("z": a plane, "yz": a line) set to one constant per axis."""
+    out = kitti_batch(batch, n_points, config=config)
+    for a in axes:
+        out[:, "xyz".index(a)] = np.float32(-0.375 if a == "z" else 0.125)
+    return out
+
+
+def offset_batch(batch: int, n_points: int, config: int = 31) -> np.ndarray:
+    """kitti_batch back in metres (x 70, y 70, z 3) and shifted by +1000 m in x: |p|^2 ~ 1e6, so the expansion formula of
+    the reference's square_distance cancels and rounds by ~0.1 m^2."""
+    out = kitti_batch(batch, n_points, config=config)
+    out[:, 0] = out[:, 0] * np.float32(70) + np.float32(1000)
+    out[:, 1] *= np.float32(70)
+    out[:, 2] *= np.float32(3)
+    return out
+
+
+OUTLIER_FAR = (2.0e5, 3.0e5)
+
+
+def outlier_batch(batch: int, n_points: int, config: int = 32) -> np.ndarray:
+    """kitti_batch with 4 points moved to |p| ~ 1e3 and two to x = -2e5 and x = +3e5, the nearer one at the lower index.
+    Both far points are more than 1e5 from any start point, so their squared distance exceeds the reference's initial
+    1e10 (pointnet_util.py:74): after the first pick the running minimum caps both at 1e10 and the tie goes to the lower
+    index, where an uncapped kernel would take the farther point."""
+    out = kitti_batch(batch, n_points, config=config)
+    rng = np.random.default_rng(config)
+    for b in range(batch):
+        pos = rng.choice(n_points, 6, replace=False)
+        d = rng.normal(size=(3, 4))
+        out[b, :3, pos[:4]] = (1000.0 * d / np.linalg.norm(d, axis=0)).T.astype(np.float32)
+        lo, hi = np.sort(pos[4:])
+        out[b, :3, lo] = np.float32([-OUTLIER_FAR[0], 0.0, 0.0])
+        out[b, :3, hi] = np.float32([OUTLIER_FAR[1], 0.0, 0.0])
+    return out
+
+
+def boundary_batch(batch: int, n_points: int, radius: float, per_level: int = 24, seed: int = 0) -> np.ndarray:
+    """[B, 4, N] for a ball query centred at the ORIGIN, which is point 0 of every cloud: `per_level` points each whose
+    squared norm ((x*x + y*y) + z*z in fp32 -- the reference's square_distance from the origin) is exactly fp32(radius**2),
+    one ulp below it and one ulp above it, and background points farther than 2 * radius.  The fine structure decides
+    membership: `sqrdists > radius ** 2` (pointnet_util.py:102) keeps the first two levels and drops the third, and a
+    threshold of fp32(fp32(radius) ** 2) -- one ulp higher at radius 0.1, 0.2, 0.4 and 0.8 -- would keep all three."""
+    rng = np.random.default_rng(seed)
+    r2 = np.float32(radius ** 2)
+    targets = (np.nextafter(r2, np.float32(0)), r2, np.nextafter(r2, np.float32(1e30)))
+    out = np.empty((batch, 4, n_points), dtype=np.float32)
+    for b in range(batch):
+        pts = []
+        for t in targets:
+            for _ in range(per_level):
+                pts.append(_on_sphere(float(radius), t, rng))
+        pts = np.array(pts, dtype=np.float32)
+        nb = n_points - 1 - len(pts)
+        d = rng.normal(size=(nb, 3))
+        far = d / np.linalg.norm(d, axis=1, keepdims=True) * rng.uniform(2.0 * radius + 0.05, 2.0 * radius + 1.0, (nb, 1))
+        xyz = np.concatenate([pts, far.astype(np.float32)])[rng.permutation(n_points - 1)]
+        out[b, :3, 0] = 0.0
+        out[b, :3, 1:] = xyz.T
+        out[b, 3] = rng.uniform(-1.0, 1.0, n_points)
+    return out
+
+
+def sqnorm_f32(p) -> np.float32:
+    """(x*x + y*y) + z*z rounded like the reference's fp32 tensor ops."""
+    x, y, z = (np.float32(v) for v in p)
+    return np.float32(np.float32(x * x + y * y) + np.float32(z * z))
+
+
+def _on_sphere(radius: float, target: np.float32, rng: np.random.Generator) -> np.ndarray:
+    """A point with sqnorm_f32(p) == target exactly: random x, y, then z found among the floats next to the real root."""
+    while True:
+        u = rng.normal(size=3)
+        u *= radius / np.linalg.norm(u)
+        x, y = np.float32(u[0]), np.float32(u[1])
+        xy = np.float32(x * x + y * y)
+        if not float(xy) < 0.9 * float(target):
+            continue
+        z = np.float32(np.sqrt(float(target) - float(xy)))
+        for _ in range(64):
+            s = sqnorm_f32((x, y, z))
+            if s == target:
+                return np.array([x, y, z if u[2] >= 0 else -z], dtype=np.float32)
+            z = np.nextafter(z, np.float32(1e30) if s < target else np.float32(0))
+
+
 def checksum(arr: np.ndarray) -> str:
     """Stable digest of an array's bytes (dtype and shape included)."""
     h = hashlib.sha256()
